@@ -19,6 +19,12 @@ arcs (NCCL all-gather + merge when N > 1).
             The cost matrix is uploaded once per problem (manager state, like `ot.M` in the
             reference's `OTManager`), not per pricing pass; `e2e_cold` adds that upload.
 `roofline`: achieved HBM GB/s of the pricing kernel alone (8 B per arc / CUDA-event time).
+
+`--dump-outputs DIR` writes the result of the last timed step (what `PriceResult` hands a caller: violator
+count, min reduced cost, top-K arc ids and reduced costs) as DIR/<name>.npy, float64, and for the second leg as
+DIR/c4_<name>.npy.  The inputs are generated from fixed seeds, so two builds run with the same arguments can be
+compared file for file.  With `--impl reference` the dump fixes the host's row sample at the first 512 seeded rows
+instead of sizing it from a timed pass.
 """
 import argparse
 import hashlib
@@ -72,7 +78,33 @@ def parse():
     ap.add_argument("--kruskal-chunk", type=int, default=0, help="sx_kruskal_set_tuning (first chunk in quarters of N)")
     ap.add_argument("--tree-only", type=int, default=0, metavar="S",
                     help="only time the tree-basis build on an S x S instance and exit")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the result of the last timed pricing step to DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.sweep or args.tree_only):
+        ap.error("--dump-outputs needs a pricing run (not --sweep or --tree-only)")
+    return args
+
+
+DUMP_MAX_TOPK = 1 << 20      # top-K entries written per leg: at most 3 x 8 MB, both legs within 64 MB
+
+
+def dump_outputs(out_dir, prefix, count, min_rc, ids, rc):
+    """Writes one pricing result, as `device.PriceResult` returns it, to out_dir/<prefix><name>.npy in float64
+    (arc ids are exact below 2^53).  A top-K list longer than DUMP_MAX_TOPK is cut to a fixed, seeded sample of
+    its positions, which are written as <prefix>topk_pos.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    ids, rc = np.asarray(ids), np.asarray(rc)
+    arrays = {"n_violating": [count], "min_rc": [min_rc]}
+    if ids.size > DUMP_MAX_TOPK:
+        pos = np.sort(np.random.default_rng(0).choice(ids.size, DUMP_MAX_TOPK, replace=False))
+        ids, rc = ids[pos], rc[pos]
+        arrays["topk_pos"] = pos
+    arrays["topk_id"], arrays["topk_rc"] = ids, rc
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def measured_peak_gbs():
@@ -118,6 +150,7 @@ class ClockSampler:
             self.proc.wait(timeout=5)
         except Exception:
             self.proc.kill()
+        self.proc = None
         sm, mx, reasons = [], [], set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         try:
@@ -228,11 +261,15 @@ def run_reference(args):
     M = (P[:, 0:1] - Q[None, :, 0]) ** 2 + (P[:, 1:2] - Q[None, :, 1]) ** 2
     b = (M + a[:, None]).min(axis=0) + 2e-3
     y = np.concatenate([a, b])
-    rate, dt = cpu_price_rate(M, y, args.topk, threads, 1)
-    # size the per-step sample so that steps + warmup take about two minutes
-    budget = 120.0 / max(1, args.steps + args.warmup)
-    rows2 = int(min(S, max(256, rows * budget / dt)))
-    rows2 = min(rows2, 8192)
+    if args.dump_outputs:
+        # a dumped result must not depend on how fast this host is: the first seeded rows, not a timed size
+        rows2 = min(S, rows)
+    else:
+        # size the per-step sample so that steps + warmup take about two minutes
+        rate, dt = cpu_price_rate(M, y, args.topk, threads, 1)
+        budget = 120.0 / max(1, args.steps + args.warmup)
+        rows2 = int(min(S, max(256, rows * budget / dt)))
+        rows2 = min(rows2, 8192)
     if rows2 != rows:
         P = rng.random((rows2, 2)); a = rng.random(rows2)
         M = (P[:, 0:1] - Q[None, :, 0]) ** 2 + (P[:, 1:2] - Q[None, :, 1]) ** 2
@@ -243,8 +280,10 @@ def run_reference(args):
         orc.price_dense_ot_blocked(M, y, args.topk, TOL, threads=threads, block_rows=64)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        orc.price_dense_ot_blocked(M, y, args.topk, TOL, threads=threads, block_rows=64)
+        result = orc.price_dense_ot_blocked(M, y, args.topk, TOL, threads=threads, block_rows=64)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "", *result)
     value = M.size * args.steps / dt
     sample = f"{rows2} of {S} rows x {D} cols per step ({M.size:.3g} arcs), oracle port, NumPy row blocks"
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
@@ -616,7 +655,13 @@ def main():
     peak, peak_src = measured_peak_gbs()
     steps, warmup = args.steps, max(args.warmup, 3)
     sampler = ClockSampler(local)
-    main_leg = pricing_leg(args, S, D, ctx, steps, warmup, sampler=sampler, want_cpu=not args.no_cpu, want_cold=True)
+    try:
+        main_leg = pricing_leg(args, S, D, ctx, steps, warmup, sampler=sampler, want_cpu=not args.no_cpu,
+                               want_cold=True)
+    finally:
+        sampler.stop()                                   # no-op after a normal leg; a failed one leaves no nvidia-smi
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "", *main_leg["result"])
     main_mgr = manager_leg(args, S, D, ctx, steps, main_leg)
     # second, shorter leg: BASELINE.json configs[3] (dense OT 20 000 x 20 000, "pricing at 1/2/4/8 B200")
     c4_leg, c4_mgr = None, None
@@ -624,6 +669,8 @@ def main():
         c4_leg = pricing_leg(args, args.c4_size, args.c4_size, ctx, steps, warmup, sampler=None, want_cpu=False,
                              want_cold=False)
         c4_mgr = manager_leg(args, args.c4_size, args.c4_size, ctx, steps, c4_leg)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, "c4_", *c4_leg["result"])
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -858,6 +905,12 @@ def pricing_leg(args, S, D, ctx, steps, warmup, sampler, want_cpu, want_cold):
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     own_ms = e0.elapsed_time(e1)                          # this rank's own clock over the same region
     phases = sp.pricer.fused_phase_us() if sp.fused else None     # in-kernel stamps of the LAST timed pass
+    # the result of the last timed step, read before any further pass reuses the pricer's buffers
+    count_dev = int(out[3].item())
+    assert int(out[6].item()) == 0, "selection status not clean: the timed pass would have to be repeated"
+    n_out = int(out[2].item())
+    ids_dev, rc_dev = out[1][:n_out].cpu().numpy(), out[0][:n_out].cpu().numpy()
+    min_dev = float(lib.sx_key_to_f64(int(out[4].item())))
     # Duration of the pricing kernel.  With the fused pass a step IS one launch of that kernel, so its average
     # launch duration is the timed region / steps (this rank's events around the region).  Only when a step is
     # several launches (separate kernels) are events put around each pricing launch, in a loop of its own: two
@@ -871,11 +924,6 @@ def pricing_leg(args, S, D, ctx, steps, warmup, sampler, want_cpu, want_cold):
         barrier()
         kern_ms = float(np.mean([k0[i].elapsed_time(k1[i]) for i in range(steps)]))
         kern_src = "CUDA events around each pricing launch, separate loop"
-    count_dev = int(out[3].item())
-    assert int(out[6].item()) == 0, "selection status not clean: the timed pass would have to be repeated"
-    n_out = int(out[2].item())
-    ids_dev, rc_dev = out[1][:n_out].cpu().numpy(), out[0][:n_out].cpu().numpy()
-    min_dev = float(lib.sx_key_to_f64(int(out[4].item())))
     digest = topk_digest(ids_dev, rc_dev, count_dev, min_dev)
     value = S * D * steps / (ms_total * 1e-3)
 
@@ -987,7 +1035,8 @@ def pricing_leg(args, S, D, ctx, steps, warmup, sampler, want_cpu, want_cold):
            "stage_us": stages,
            "gpu_launches": launches, "violating_arcs": count_dev, "topk_digest": digest, "merge_check": merge_check,
            "e2e": e2e, "e2e_pinned": e2e_pinned, "e2e_cold": cold, "cpu_baseline": cpu_baseline, "clocks": clocks,
-           "exchange": sp.exchange, "fused": sp.fused, "y_host": y_host, "row_bounds": row_bounds, "balance": balance}
+           "exchange": sp.exchange, "fused": sp.fused, "y_host": y_host, "row_bounds": row_bounds, "balance": balance,
+           "result": (count_dev, min_dev, ids_dev, rc_dev)}
     del sp, M_loc, y_dev
     torch.cuda.empty_cache()
     barrier()
