@@ -54,7 +54,7 @@ extern "C" {
 #define SX_ERR_PEER_TIMEOUT    -8   /* sx_exchange_blocks: a peer never raised its flag */
 #define SX_ERR_PUSH_ASSERT     -9   /* sx_push_tree_h: the reference's assertions would fire (tree_BI.py:93-94) */
 
-#define SX_ABI_VERSION 4
+#define SX_ABI_VERSION 5
 
 /* Endpoint convention of sx_tree_potentials (which end of an arc carries +1 in A). */
 #define SX_PLUS_IS_HEAD 0   /* OT:  A[S+j,k] = +1, A[i,k] = -1      (formats.py:156-158)     */
@@ -69,8 +69,9 @@ typedef struct sx_price_header {
 } sx_price_header;
 
 #define SX_STATUS_CAND_OVERFLOW  1   /* candidate buffer too small: enlarge it and price again */
-#define SX_STATUS_NEED_SORTED    2   /* too many ties at the K-th reduced cost for the fast selection:
-                                        call sx_topk_select_sorted on the same candidates */
+#define SX_STATUS_DUPLICATE_CANDIDATES 2   /* the candidates repeat one (rc, id) pair too often to select
+                                              from: the same arcs were priced into one pass more than once.
+                                              The selection is void; no repeat can fix it */
 #define SX_STATUS_K_MISMATCH     4   /* sx_topk_select asked for more arcs than sx_price_pass_begin
                                         announced: the candidates were pruned for the smaller K */
 #define SX_STATUS_NAN_RC         8   /* some reduced cost was NaN.  It is neither counted in n_violating nor
@@ -80,7 +81,7 @@ typedef struct sx_price_header {
 #define SX_STATUS_NEED_UNFUSED  16   /* sx_price_dense_ot_fused could not finish its selection (more than 4096
                                         candidates tie around the K-th value): run the pass again with
                                         sx_price_pass_begin / sx_price_dense_ot / sx_topk_select */
-#define SX_STATUS_REPEAT_MASK   19   /* bits that ask for the pass / selection to be repeated */
+#define SX_STATUS_REPEAT_MASK   17   /* bits that ask for the pass to be repeated */
 
 /* Selection state of a pricing pass (opaque device memory, sx_select_state_bytes() bytes, 16 B
  * aligned): candidate counter, pruning bound and the reduced-cost histogram the bound is derived
@@ -241,6 +242,8 @@ SX_API int    sx_push_tree_h(const int64_t *tree_h, const double *flow_h, int64_
  * sx_price_pass_begin must be enqueued before the first sx_price_* call of a pass (it clears the
  *   header and `sel`, and records the K the pass prunes for; sel may be NULL when cand_cap = 0);
  *   several calls (row slabs, arc-list tail) may then accumulate into one header / candidate list.
+ *   A pass must not price an arc twice: the selection ranks distinct (rc, id) pairs (see
+ *   SX_STATUS_DUPLICATE_CANDIDATES).
  */
 SX_API size_t sx_select_state_bytes(void);
 SX_API int    sx_price_pass_begin(sx_price_header *header, sx_select_state *sel, int64_t K, void *stream);
@@ -305,12 +308,12 @@ SX_API int    sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0,
  * id ascending).  sel / header are the pass's selection state and header (the candidate count
  * lives in sel).  out_rc / out_id have capacity K; out_n (device int64) = min(K, #violators).
  * Entries past out_n are filled with (+inf, -1) so fixed-size blocks can be exchanged.
- * sx_topk_select: K <= SX_TOPK_MAX_K runs the histogram filter + all-pairs rank (two launches,
- *   no host round trip); if it cannot finish (more than 8192 candidates tie around the K-th
- *   value) it raises SX_STATUS_NEED_SORTED in header->status and the caller runs
- *   sx_topk_select_sorted on the same buffers.  K > SX_TOPK_MAX_K goes to the sorted path directly.
- * sx_topk_select_sorted: bitonic slice sort + rank merge (K <= SX_TOPK_MAX_K) or two stable radix
- *   argsorts (larger K; synchronises the stream once to read the candidate count).
+ * sx_topk_select: K <= SX_TOPK_MAX_K runs the histogram filter, radix refinement of the boundary
+ *   bin on (rc, id) and an all-pairs rank in one cooperative launch (no host round trip); it
+ *   always finishes on distinct candidates, however many of them tie on rc.  When one (rc, id)
+ *   pair at the K-th position has more copies than 8192 minus the candidates ranked before it,
+ *   it raises SX_STATUS_DUPLICATE_CANDIDATES and leaves out_n = 0.  Larger K runs two stable
+ *   radix argsorts (synchronises the stream once to read the candidate count).
  * sx_topk_merge merges G sorted, padded blocks (as exchanged between G ranks) into one.  Block g
  *   has its rc list at blocks_rc + g * block_stride and its ids at blocks_id + g * block_stride
  *   (strides in 8-byte elements, so the gathered buffer is consumed in place).  Optionally folds
@@ -324,9 +327,6 @@ SX_API int    sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0,
 #define SX_TOPK_MAX_K 1024
 SX_API size_t sx_topk_workspace_bytes(int64_t cand_cap, int64_t K);
 SX_API int    sx_topk_select(const double *cand_rc, const int64_t *cand_id, int64_t cand_cap,
-                      sx_select_state *sel, sx_price_header *header, int64_t K, double *out_rc,
-                      int64_t *out_id, int64_t *out_n, void *ws, size_t ws_bytes, void *stream);
-SX_API int    sx_topk_select_sorted(const double *cand_rc, const int64_t *cand_id, int64_t cand_cap,
                       sx_select_state *sel, sx_price_header *header, int64_t K, double *out_rc,
                       int64_t *out_id, int64_t *out_n, void *ws, size_t ws_bytes, void *stream);
 SX_API size_t sx_topk_merge_workspace_bytes(int64_t G);

@@ -26,7 +26,7 @@ namespace {
 
 using namespace sx;
 
-enum Mode { kFused = 0, kSeparate = 1, kSeparateSorted = 2 };
+enum Mode { kFused = 0, kSeparate = 1 };
 enum Cmd { kIdle = 0, kPrice = 1, kGrow = 2, kQuit = 3 };
 
 struct DevCtx {
@@ -121,9 +121,8 @@ int run_pass(sx_ot_pricer *p, DevCtx *c) {
         SXP(sx_price_dense_ot(c->M, p->ld, c->row0, c->S_loc, D, c->y_loc, c->y_loc + c->S_loc, p->tol, hdr,
                               (sx_select_state *)c->sel, c->cand_rc, c->cand_id, cap, nullptr, 0, -1, c->st));
         if (p->K > 0) {
-            auto fn = p->mode == kSeparateSorted ? sx_topk_select_sorted : sx_topk_select;
-            SXP(fn(c->cand_rc, c->cand_id, cap, (sx_select_state *)c->sel, hdr, p->K, (double *)c->block, c->block + Kp,
-                   c->block + 2 * Kp + 4, c->topk_ws, c->topk_ws_bytes, c->st));
+            SXP(sx_topk_select(c->cand_rc, c->cand_id, cap, (sx_select_state *)c->sel, hdr, p->K, (double *)c->block,
+                               c->block + Kp, c->block + 2 * Kp + 4, c->topk_ws, c->topk_ws_bytes, c->st));
         }
         if (p->G > 1) SXP(sx_exchange_push_ll(c->block, p->blk, c->peer_bufs_dev, c->g, p->G, c->st));
     }
@@ -359,8 +358,6 @@ extern "C" int sx_ot_pricer_price_h(sx_ot_pricer *p, const double *y_src_h, cons
             p->new_cap = cap;
             SXP(run_all(p, kGrow));
             p->cap = cap;
-        } else if (status & SX_STATUS_NEED_SORTED) {
-            p->mode = kSeparateSorted;
         } else {
             p->mode = kSeparate;
         }

@@ -72,11 +72,11 @@ __device__ __forceinline__ bool keyid_less(const KeyId &a, const KeyId &b) {
 }
 
 // bits of sx_price_header.status
-constexpr unsigned long long kStatusCandOverflow = 1ull;   // candidate buffer too small: grow and price again
-constexpr unsigned long long kStatusNeedSlowPath = 2ull;   // too many survivors (ties): use sx_topk_select_sorted
-constexpr unsigned long long kStatusKMismatch    = 4ull;   // selection asked for more than the pass pruned for
-constexpr unsigned long long kStatusNeedUnfused  = 16ull;  // fused pass could not finish its selection: run the separate kernels
-constexpr unsigned long long kStatusNanRc        = 8ull;    // a reduced cost was NaN: not optimal (np.all(rc >= -tol) is False)
+constexpr unsigned long long kStatusCandOverflow        = 1ull;   // candidate buffer too small: grow and price again
+constexpr unsigned long long kStatusDuplicateCandidates = 2ull;   // one (rc, id) pair repeats too often: selection void
+constexpr unsigned long long kStatusKMismatch           = 4ull;   // selection asked for more than the pass pruned for
+constexpr unsigned long long kStatusNeedUnfused         = 16ull;  // fused pass could not finish its selection: run the separate kernels
+constexpr unsigned long long kStatusNanRc               = 8ull;    // a reduced cost was NaN: not optimal (np.all(rc >= -tol) is False)
 
 // Monotone (non-strict) 19-bit image of a reduced cost: a < b  =>  bin(a) <= bin(b).
 // Negative values (every violator when tol >= 0) use the full resolution; anything >= +0 clamps

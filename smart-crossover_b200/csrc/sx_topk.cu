@@ -4,25 +4,23 @@
 // only tests `np.all(rc >= -tol)`, net_manager.py:318,496): among the candidates (rc, arc id)
 // compacted by the pricing kernels, return the K smallest by (rc ascending, id ascending).
 // (rc, id) is a strict total order, so the result does not depend on the (unordered)
-// compaction, on the slicing below, or on how many GPUs priced the matrix.
+// compaction or on how many GPUs priced the matrix.
 //
-// Fast path, K <= 1024 (device-driven, two launches, no host round trip):
+// K <= 1024: ONE cooperative launch (topk_select_kernel), no host round trip:
 //   1. filter: the pricing kernels left a histogram of the candidates' reduced costs
 //      (sx_select.cuh); b* = the smallest bin whose cumulative count reaches K.  Candidates
-//      with bin <= b* survive: the K best plus the rest of bin b* (0.4 % wide);
-//   2. all-pairs rank: every survivor counts the survivors below it; that count is its
+//      with bin < b* are among the K best, bin b* (0.4 % wide) is the boundary list;
+//   2. refine: while the list is too long, an 11-bit digit of (key, id) splits the boundary list
+//      again; a list of distinct (key, id) pairs shrinks to one element within 12 levels;
+//   3. all-pairs rank: every survivor counts the survivors below it; that count is its
 //      position in the output.  O(n_surv^2) compares spread over the whole GPU (1 to 32 lanes
 //      per element), a few microseconds for the typical 1-2 K survivors.
-//   More than 8192 survivors (massive ties around the K-th value) raise
-//   SX_STATUS_NEED_SORTED in the pricing header and the caller runs the sorted path.
-// The same all-pairs rank merges the per-GPU lists after the exchange (sx_topk_merge).
-// Sorted path (sx_topk_select_sorted), K <= 1024:
-//   1. every CTA bitonic-sorts one slice of 4096 candidates -- the 5 innermost stages of each
-//      merge step run on registers with warp shuffles, the wider ones through shared memory --
-//      and keeps the slice's K best as a padded, sorted list;
-//   2. rank merge: an element's global rank is the sum over lists of lower_bound(list, element);
-//      elements above the smallest "K-th of a full list" cannot be in the answer and are skipped.
+//   The candidates must be distinct arcs.  Only copies of one (rc, id) pair -- the same arc priced
+//   into one pass many times -- can keep the list long; the selection is then void and raises
+//   SX_STATUS_DUPLICATE_CANDIDATES in the pricing header.
 // K > 1024: two stable radix argsorts (by id, then by rc) over the candidates.
+// Merge of G sorted, padded per-GPU lists after the exchange (sx_topk_merge): an element's position is
+// the number of entries below it in every list (binary searches).
 #include <math.h>
 
 #include <cooperative_groups.h>
@@ -35,17 +33,10 @@ namespace cg = cooperative_groups;
 
 namespace sx {
 
-constexpr int kTkSlice   = 4096;
-constexpr int kTkThreads = 1024;
-constexpr int kTkItems   = kTkSlice / kTkThreads;   // 4
-
 struct Cand {
     double    rc;
     long long id;
 };
-__device__ __forceinline__ bool cand_less(const Cand &a, const Cand &b) {
-    return a.rc < b.rc || (a.rc == b.rc && a.id < b.id);
-}
 __device__ __forceinline__ Cand cand_pad() { return Cand{INFINITY, -1}; }
 // padding must sort after every real candidate: compare as (+inf, max id)
 __device__ __forceinline__ bool cand_less_p(const Cand &a, const Cand &b) {
@@ -59,84 +50,6 @@ __device__ __forceinline__ Cand shfl_xor_cand(const Cand &c, int mask) {
     r.rc = __shfl_xor_sync(0xffffffffu, c.rc, mask);
     r.id = __shfl_xor_sync(0xffffffffu, c.id, mask);
     return r;
-}
-
-// One CTA sorts candidates [b*4096, (b+1)*4096) and writes its K best (padded) to lists[b].
-__global__ void __launch_bounds__(kTkThreads)
-topk_slice_sort_kernel(const double *__restrict__ cand_rc, const long long *__restrict__ cand_id,
-                       const unsigned long long *__restrict__ n_cand_dev, long long cand_cap, int K,
-                       double *__restrict__ lists_rc, long long *__restrict__ lists_id) {
-    extern __shared__ __align__(16) unsigned char tk_raw[];
-    Cand *sm = reinterpret_cast<Cand *>(tk_raw);
-    unsigned long long n64 = *n_cand_dev;
-    const long long n = n64 > (unsigned long long)cand_cap ? cand_cap : (long long)n64;
-    const long long base = (long long)blockIdx.x * kTkSlice;
-    double    *out_rc = lists_rc + (long long)blockIdx.x * K;
-    long long *out_id = lists_id + (long long)blockIdx.x * K;
-    if (base >= n) {   // empty slice: all padding
-        for (int i = threadIdx.x; i < K; i += kTkThreads) { out_rc[i] = INFINITY; out_id[i] = -1; }
-        return;
-    }
-    // element index i = q * 1024 + tid: bits 0-4 = lane, 5-9 = warp, 10-11 = register slot
-    Cand e[kTkItems];
-#pragma unroll
-    for (int q = 0; q < kTkItems; ++q) {
-        const long long g = base + q * kTkThreads + threadIdx.x;
-        e[q] = (g < n) ? Cand{cand_rc[g], cand_id[g]} : cand_pad();
-    }
-    // both loops have compile-time trip counts and are fully unrolled, so every e[] index is static
-    // (a dynamic index would push e[] to local memory)
-#pragma unroll
-    for (int k = 2; k <= kTkSlice; k <<= 1) {
-#pragma unroll
-        for (int j = k >> 1; j > 0; j >>= 1) {
-            if (j >= kTkThreads) {
-                // partner lives in another register slot of the same thread
-                const int dq = j / kTkThreads;
-#pragma unroll
-                for (int q = 0; q < kTkItems; ++q) {
-                    if ((q & dq) == 0) {
-                        const int i = q * kTkThreads + threadIdx.x;
-                        const bool asc = (i & k) == 0;
-                        Cand &lo = e[q], &hi = e[q | dq];
-                        if (cand_less_p(hi, lo) == asc) { Cand t = lo; lo = hi; hi = t; }
-                    }
-                }
-            } else if (j >= 32) {
-                // partner lives in another warp: exchange through shared memory
-                __syncthreads();
-#pragma unroll
-                for (int q = 0; q < kTkItems; ++q) sm[q * kTkThreads + threadIdx.x] = e[q];
-                __syncthreads();
-#pragma unroll
-                for (int q = 0; q < kTkItems; ++q) {
-                    const int i = q * kTkThreads + threadIdx.x;
-                    const Cand other = sm[i ^ j];
-                    const bool asc = (i & k) == 0, lower = (i & j) == 0;
-                    const bool take_min = lower == asc;
-                    const bool other_smaller = cand_less_p(other, e[q]);
-                    if (take_min == other_smaller) e[q] = other;
-                }
-            } else {
-                // partner lives in another lane of the same warp: warp shuffle
-#pragma unroll
-                for (int q = 0; q < kTkItems; ++q) {
-                    const int i = q * kTkThreads + threadIdx.x;
-                    const Cand other = shfl_xor_cand(e[q], j);
-                    const bool asc = (i & k) == 0, lower = (i & j) == 0;
-                    const bool take_min = lower == asc;
-                    const bool other_smaller = cand_less_p(other, e[q]);
-                    if (take_min == other_smaller) e[q] = other;
-                }
-            }
-        }
-    }
-    // sorted ascending over i; the K best are i < K
-#pragma unroll
-    for (int q = 0; q < kTkItems; ++q) {
-        const int i = q * kTkThreads + threadIdx.x;
-        if (i < K) { out_rc[i] = e[q].rc; out_id[i] = e[q].id; }
-    }
 }
 
 // number of elements of a sorted, padded list prefix [0, len) that are  < x  (strict)
@@ -160,20 +73,14 @@ __device__ __forceinline__ int upper_bound_list(const double *rc, const long lon
     return lo;
 }
 
-__global__ void topk_fill_kernel(double *out_rc, long long *out_id, long long *out_n, int K) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < K) { out_rc[i] = INFINITY; out_id[i] = -1; }
-    if (i == 0) *out_n = 0;
-}
-
-// Rank merge, step 1 (one CTA).  lists: L sorted, padded lists of length K.
+// Rank merge of sx_topk_merge when G * K > 2^22 (too many elements for one thread each), step 1 (one CTA).
+// lists: L sorted, padded lists of length K.
 //   thr      = smallest last element over the lists: the global K-th best is <= it, so only the
 //              prefix of each list with elements <= thr can be in the answer;
 //   plen[l]  = length of that prefix;  poff[l] = exclusive prefix sum;  poff[L] = work total.
 __global__ void __launch_bounds__(1024)
 topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restrict__ lists_id, long long LS, int L,
-                 int K, const unsigned long long *n_cand_dev, long long cand_cap, int *__restrict__ plen,
-                 int *__restrict__ poff, double *__restrict__ out_rc, long long *__restrict__ out_id,
+                 int K, int *__restrict__ plen, int *__restrict__ poff, double *__restrict__ out_rc, long long *__restrict__ out_id,
                  long long *out_n, const long long *headers, long long *out_summary) {
     // outputs start as padding; the rank kernel (next launch) overwrites the first out_n entries
     for (int i = threadIdx.x; i < K; i += blockDim.x) { out_rc[i] = INFINITY; out_id[i] = -1; }
@@ -189,14 +96,6 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
     __shared__ Cand s_thr[32];
     __shared__ int  s_warp[32];
     __shared__ int  s_carry;
-    int Lu = L;
-    long long n_real = -1;
-    if (n_cand_dev) {   // select path: only the first ceil(n / 4096) slices hold data
-        unsigned long long n64 = *n_cand_dev;
-        n_real = n64 > (unsigned long long)cand_cap ? cand_cap : (long long)n64;
-        Lu = (int)((n_real + kTkSlice - 1) / kTkSlice);
-        if (Lu > L) Lu = L;
-    }
     const int lane = lane_id(), warp = threadIdx.x >> 5;
     __shared__ long long s_red[32];
     auto block_sum = [&](long long v) -> long long {
@@ -225,7 +124,7 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
     // bound 1: the smallest "last element of a list" (padding = +inf: no constraint)
     Cand thr = cand_pad();
     long long n_real_lists = 0;
-    for (int l = threadIdx.x; l < Lu; l += blockDim.x) {
+    for (int l = threadIdx.x; l < L; l += blockDim.x) {
         const long long *ids = lists_id + (long long)l * LS;
         const Cand c{lists_rc[(long long)l * LS + K - 1], ids[K - 1]};
         if (cand_less_p(c, thr)) thr = c;
@@ -244,11 +143,11 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
         while (lo < hi) {
             const int mid = (lo + hi) >> 1;
             long long part = 0;
-            for (int l = threadIdx.x; l < Lu; l += blockDim.x) part += plen[l] < mid ? plen[l] : mid;
+            for (int l = threadIdx.x; l < L; l += blockDim.x) part += plen[l] < mid ? plen[l] : mid;
             if (block_sum(part) >= K) hi = mid; else lo = mid + 1;
         }
         Cand deep = Cand{-INFINITY, 0};
-        for (int l = threadIdx.x; l < Lu; l += blockDim.x) {
+        for (int l = threadIdx.x; l < L; l += blockDim.x) {
             const int take = plen[l] < lo ? plen[l] : lo;
             if (take > 0) {
                 const Cand c{lists_rc[(long long)l * LS + take - 1], lists_id[(long long)l * LS + take - 1]};
@@ -264,9 +163,9 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
     for (int base = 0; base < L; base += blockDim.x) {
         const int l = base + threadIdx.x;
         int len = 0;
-        if (l < Lu) len = upper_bound_list(lists_rc + (long long)l * LS, lists_id + (long long)l * LS, K, thr);
+        if (l < L) len = upper_bound_list(lists_rc + (long long)l * LS, lists_id + (long long)l * LS, K, thr);
         // do not count padding (id < 0) that ties with an all-padding threshold
-        if (l < Lu && len > 0) {
+        if (l < L && len > 0) {
             int lo = 0, hi = len;                       // first padding entry within [0, len)
             while (lo < hi) { const int mid = (lo + hi) >> 1; if (lists_id[(long long)l * LS + mid] >= 0) lo = mid + 1; else hi = mid; }
             len = lo;
@@ -289,8 +188,7 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
     }
     if (threadIdx.x == 0) {
         poff[L] = (int)real_total;
-        long long n_out = n_real >= 0 ? n_real : real_total;   // merge path: every real entry below thr counts
-        *out_n = n_out < K ? n_out : K;
+        *out_n = real_total < K ? real_total : K;
     }
 }
 
@@ -481,6 +379,9 @@ topk_select_kernel(const double *__restrict__ cand_rc, const long long *__restri
     grid.sync();
 
     // ---- refinement levels ----
+    // Each level leaves a list that agrees on every bit from the chosen digit's lowest bit up, so 6 levels
+    // settle the 64-bit key and 6 more the 63-bit id: only copies of one (key, id) can reach kMaxLevels.
+    static_assert(kMaxLevels >= (64 + 10) / 11 + (63 + 10) / 11, "refinement levels cannot settle a (key, id)");
     int level = 0;
     bool failed = false;
     for (;; ++level) {
@@ -560,7 +461,7 @@ topk_select_kernel(const double *__restrict__ cand_rc, const long long *__restri
         for (int i = n_out + threadIdx.x; i < K; i += kApThreads) { out_rc[i] = INFINITY; out_id[i] = -1; }
         if (threadIdx.x == 0) {
             *out_n = n_out;
-            if (failed) atomicOr(&hdr->status, kStatusNeedSlowPath);
+            if (failed) atomicOr(&hdr->status, kStatusDuplicateCandidates);
         }
     }
     if (n_s == 0) return;
@@ -813,61 +714,19 @@ using namespace sx;
 extern "C" size_t sx_topk_workspace_bytes(int64_t cand_cap, int64_t K) {
     if (cand_cap < 0 || K < 0) return 0;
     const size_t fast = carve_bytes((size_t)kSurvCap, 16) + 2 * carve_bytes((size_t)(cand_cap > 0 ? cand_cap : 1), 16);
-    if (K <= SX_TOPK_MAX_K) {
-        const size_t L = ((size_t)cand_cap + kTkSlice - 1) / kTkSlice + 1;
-        return fast + carve_bytes(L * (size_t)(K > 0 ? K : 1), 8) * 2 + 2 * carve_bytes(L + 2, 4) + 256;
-    }
+    if (K <= SX_TOPK_MAX_K) return fast + 256;
     return fast + 2 * carve_bytes((size_t)cand_cap, 8) + 2 * carve_bytes((size_t)cand_cap, 4) +
            sx_argsort_workspace_bytes(cand_cap) + 256;
 }
 
-static int topk_check_args(const double *cand_rc, const int64_t *cand_id, int64_t cand_cap,
-                           const sx_select_state *sel, const sx_price_header *header, int64_t K,
-                           const double *out_rc, const int64_t *out_id, const int64_t *out_n, const void *ws,
-                           size_t ws_bytes) {
-    if (K <= 0 || cand_cap < 0 || !sel || !header || !out_rc || !out_id || !out_n) return SX_ERR_INVALID;
-    if (cand_cap > 0 && (!cand_rc || !cand_id)) return SX_ERR_INVALID;
-    if (!ws || ws_bytes < sx_topk_workspace_bytes(cand_cap, K)) return SX_ERR_WORKSPACE;
-    return SX_OK;
-}
-
-extern "C" int sx_topk_select_sorted(const double *cand_rc, const int64_t *cand_id, int64_t cand_cap,
-                                     sx_select_state *sel, sx_price_header *header, int64_t K, double *out_rc,
-                                     int64_t *out_id, int64_t *out_n, void *ws, size_t ws_bytes, void *stream) {
-    int arg = topk_check_args(cand_rc, cand_id, cand_cap, sel, header, K, out_rc, out_id, out_n, ws, ws_bytes);
-    if (arg != SX_OK) return arg;
-    cudaStream_t st = (cudaStream_t)stream;
-    const unsigned long long *n_cand_dev = &((const SelState *)sel)->n_cand;
-    Carver cv(ws);
-    cv.take<KeyId>(kSurvCap);
-    cv.take<KeyId>(cand_cap > 0 ? cand_cap : 1);
-    cv.take<KeyId>(cand_cap > 0 ? cand_cap : 1);
-    if (K <= SX_TOPK_MAX_K) {
-        const int L = (int)((cand_cap + kTkSlice - 1) / kTkSlice);
-        if (L == 0) {
-            topk_fill_kernel<<<(int)((K + 255) / 256), 256, 0, st>>>(out_rc, (long long *)out_id, (long long *)out_n, (int)K);
-            SX_LAUNCH_CHECK();
-            return SX_OK;
-        }
-        double *lists_rc = cv.take<double>((size_t)(L + 1) * K);
-        long long *lists_id = cv.take<long long>((size_t)(L + 1) * K);
-        const size_t smem = sizeof(Cand) * kTkSlice;
-        SX_CUDA(cudaFuncSetAttribute(topk_slice_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        topk_slice_sort_kernel<<<L, kTkThreads, smem, st>>>(cand_rc, (const long long *)cand_id, n_cand_dev, cand_cap,
-                                                            (int)K, lists_rc, lists_id);
-        SX_LAUNCH_CHECK();
-        int *plen = cv.take<int>(L + 2), *poff = cv.take<int>(L + 2);
-        topk_prep_kernel<<<1, 1024, 0, st>>>(lists_rc, lists_id, K, L, (int)K, n_cand_dev, cand_cap, plen, poff, out_rc,
-                                             (long long *)out_id, (long long *)out_n, nullptr, nullptr);
-        SX_LAUNCH_CHECK();
-        topk_rank_kernel<<<num_sms() * 4, 256, 0, st>>>(lists_rc, lists_id, K, L, (int)K, plen, poff, out_rc,
-                                                      (long long *)out_id);
-        SX_LAUNCH_CHECK();
-        return SX_OK;
-    }
-    // large K: the candidate count is needed on the host to size the sorts (one stream sync)
+// K > SX_TOPK_MAX_K: two stable radix argsorts over the candidates, by id, then by rc.  The candidate count
+// is needed on the host to size the sorts (one stream synchronisation).  cv continues after the buffers of
+// the K <= SX_TOPK_MAX_K selection.
+static int topk_select_large_k(const double *cand_rc, const int64_t *cand_id, int64_t cand_cap, const SelState *sel,
+                               int64_t K, double *out_rc, int64_t *out_id, int64_t *out_n, Carver &cv,
+                               size_t ws_bytes, cudaStream_t st) {
     unsigned long long n64 = 0;
-    SX_CUDA(cudaMemcpyAsync(&n64, n_cand_dev, sizeof(n64), cudaMemcpyDeviceToHost, st));
+    SX_CUDA(cudaMemcpyAsync(&n64, &sel->n_cand, sizeof(n64), cudaMemcpyDeviceToHost, st));
     SX_CUDA(cudaStreamSynchronize(st));
     const long long n = n64 > (unsigned long long)cand_cap ? cand_cap : (long long)n64;
     double *rc1 = cv.take<double>(cand_cap);
@@ -892,18 +751,18 @@ extern "C" int sx_topk_select_sorted(const double *cand_rc, const int64_t *cand_
 extern "C" int sx_topk_select(const double *cand_rc, const int64_t *cand_id, int64_t cand_cap,
                               sx_select_state *sel, sx_price_header *header, int64_t K, double *out_rc,
                               int64_t *out_id, int64_t *out_n, void *ws, size_t ws_bytes, void *stream) {
-    if (K > SX_TOPK_MAX_K)
-        return sx_topk_select_sorted(cand_rc, cand_id, cand_cap, sel, header, K, out_rc, out_id, out_n, ws, ws_bytes,
-                                     stream);
-    int arg = topk_check_args(cand_rc, cand_id, cand_cap, sel, header, K, out_rc, out_id, out_n, ws, ws_bytes);
-    if (arg != SX_OK) return arg;
+    if (K <= 0 || cand_cap < 0 || !sel || !header || !out_rc || !out_id || !out_n) return SX_ERR_INVALID;
+    if (cand_cap > 0 && (!cand_rc || !cand_id)) return SX_ERR_INVALID;
+    if (!ws || ws_bytes < sx_topk_workspace_bytes(cand_cap, K)) return SX_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
+    SelState *sst = (SelState *)sel;
     Carver cv(ws);
     KeyId *sure = cv.take<KeyId>(kSurvCap);
     KeyId *listA = cv.take<KeyId>(cand_cap > 0 ? cand_cap : 1);
     KeyId *listB = cv.take<KeyId>(cand_cap > 0 ? cand_cap : 1);
+    if (K > SX_TOPK_MAX_K)
+        return topk_select_large_k(cand_rc, cand_id, cand_cap, sst, K, out_rc, out_id, out_n, cv, ws_bytes, st);
     const long long *cid = (const long long *)cand_id;
-    SelState *sst = (SelState *)sel;
     int Ki = (int)K;
     long long *oid = (long long *)out_id, *on = (long long *)out_n;
     void *args[] = {(void *)&cand_rc, (void *)&cid, (void *)&cand_cap, (void *)&sst, (void *)&header, (void *)&Ki,
@@ -944,8 +803,8 @@ extern "C" int sx_topk_merge(const double *blocks_rc, const int64_t *blocks_id, 
     }
     Carver cv(ws);
     int *plen = cv.take<int>(G + 2), *poff = cv.take<int>(G + 2);
-    topk_prep_kernel<<<1, 1024, 0, st>>>(blocks_rc, (const long long *)blocks_id, block_stride, (int)G, (int)K, nullptr,
-                                         0, plen, poff, out_rc, (long long *)out_id, (long long *)out_n,
+    topk_prep_kernel<<<1, 1024, 0, st>>>(blocks_rc, (const long long *)blocks_id, block_stride, (int)G, (int)K, plen,
+                                         poff, out_rc, (long long *)out_id, (long long *)out_n,
                                          (const long long *)headers, (long long *)out_summary);
     SX_LAUNCH_CHECK();
     topk_rank_kernel<<<num_sms() * 2, 256, 0, st>>>(blocks_rc, (const long long *)blocks_id, block_stride, (int)G, (int)K,

@@ -18,12 +18,12 @@ SX_PLUS_IS_HEAD = 0
 SX_PLUS_IS_TAIL = 1
 SX_TOPK_MAX_K = 1024
 SX_STATUS_CAND_OVERFLOW = 1
-SX_STATUS_NEED_SORTED = 2
+SX_STATUS_DUPLICATE_CANDIDATES = 2
 SX_STATUS_K_MISMATCH = 4
 SX_STATUS_NAN_RC = 8
 SX_STATUS_NEED_UNFUSED = 16
-SX_STATUS_REPEAT_MASK = 19
-SX_ABI_VERSION = 4
+SX_STATUS_REPEAT_MASK = 17
+SX_ABI_VERSION = 5
 
 
 class SxError(RuntimeError):
@@ -95,7 +95,6 @@ SIGNATURES = {
                                        _p, _int, _int, _p, _p, _p, _sz, _p]),
     "sx_topk_workspace_bytes": (_sz, [_i64, _i64]),
     "sx_topk_select": (_int, [_p, _p, _i64, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
-    "sx_topk_select_sorted": (_int, [_p, _p, _i64, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
     "sx_topk_merge_workspace_bytes": (_sz, [_i64]),
     "sx_topk_merge": (_int, [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _p, _i64, _p, _sz, _p]),
     "sx_exchange_buffer_bytes": (_sz, [_i64, _int]),

@@ -290,36 +290,26 @@ class Pricer:
               "sx_price_arcs")
         self.launches += 1
 
-    def select(self, sorted_path: bool = False):
-        """Enqueue the top-K selection over the candidates (device only).  `sorted_path` forces the
-        slice-sort selection, which the fast one asks for through SX_STATUS_NEED_SORTED."""
+    def select(self):
+        """Enqueue the top-K selection over the candidates (device only)."""
         if self.K > 0:
-            fn = lib.sx_topk_select_sorted if sorted_path else lib.sx_topk_select
-            check(fn(_ptr(self.cand_rc), _ptr(self.cand_id), self.cap, _ptr(self.sel), _ptr(self.header),
-                     self.K, _ptr(self.out_rc), _ptr(self.out_id), _ptr(self.out_n),
-                     _ptr(self.ws), self.ws.numel(), _stream()), "sx_topk_select")
-            if self.K > _native.SX_TOPK_MAX_K:
-                self.launches += 6
-            else:
-                self.launches += 3 if sorted_path else 2
+            check(lib.sx_topk_select(_ptr(self.cand_rc), _ptr(self.cand_id), self.cap, _ptr(self.sel),
+                                     _ptr(self.header), self.K, _ptr(self.out_rc), _ptr(self.out_id),
+                                     _ptr(self.out_n), _ptr(self.ws), self.ws.numel(), _stream()), "sx_topk_select")
+            self.launches += 6 if self.K > _native.SX_TOPK_MAX_K else 2
 
     def fetch(self) -> PriceResult:
-        """Device -> pinned host copy of the block (top-K + header + count); one synchronisation.
-        Runs the sorted selection and reads again if the fast one asked for it."""
-        while True:
-            self.h_block.copy_(self.block, non_blocking=True)
-            torch.cuda.current_stream().synchronize()
-            h = self.h_block.numpy()
-            Kp = self.Kp
-            self.status = int(h[2 * Kp + 3])
-            if self.status & _native.SX_STATUS_K_MISMATCH:
-                raise ValueError("top-k selection asked for more arcs than the pricing pass was started for")
-            if self.K > 0 and (self.status & _native.SX_STATUS_NEED_SORTED) \
-                    and not (self.status & _native.SX_STATUS_CAND_OVERFLOW):
-                self.header[3:4].zero_()
-                self.select(sorted_path=True)
-                continue
-            break
+        """Device -> pinned host copy of the block (top-K + header + count); one synchronisation."""
+        self.h_block.copy_(self.block, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+        h = self.h_block.numpy()
+        Kp = self.Kp
+        self.status = int(h[2 * Kp + 3])
+        if self.status & _native.SX_STATUS_K_MISMATCH:
+            raise ValueError("top-k selection asked for more arcs than the pricing pass was started for")
+        if self.status & _native.SX_STATUS_DUPLICATE_CANDIDATES:
+            raise ValueError("top-k selection found one arc priced into the pass many times: "
+                             "a pass must price every arc at most once")
         nviol = int(h[2 * Kp]) & 0xFFFFFFFFFFFFFFFF
         min_rc = float(lib.sx_key_to_f64(int(h[2 * Kp + 1])))
         k = int(h[2 * Kp + 4]) if self.K > 0 else 0

@@ -141,8 +141,7 @@ class ShardedDensePricer:
         return self.pricer.launches + self._merge_launches + self._replayed_launches - self._capture_overcount
 
     # -- device-only step: everything stays on the GPU(s) --------------------------------------
-    def enqueue(self, y_dev: torch.Tensor, kernel_events=None, sorted_path: bool = False, stage_events=None,
-                y_parts=None, unfused: bool = False):
+    def enqueue(self, y_dev: torch.Tensor, kernel_events=None, stage_events=None, y_parts=None, unfused: bool = False):
         """Enqueue one pricing pass; returns device tensors
         (rc[K], id[K], n_out, count, min key, largest per-rank count, status).  A non-zero status
         (SX_STATUS_*) means the pass must be repeated (`price` does that).  `kernel_events` =
@@ -154,7 +153,7 @@ class ShardedDensePricer:
         y_src, y_dst = y_parts if y_parts is not None else (y_dev[self.row0:self.row0 + self.S_loc],
                                                               y_dev[self.S:self.S + self.D])
         mark = (lambda i: stage_events[i].record()) if stage_events is not None else (lambda i: None)
-        fused = self.fused and not sorted_path and not unfused
+        fused = self.fused and not unfused
         mark(0)
         if fused:
             # ONE launch: state clear of the next pass, pricing, selection and (exchange "ll") the push of the
@@ -180,7 +179,7 @@ class ShardedDensePricer:
             if kernel_events is not None:
                 kernel_events[1].record()
             mark(1)
-            p.select(sorted_path=sorted_path)
+            p.select()
         mark(2)
         Kp = max(self.K, 1)
         if self.world == 1:
@@ -226,13 +225,12 @@ class ShardedDensePricer:
         return self._m_rc, self._m_id, self._m_n[0], self._m_sum[0], self._m_sum[1], self._m_sum[2], self._m_sum[3]
 
     # -- host-facing call: duals in, (count, min, top-K) out --------------------------------------
-    def _step(self, sorted_path: bool = False, unfused: bool = False):
+    def _step(self, unfused: bool = False):
         """H2D of the duals this rank needs (its rows + every sink), one pass, D2H of the result."""
         r0 = self.row0                                             # y_loc = [this rank's S_loc source duals | D sink duals]
         self.y_loc[:self.S_loc].copy_(self.h_y[r0:r0 + self.S_loc], non_blocking=True)
         self.y_loc[self.S_loc:].copy_(self.h_y[self.S:], non_blocking=True)
-        self.enqueue(None, sorted_path=sorted_path, y_parts=(self.y_loc[:self.S_loc], self.y_loc[self.S_loc:]),
-                     unfused=unfused)
+        self.enqueue(None, y_parts=(self.y_loc[:self.S_loc], self.y_loc[self.S_loc:]), unfused=unfused)
         if self.world == 1:
             self.pricer.h_block.copy_(self.pricer.block, non_blocking=True)
         else:
@@ -303,7 +301,7 @@ class ShardedDensePricer:
         if self._dead:
             raise RuntimeError("this pricer saw a peer-exchange timeout; its epoch counters may be out of step with "
                                "the peers': build a new one")
-        sorted_path, unfused = False, False
+        unfused = False
         first = True
         while True:
             if first and self._graph is not None:
@@ -312,20 +310,18 @@ class ShardedDensePricer:
                 if self.fused:
                     self.pricer.note_replayed_fused_passes(1)
             else:
-                self._step(sorted_path=sorted_path, unfused=unfused)
+                self._step(unfused=unfused)
             first = False
             torch.cuda.current_stream().synchronize()
             res, status, cmax = self._read_result()
             # Every rank reads the same folded status, so all ranks repeat the pass together: with a larger
-            # candidate buffer after an overflow, with the sorted selection after SX_STATUS_NEED_SORTED.
+            # candidate buffer after an overflow, with the separate kernels after SX_STATUS_NEED_UNFUSED.
             res.status = status
             if self.K == 0 or (status & _native.SX_STATUS_REPEAT_MASK) == 0:
                 return res
             if status & _native.SX_STATUS_CAND_OVERFLOW:
                 self.pricer.grow(cmax)
                 self._graph, self._capture_tried = None, False      # buffers moved: record again next time
-            elif status & _native.SX_STATUS_NEED_SORTED:
-                sorted_path = True
             else:                                                   # SX_STATUS_NEED_UNFUSED: the separate kernels refine
                 unfused = True
 

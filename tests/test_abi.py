@@ -23,8 +23,7 @@ def test_header_declares_the_expected_entry_points():
     names = _declared()
     for must in ("sx_score_ot", "sx_score_mcf", "sx_argsort_f64", "sx_kruskal_order", "sx_kruskal",
                  "sx_tree_potentials", "sx_price_pass_begin", "sx_price_dense_ot", "sx_price_arcs", "sx_topk_select",
-                 "sx_topk_select_sorted", "sx_exchange_blocks",
-                 "sx_topk_merge", "sx_price_dense_ot_h"):
+                 "sx_exchange_blocks", "sx_topk_merge", "sx_price_dense_ot_h"):
         assert must in names
     assert len(names) >= 24
 
@@ -35,7 +34,7 @@ def test_library_exports_every_declared_symbol():
     for name in _declared():
         assert hasattr(lib, name), f"{name} declared in sxcross.h but not exported"
     lib.sx_abi_version.restype = ctypes.c_int
-    assert lib.sx_abi_version() == 4
+    assert lib.sx_abi_version() == 5
     lib.sx_error_string.restype = ctypes.c_char_p
     assert b"spanning" in lib.sx_error_string(-5)
 

@@ -504,7 +504,7 @@ def test_price_many_violators_are_pruned(dev, fused_mode, frac, K):
 
 def test_price_all_equal_reduced_costs(dev, fused_mode):
     """Every arc has the same reduced cost: no bound can prune and 60 000 candidates tie at the K-th
-    value; the selection refines on the arc id (ids win ties).  The sorted path gives the same."""
+    value; the selection refines on the arc id (ids win ties)."""
     S, D, K = 300, 200, 100
     M = np.full((S, D), 2.0)
     y = np.concatenate([np.zeros(S), np.full(D, 3.0)])            # rc = -1 everywhere
@@ -513,11 +513,51 @@ def test_price_all_equal_reduced_costs(dev, fused_mode):
     assert res.n_violating == S * D and res.min_rc == -1.0
     assert np.array_equal(res.topk_id, np.arange(K)) and np.all(res.topk_rc == -1.0)
     assert pr.status == 0
+
+
+@pytest.mark.parametrize("K", [501, 1024])
+def test_selection_refines_key_and_large_ids_within_the_level_bound(dev, K):
+    """The boundary bin holds 100 000 exact ties at rank K plus a few thousand near-ties that differ from
+    them only in low mantissa bits, and the arc ids straddle 2^62: the selection has to refine on the key
+    first, then on the high and low bits of the id, and still finishes with the exact top K."""
+    rng = np.random.default_rng(K)
+    tie = -(1.0 + 2.0 ** -9 + 12345 * 2.0 ** -52)                 # middle of its 0.4 %-wide histogram bin
+    rc = np.concatenate([
+        -3.0 + rng.random(500),                                   # the 500 best arcs, in lower bins
+        np.full(100_000, tie),                                    # rank K falls inside this tie
+        tie + rng.integers(1, 12345, 3000) * 2.0 ** -52,          # same bin as the tie, above it in the low bits
+        tie + rng.integers(1 << 30, 1 << 40, 3000) * 2.0 ** -52,  # same bin, higher key bits
+        rng.random(2000)])                                        # not violating
+    rc = rc[rng.permutation(rc.size)]
+    id0 = 2 ** 62 - 50_000
+    n_nodes = 64
+    tail = rng.integers(0, n_nodes, rc.size).astype(np.int32)
+    head = rng.integers(0, n_nodes, rc.size).astype(np.int32)
+    y = np.zeros(n_nodes)                                         # rc = c - (0 - 0) = c exactly
+    cnt, mn, ids, vals = orc.price_summary(rc, K=K)
+    assert vals[499] < tie == vals[500] == vals[-1]                 # rank K lies inside the tie
+    pr = dev.Pricer(torch.device("cuda"), K)
     pr.reset()
-    pr.price_dense(cu(M), D, 0, S, D, cu(y[:S]), cu(y[S:]))
-    pr.select(sorted_path=True)
-    alt = pr.fetch()
-    assert np.array_equal(alt.topk_id, np.arange(K)) and alt.n_violating == S * D
+    pr.price_arcs(cu(rc), cu(tail), cu(head), None, cu(y), id0=id0)
+    pr.select()
+    res = pr.fetch()
+    assert pr.status == 0 and res.n_violating == cnt
+    assert np.array_equal(res.topk_id, ids + id0) and res.topk_rc.tobytes() == vals.tobytes()
+
+
+def test_selection_flags_an_arc_priced_into_one_pass_many_times(dev):
+    """A pass that prices the same arc 8 300 times leaves more copies of one (rc, id) than the selection can
+    rank: the result is void, SX_STATUS_DUPLICATE_CANDIDATES is raised and `fetch` refuses it."""
+    from smart_crossover import _native
+    pr = dev.Pricer(torch.device("cuda"), 16)
+    c, tail, head, y = cu(np.array([-1.0])), cu(np.array([0], np.int32)), cu(np.array([1], np.int32)), cu(np.zeros(2))
+    pr.reset()
+    for _ in range(8300):
+        pr.price_arcs(c, tail, head, None, y)
+    pr.select()
+    with pytest.raises(ValueError):
+        pr.fetch()
+    assert pr.status & _native.SX_STATUS_DUPLICATE_CANDIDATES
 
 
 def test_price_near_ties_at_the_kth_value(dev, fused_mode):
@@ -616,6 +656,42 @@ def test_price_row_slabs_and_merge(dev):
     assert total == whole.n_violating
     assert np.array_equal(out_id[:k].cpu().numpy(), whole.topk_id)
     assert np.array_equal(out_rc[:k].cpu().numpy(), whole.topk_rc)
+
+
+def test_topk_merge_above_the_one_thread_per_element_size(dev):
+    """sx_topk_merge with G * K > 2^22 (5 blocks of 2^20, 84 MB as an all-gathered (G, 2K + 4) buffer) runs the
+    prefix bound + rank merge.  Sorted, padded blocks with many rc ties, tails of padding and one block that is
+    all padding, against a NumPy lexsort of all real entries; the pricing headers fold into the summary."""
+    G, K = 5, 1 << 20
+    rng = np.random.default_rng(2024)
+    for n_real in ([K, K - 12345, 0, K // 3, 777], [1000, 0, 0, 5000, 3]):
+        ids_all = rng.permutation(sum(n_real)).astype(np.int64) * 3 + 7      # distinct across blocks
+        buf = np.zeros((G, 2 * K + 4), dtype=np.int64)
+        rc_real, id_real, off = [], [], 0
+        for g, n in enumerate(n_real):
+            rc = -1.0 - np.round(rng.random(n) * 1000) / 1000                # about a thousand distinct values
+            ids = ids_all[off:off + n]
+            off += n
+            o = np.lexsort((ids, rc))
+            buf[g, :K] = np.float64(np.inf).view(np.int64)
+            buf[g, K:2 * K] = -1
+            buf[g, :n] = rc[o].view(np.int64)
+            buf[g, K:K + n] = ids[o]
+            buf[g, 2 * K:] = [n, rng.integers(-1000, 1000), 0, 8 * (g == 1)]  # n_violating, min key, -, status
+            rc_real.append(rc)
+            id_real.append(ids)
+        rc_real, id_real = np.concatenate(rc_real), np.concatenate(id_real)
+        o = np.lexsort((id_real, rc_real))[:K]
+        gathered = cu(buf)
+        out_rc, out_id, out_n, summary = dev.topk_merge(gathered[:, :K].view(torch.float64), gathered[:, K:2 * K],
+                                                        gathered[:, 2 * K:])
+        k = int(out_n.item())
+        assert k == o.size
+        assert np.array_equal(out_id[:k].cpu().numpy(), id_real[o])
+        assert out_rc[:k].cpu().numpy().tobytes() == rc_real[o].tobytes()
+        assert np.all(out_id[k:].cpu().numpy() == -1) and np.all(np.isinf(out_rc[k:].cpu().numpy()))
+        hdr = buf[:, 2 * K:]
+        assert summary.cpu().numpy().tolist() == [int(hdr[:, 0].sum()), int(hdr[:, 1].min()), int(hdr[:, 0].max()), 8]
 
 
 @pytest.mark.parametrize("G,K", [(2, 128), (8, 1024), (5, 33)])
