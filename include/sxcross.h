@@ -54,7 +54,7 @@ extern "C" {
 #define SX_ERR_PEER_TIMEOUT    -8   /* sx_exchange_blocks: a peer never raised its flag */
 #define SX_ERR_PUSH_ASSERT     -9   /* sx_push_tree_h: the reference's assertions would fire (tree_BI.py:93-94) */
 
-#define SX_ABI_VERSION 5
+#define SX_ABI_VERSION 6
 
 /* Endpoint convention of sx_tree_potentials (which end of an arc carries +1 in A). */
 #define SX_PLUS_IS_HEAD 0   /* OT:  A[S+j,k] = +1, A[i,k] = -1      (formats.py:156-158)     */
@@ -78,10 +78,7 @@ typedef struct sx_price_header {
                                         selected (NumPy: NaN < -tol is False), but the optimality test
                                         `np.all(rc >= -tol)` (net_manager.py:318,496) is False: callers must
                                         treat the pass as NOT optimal.  Informational, no repeat needed. */
-#define SX_STATUS_NEED_UNFUSED  16   /* sx_price_dense_ot_fused could not finish its selection (more than 4096
-                                        candidates tie around the K-th value): run the pass again with
-                                        sx_price_pass_begin / sx_price_dense_ot / sx_topk_select */
-#define SX_STATUS_REPEAT_MASK   17   /* bits that ask for the pass to be repeated */
+#define SX_STATUS_REPEAT_MASK    1   /* bits that ask for the pass to be repeated */
 
 /* Selection state of a pricing pass (opaque device memory, sx_select_state_bytes() bytes, 16 B
  * aligned): candidate counter, pruning bound and the reduced-cost histogram the bound is derived
@@ -284,14 +281,14 @@ SX_API int    sx_price_set_tma_options(int l2_promotion, int evict_first);
  *     multi-GPU pass is one launch per GPU: [K rc bits | K ids | n_out | total n_violating, min key,
  *     largest single n_violating, OR of the status words]; status_dev receives SX_ERR_PEER_TIMEOUT if
  *     a peer never shows up.  NULL: follow with sx_topk_merge_ll.
- *   ws: sx_fused_workspace_bytes() bytes.
- * status bits SX_STATUS_CAND_OVERFLOW / SX_STATUS_NEED_UNFUSED ask for a repeat with the separate calls
- * (the block is still well formed and pushed, so no peer waits).  Needs 16 B aligned M and even ld
- * (SX_ERR_UNALIGNED otherwise: use the separate calls).
+ *   ws: sx_topk_workspace_bytes(cand_cap, K) bytes, as sx_topk_select takes.
+ * The selection is the one of sx_topk_select and finishes on any candidate list of distinct arcs.  Status bit
+ * SX_STATUS_CAND_OVERFLOW asks for a larger candidate buffer and a repeat (the block is still well formed and
+ * pushed, so no peer waits).  Needs 16 B aligned M and even ld (SX_ERR_UNALIGNED otherwise: use the separate
+ * calls).
  */
 typedef struct sx_fused_state sx_fused_state;
 SX_API size_t sx_fused_state_bytes(void);
-SX_API size_t sx_fused_workspace_bytes(void);
 /* diagnostics: byte offset inside the state of 8 x uint64 %globaltimer stamps (ns) that CTA 0 of the last
  * pass took at: start, end of its pricing, after barrier 1, after the filter, after barrier 2, after the rank */
 SX_API size_t sx_fused_state_timestamps_offset(void);
@@ -404,7 +401,7 @@ SX_API int    sx_sinkhorn_ot(const double *M, int64_t ld, int64_t S, int64_t D, 
  * sx_ot_pricer_price_h: y_src_h (S source duals) and y_dst_h (D sink duals) are HOST vectors (pageable is
  *   fine: each worker copies its slice into pinned staging); returns count / min / top-K on the host and
  *   (status_h, may be NULL) the SX_STATUS_* bits that survived (SX_STATUS_NAN_RC).  Repeats the pass
- *   internally when the fused kernel asks for it (candidate overflow, ties).
+ *   internally, with a larger candidate buffer, when the candidates overflowed it.
  * sx_ot_pricer_info: device / row range of shard g.  sx_ot_pricer_stats: passes, repeated passes, whether the
  *   fused kernel and the in-kernel merge are in use.
  */

@@ -9,9 +9,11 @@
 //            alternate passes), so no pass ever waits for a clear;
 //   pricing  the TMA pipeline of sx_price_tma.cuh, unchanged: count, min, candidate list + histogram;
 //   barrier  grid-wide (the kernel is launched cooperatively: all CTAs are resident);
-//   filter   only when the candidate list is longer than kFusedDirectCap: every CTA derives the bound b*
-//            from the histogram (one warp, 9 KB of L2 reads) and keeps its share of the candidates with
-//            bin <= b* (the K best plus the rest of one 0.4 %-wide bin); second barrier;
+//   select   select_topk (sx_select.cuh), the selection topk_select_kernel runs too: a candidate list of at
+//            most kDirectCap is ranked as it is; a longer one is first split by the histogram's bound b*
+//            (every CTA derives it: one warp, 9 KB of L2 reads) into the sure candidates and the boundary
+//            list, which radix refinement shortens further only under massive ties at the K-th value;
+//            second barrier;
 //   rank     all-pairs rank of the candidates / survivors spread over the grid (1-32 lanes per element);
 //            the lanes of an element write it to its position in the local result block AND, with G > 1,
 //            store it as flag-in-data slots straight into every peer's exchange buffer (NVLink; sx_ll.cuh),
@@ -20,11 +22,8 @@
 //            out of the local exchange buffer as they land (staging is the wait), rank every element by
 //            G - 1 binary searches in shared memory and write the merged top-K.
 //
-// If too many candidates survive the filter (massive ties at the K-th value) or the candidate buffer
-// overflowed, the pass raises SX_STATUS_NEED_UNFUSED / SX_STATUS_CAND_OVERFLOW in the header -- it still
-// pushes a well-formed (padded) block so that no peer waits -- and the caller repeats the pass with the
-// separate kernels (sx_price_pass_begin / sx_price_dense_ot / sx_topk_select / sx_exchange_push_ll /
-// sx_topk_merge_ll), which own the refinement levels and the sorted fallback.
+// If the candidate buffer overflowed, the pass raises SX_STATUS_CAND_OVERFLOW in the header -- it still
+// pushes a well-formed block so that no peer waits -- and the caller grows the buffer and repeats the pass.
 #include <stdlib.h>
 
 #include "sx_gridbar.cuh"
@@ -33,11 +32,7 @@
 
 namespace sx {
 
-constexpr int kFusedDirectCap = 2048;   // candidate lists up to this length are ranked as they are (the all-pairs
-                                        // rank is quadratic: 6990 candidates took 45 us, the filter path 12)
-constexpr int kFusedSurvCap   = 4096;   // survivors of the filter the in-kernel rank takes (64 KB list)
-constexpr int kFusedTile      = 2048;   // elements staged in shared memory at a time (32 KB)
-constexpr int kMergeCtas      = 64;     // CTAs (from the end of the grid) that merge the G blocks
+constexpr int kMergeCtas = 64;          // CTAs (from the end of the grid) that merge the G blocks
 
 struct FusedCtl {
     unsigned long long pass;      // passes completed; parity selects the selection state in use
@@ -59,7 +54,7 @@ struct FusedParams {
     long long        cand_cap;
     unsigned         K;              // >= 1 (layout); cand_cap == 0 means count / min only
     long long       *block;          // local result block [K rc bits | K ids | header (4) | n_out | pad]
-    KeyId           *surv;           // kFusedSurvCap entries
+    SelLists         lists;          // lists of the selection (workspace of sx_topk_workspace_bytes)
     char *const     *peer_bufs;      // LL exchange buffers of the G ranks, or nullptr (no exchange)
     int              rank, G;
     long long        block_len;
@@ -87,10 +82,10 @@ __device__ __forceinline__ uint4 *ll_slot(char *buf, const FusedParams &f, unsig
 template <int ROWS, int STAGES, int CWARPS, int MINB>
 __global__ void __launch_bounds__((CWARPS + 1) * 32, MINB)
 price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p0, const FusedParams f) {
-    static_assert((size_t)STAGES * ROWS * kBoxCols * sizeof(double) >= (size_t)kFusedTile * sizeof(KeyId),
-                  "the stage ring is reused as the rank tile");
+    static_assert((size_t)STAGES * ROWS * kBoxCols * sizeof(double) >= sizeof(SelScratch),
+                  "the stage ring is reused as the selection's shared memory");
+    static_assert(CWARPS * 32 == kSelThreads, "the consumer warps select, the producer warp joins the barriers");
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ unsigned s_b;
     __shared__ long long s_hdr[4];
     __shared__ int s_real;
     const int tid = threadIdx.x, nthr = blockDim.x;
@@ -139,90 +134,24 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
 
     const unsigned long long n64 = __ldcg(&sel->n_cand);
     const long long n = n64 > (unsigned long long)f.cand_cap ? f.cand_cap : (long long)n64;
-    const bool direct = n <= kFusedDirectCap;
-    bool incomplete = false;
-    int  n_s = (int)n;
-    if (!direct) {
-        // ---- filter: candidates with bin <= b* survive ----
-        if (tid < 32) {
-            const unsigned b = warp_find_bound(sel, f.K, nullptr);
-            if (tid == 0) s_b = b;
-        }
-        __syncthreads();
-        const unsigned b1 = s_b;
-        for (long long base = (long long)blockIdx.x * nthr; base < n; base += (long long)gridDim.x * nthr) {
-            const long long i = base + tid;
-            KeyId v{~0ull, 0x7fffffffffffffffll};
-            bool keep = false;
-            if (i < n) {
-                v.key = f64_to_sort_key(__ldcg(f.cand_rc + i));
-                v.id  = __ldcg(f.cand_id + i);
-                const unsigned long long kb = v.key >> (64 - 1 - kFineBits);            // = cand_bin(rc)
-                keep = (kb < (unsigned long long)kFineBins ? (unsigned)kb : kFineBins - 1u) <= b1;
-            }
-            const unsigned m = __ballot_sync(0xffffffffu, keep);
-            if (m) {
-                unsigned pos = 0;
-                if (lane_id() == 0) pos = atomicAdd(&sel->n_sure, (unsigned)__popc(m));
-                pos = __shfl_sync(0xffffffffu, pos, 0) + __popc(m & ((1u << lane_id()) - 1u));
-                if (keep && pos < (unsigned)kFusedSurvCap)
-                    __stcg(reinterpret_cast<ulonglong2 *>(f.surv + pos), make_ulonglong2(v.key, (unsigned long long)v.id));
-            }
-        }
-        stamp(ctl, 3);
-        grid_barrier(&ctl->bar);      // survivor list complete
-        const unsigned n_s_raw = __ldcg(&sel->n_sure);
-        incomplete = n_s_raw > (unsigned)kFusedSurvCap;
-        n_s = incomplete ? 0 : (int)n_s_raw;
-    } else {
-        stamp(ctl, 3);
-    }
+    // ---- selection; the lanes of an element emit it ----
+    stamp(ctl, 3);        // a list ranked as it is has no second barrier; a longer one stamps 3 and 4 around it
     stamp(ctl, 4);
-    const int n_out = n_s < K ? n_s : K;
-    auto load = [&](int j) -> KeyId {
-        return direct ? KeyId{f64_to_sort_key(__ldcg(f.cand_rc + j)), __ldcg(f.cand_id + j)} : ld_keyid(f.surv + j);
-    };
-
-    // ---- all-pairs rank, spread over the grid; the lanes of an element emit it ----
-    if (n_s > 0) {
-        KeyId *tile = reinterpret_cast<KeyId *>(smem_raw);
-        constexpr int kRankThreads = CWARPS * 32;                  // the producer warp only joins the barriers
-        const int T = gridDim.x * kRankThreads;
-        int L = 32;
-        while (L > 1 && (long long)n_s * L > T) L >>= 1;
-        const int groups = T / L;                                  // elements ranked per sweep of the grid
-        for (int e0 = 0; e0 < n_s; e0 += groups) {
-            const int cta_first = e0 + (blockIdx.x * kRankThreads) / L;
-            if (cta_first >= n_s) break;                           // CTA-uniform
-            const int  e = cta_first + tid / L, sub = tid % L;
-            const bool active = tid < kRankThreads && e < n_s;
-            KeyId mine{~0ull, 0x7fffffffffffffffll};
-            if (active) mine = load(e);
-            int cnt = 0;
-            for (int t0 = 0; t0 < n_s; t0 += kFusedTile) {
-                const int tn = n_s - t0 < kFusedTile ? n_s - t0 : kFusedTile;
-                __syncthreads();
-                for (int j = tid; j < tn; j += nthr) tile[j] = load(t0 + j);
-                __syncthreads();
-                if (active) {
-#pragma unroll 4
-                    for (int j = sub; j < tn; j += L) cnt += keyid_less(tile[j], mine) ? 1 : 0;
+    const SelResult sr = select_topk(
+        f.cand_rc, f.cand_id, n, f.cand_cap, sel, K, f.lists, *reinterpret_cast<SelScratch *>(smem_raw),
+        [ctl] { stamp(ctl, 3); grid_barrier(&ctl->bar); stamp(ctl, 4); },
+        [&](const KeyId &v, int rank, int sub, int L) {
+            if (rank >= K) return;
+            const unsigned long long rc_bits = (unsigned long long)__double_as_longlong(sort_key_to_f64(v.key));
+            if (sub == 0) { f.block[rank] = (long long)rc_bits; f.block[K + rank] = v.id; }
+            if (f.peer_bufs)
+                for (int q = sub; q < f.G; q += L) {
+                    ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, rank), flag, rc_bits);
+                    ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, (long long)K + rank), flag,
+                                  (unsigned long long)v.id);
                 }
-            }
-            if (tid < kRankThreads)
-                for (int o = L >> 1; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-            if (active && cnt < K) {
-                const unsigned long long rc_bits = (unsigned long long)__double_as_longlong(sort_key_to_f64(mine.key));
-                if (sub == 0) { f.block[cnt] = (long long)rc_bits; f.block[K + cnt] = mine.id; }
-                if (f.peer_bufs)
-                    for (int q = sub; q < f.G; q += L) {
-                        ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, cnt), flag, rc_bits);
-                        ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, (long long)K + cnt), flag,
-                                      (unsigned long long)mine.id);
-                    }
-            }
-        }
-    }
+        });
+    const int n_out = sr.n_out;
     stamp(ctl, 5);
 
     // ---- padding, header and count: the last CTA (it rarely has rank work) ----
@@ -243,7 +172,7 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
             if (tid == 2) w = __ldcg(&sel->hdr.n_priced);
             if (tid == 3)
                 w = __ldcg(&sel->hdr.status) | (n64 > (unsigned long long)f.cand_cap ? kStatusCandOverflow : 0ull) |
-                    (incomplete ? kStatusNeedUnfused : 0ull);
+                    (sr.duplicates ? kStatusDuplicateCandidates : 0ull);
             if (tid == 4) w = (unsigned long long)n_out;
             f.block[2 * K + tid] = (long long)w;
             if (f.peer_bufs)
@@ -389,7 +318,6 @@ constexpr int kFRows = 16, kFStages = 3, kFWarps = 8, kFMinB = 2;
 using namespace sx;
 
 extern "C" size_t sx_fused_state_bytes(void) { return sizeof(FusedState); }
-extern "C" size_t sx_fused_workspace_bytes(void) { return (size_t)kFusedSurvCap * sizeof(KeyId); }
 extern "C" size_t sx_fused_state_timestamps_offset(void) { return offsetof(FusedState, ctl) + offsetof(FusedCtl, ts); }
 
 extern "C" int sx_fused_state_init(sx_fused_state *state, int64_t K, void *stream) {
@@ -418,7 +346,7 @@ extern "C" int sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0
     if (peer_bufs_dev && (G < 1 || rank < 0 || rank >= G)) return SX_ERR_INVALID;
     if (merged_out && (!peer_bufs_dev || !status_dev)) return SX_ERR_INVALID;
     if (merged_out && !sx_fused_merge_fits(K, G)) return SX_ERR_TOO_LARGE;
-    if (!ws || ws_bytes < sx_fused_workspace_bytes()) return SX_ERR_WORKSPACE;
+    if (!ws || ws_bytes < sx_topk_workspace_bytes(cand_cap, K)) return SX_ERR_WORKSPACE;
     if (((uintptr_t)M % 16) != 0 || (ld % 2) != 0) return SX_ERR_UNALIGNED;
     if (D >= (1ll << 31) || S_loc >= (1ll << 31)) return SX_ERR_TOO_LARGE;
     cudaStream_t st = (cudaStream_t)stream;
@@ -436,7 +364,8 @@ extern "C" int sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0
 
     FusedParams f;
     f.state = (FusedState *)state; f.cand_rc = cand_rc; f.cand_id = (const long long *)cand_id; f.cand_cap = cand_cap;
-    f.K = (unsigned)K; f.block = (long long *)block; f.surv = (KeyId *)ws;
+    Carver cv(ws);
+    f.K = (unsigned)K; f.block = (long long *)block; f.lists = carve_sel_lists(cv, cand_cap);
     f.peer_bufs = (char *const *)peer_bufs_dev; f.rank = rank; f.G = peer_bufs_dev ? G : 1; f.block_len = block_len;
     f.merged = (long long *)merged_out; f.xstatus = (int *)status_dev; f.timeout_ns = 10ull * 1000 * 1000 * 1000;
     static int steal = -1;

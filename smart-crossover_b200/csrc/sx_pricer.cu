@@ -26,7 +26,6 @@ namespace {
 
 using namespace sx;
 
-enum Mode { kFused = 0, kSeparate = 1 };
 enum Cmd { kIdle = 0, kPrice = 1, kGrow = 2, kQuit = 3 };
 
 struct DevCtx {
@@ -37,7 +36,7 @@ struct DevCtx {
     double *y_loc = nullptr;
     double *cand_rc = nullptr;
     int64_t *cand_id = nullptr;
-    void *fstate = nullptr, *fws = nullptr, *sel = nullptr, *topk_ws = nullptr;
+    void *fstate = nullptr, *sel = nullptr, *topk_ws = nullptr;
     size_t topk_ws_bytes = 0;
     int64_t *block = nullptr, *merged = nullptr;
     char *ll_buf = nullptr;
@@ -63,7 +62,6 @@ struct sx_ot_pricer {
     std::vector<DevCtx *> ctx;
     // arguments of the pass in flight (read by the workers)
     const double *y_src_h = nullptr, *y_dst_h = nullptr;
-    int mode = kFused;
     int64_t new_cap = 0;
     unsigned long long passes = 0, repeats = 0;
 };
@@ -109,12 +107,12 @@ int run_pass(sx_ot_pricer *p, DevCtx *c) {
     }
     const int64_t cap = p->K > 0 ? p->cap : 0;
     int32_t *xstatus = reinterpret_cast<int32_t *>(c->merged + 2 * Kp + 5);
-    if (p->mode == kFused) {
+    if (p->fusable) {
         SXP(sx_price_dense_ot_fused(c->M, p->ld, c->row0, c->S_loc, D, c->y_loc, c->y_loc + c->S_loc, p->tol,
                                     (sx_fused_state *)c->fstate, c->cand_rc, c->cand_id, cap, Kp, c->block, p->blk,
                                     p->G > 1 ? c->peer_bufs_dev : nullptr, c->g, p->G,
-                                    (p->G > 1 && p->merge_in_kernel) ? c->merged : nullptr, xstatus, c->fws,
-                                    sx_fused_workspace_bytes(), c->st));
+                                    (p->G > 1 && p->merge_in_kernel) ? c->merged : nullptr, xstatus, c->topk_ws,
+                                    c->topk_ws_bytes, c->st));
     } else {
         sx_price_header *hdr = reinterpret_cast<sx_price_header *>(c->block + 2 * Kp);
         SXP(sx_price_pass_begin(hdr, (sx_select_state *)c->sel, p->K, c->st));
@@ -126,7 +124,7 @@ int run_pass(sx_ot_pricer *p, DevCtx *c) {
         }
         if (p->G > 1) SXP(sx_exchange_push_ll(c->block, p->blk, c->peer_bufs_dev, c->g, p->G, c->st));
     }
-    if (p->G > 1 && !(p->mode == kFused && p->merge_in_kernel))
+    if (p->G > 1 && !(p->fusable && p->merge_in_kernel))
         SXP(sx_topk_merge_ll(c->ll_buf, p->blk, p->G, Kp, (double *)c->merged, c->merged + Kp, c->merged + 2 * Kp,
                              c->merged + 2 * Kp + 1, xstatus, c->st));
     SX_CUDA(cudaMemcpyAsync(c->h_out, p->G > 1 ? c->merged : c->block, (size_t)p->blk * 8, cudaMemcpyDeviceToHost, c->st));
@@ -203,8 +201,8 @@ int run_all(sx_ot_pricer *p, int cmd) {
 void free_ctx(DevCtx *c) {
     cudaSetDevice(c->dev);
     if (c->st) cudaStreamSynchronize(c->st);
-    void *dev_ptrs[] = {c->y_loc, c->cand_rc, c->cand_id, c->fstate, c->fws, c->sel, c->topk_ws, c->block, c->merged,
-                        c->ll_buf, c->peer_bufs_dev};
+    void *dev_ptrs[] = {c->y_loc, c->cand_rc, c->cand_id, c->fstate, c->sel, c->topk_ws, c->block, c->merged, c->ll_buf,
+                        c->peer_bufs_dev};
     for (void *q : dev_ptrs) if (q) cudaFree(q);
     if (c->h_y) cudaFreeHost(c->h_y);
     if (c->h_out) cudaFreeHost(c->h_out);
@@ -286,7 +284,6 @@ extern "C" int sx_ot_pricer_create(int ndev, const int *devs, const double *cons
         if ((rc = alloc_candidates(p, c, p->cap)) != SX_OK) return fail(rc);
         if (p->fusable) {
             SXA(cudaMalloc(&c->fstate, sx_fused_state_bytes()));
-            SXA(cudaMalloc(&c->fws, sx_fused_workspace_bytes()));
             if ((rc = sx_fused_state_init((sx_fused_state *)c->fstate, Kp, c->st)) != SX_OK) return fail(rc);
         }
         if (ndev > 1) {
@@ -330,7 +327,6 @@ extern "C" int sx_ot_pricer_price_h(sx_ot_pricer *p, const double *y_src_h, cons
     if (p->dead) return SX_ERR_PEER_TIMEOUT;
     const int64_t Kp = p->Kp;
     p->y_src_h = y_src_h; p->y_dst_h = y_dst_h;
-    p->mode = p->fusable ? kFused : kSeparate;
     ++p->passes;
     unsigned long long status = 0, count = 0, cmax = 0;
     long long min_key = 0;
@@ -348,19 +344,16 @@ extern "C" int sx_ot_pricer_price_h(sx_ot_pricer *p, const double *y_src_h, cons
             count = (unsigned long long)h[2 * Kp]; min_key = h[2 * Kp + 1]; status = (unsigned long long)h[2 * Kp + 3];
             n_out = h[2 * Kp + 4]; cmax = count;
         }
-        if (p->K == 0 || (status & SX_STATUS_REPEAT_MASK) == 0) break;
+        if (p->K == 0 || (status & SX_STATUS_CAND_OVERFLOW) == 0) break;
+        // the candidate buffer overflowed on some device: every device grows it and prices again
         ++p->repeats;
-        if (status & SX_STATUS_CAND_OVERFLOW) {
-            if (p->cap >= kMaxCap) return SX_ERR_TOO_LARGE;
-            int64_t cap = 4 * p->cap > 1024 ? 4 * p->cap : 1024;
-            if (cap > kMaxCap) cap = kMaxCap;
-            if (cmax && (int64_t)cmax < cap) cap = (int64_t)cmax > 1024 ? (int64_t)cmax : 1024;
-            p->new_cap = cap;
-            SXP(run_all(p, kGrow));
-            p->cap = cap;
-        } else {
-            p->mode = kSeparate;
-        }
+        if (p->cap >= kMaxCap) return SX_ERR_TOO_LARGE;
+        int64_t cap = 4 * p->cap > 1024 ? 4 * p->cap : 1024;
+        if (cap > kMaxCap) cap = kMaxCap;
+        if (cmax && (int64_t)cmax < cap) cap = (int64_t)cmax > 1024 ? (int64_t)cmax : 1024;
+        p->new_cap = cap;
+        SXP(run_all(p, kGrow));
+        p->cap = cap;
     }
     *n_violating_h = count;
     *min_rc_h = min_key_to_f64(min_key);

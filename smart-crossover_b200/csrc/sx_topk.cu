@@ -6,10 +6,11 @@
 // (rc, id) is a strict total order, so the result does not depend on the (unordered)
 // compaction or on how many GPUs priced the matrix.
 //
-// K <= 1024: ONE cooperative launch (topk_select_kernel), no host round trip:
-//   1. filter: the pricing kernels left a histogram of the candidates' reduced costs
-//      (sx_select.cuh); b* = the smallest bin whose cumulative count reaches K.  Candidates
-//      with bin < b* are among the K best, bin b* (0.4 % wide) is the boundary list;
+// K <= 1024: ONE cooperative launch (topk_select_kernel), no host round trip.  It runs select_topk
+// (sx_select.cuh), the same selection the fused pricing pass runs in its own kernel (sx_fused.cu):
+//   1. filter: the pricing kernels left a histogram of the candidates' reduced costs; b* = the
+//      smallest bin whose cumulative count reaches K.  Candidates with bin < b* are among the K
+//      best, bin b* (0.4 % wide) is the boundary list;
 //   2. refine: while the list is too long, an 11-bit digit of (key, id) splits the boundary list
 //      again; a list of distinct (key, id) pairs shrinks to one element within 12 levels;
 //   3. all-pairs rank: every survivor counts the survivors below it; that count is its
@@ -220,134 +221,12 @@ topk_rank_kernel(const double *__restrict__ lists_rc, const long long *__restric
     }
 }
 
-// ---- fast path ----------------------------------------------------------------------------
-constexpr int kApThreads = 256;
-constexpr int kApTile    = 2048;
-constexpr int kRankCap   = 4096;   // refine until sure + boundary fit this; the rank itself takes up to kSurvCap
-
-// All-pairs rank of n elements given by load(e) (padding sorts last).  Every thread of the grid
-// takes part; L = 1..32 lanes share one element and split the comparison range.  emit(e, rank)
-// is called once per real element.  Needs n <= gridDim.x * kApThreads.
-template <class LoadFn, class EmitFn>
-__device__ __forceinline__ void all_pairs_rank(int n, LoadFn load, EmitFn emit) {
-    __shared__ KeyId tile[kApTile];
-    const int T = gridDim.x * kApThreads;
-    int L = 32;
-    while (L > 1 && (long long)n * L > T) L >>= 1;
-    const int gtid = blockIdx.x * kApThreads + threadIdx.x;
-    const int e = gtid / L, sub = gtid % L;
-    if ((blockIdx.x * kApThreads) / L >= n) return;            // CTA-uniform: nothing to rank here
-    KeyId mine{~0ull, 0x7fffffffffffffffll};
-    const bool real = e < n;
-    if (real) mine = load(e);
-    const bool valid = real && mine.key != ~0ull;
-    int cnt = 0;
-    for (int t0 = 0; t0 < n; t0 += kApTile) {
-        const int tn = n - t0 < kApTile ? n - t0 : kApTile;
-        __syncthreads();
-        for (int j = threadIdx.x; j < tn; j += kApThreads) tile[j] = load(t0 + j);
-        __syncthreads();
-        if (valid) {
-#pragma unroll 4
-            for (int j = sub; j < tn; j += L) cnt += keyid_less(tile[j], mine) ? 1 : 0;
-        }
-    }
-    for (int o = L >> 1; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-    if (valid && sub == 0) emit(e, cnt);
-}
-
-template <class T> __device__ __forceinline__ T warp_max(T v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        T w = __shfl_xor_sync(0xffffffffu, v, o);
-        v = w > v ? w : v;
-    }
-    return v;
-}
-
-// One partition step of the selection, executed by the whole grid: every element e of this CTA's
-// strided share is classified by cls(e) -> 0 (sure), 1 (new boundary list) or 2 (dropped) and
-// moved to the end of `sure` / into `bnd`.  Counts are aggregated per CTA (one atomicAdd per list
-// and CTA, one set of range atomics per CTA): the classification runs twice, first to count, then
-// to scatter.  Also tracks the (key, id) range of the new boundary list for the next level.
-template <class LoadFn, class ClsFn>
-__device__ __forceinline__ void partition_step(long long n, LoadFn load, ClsFn cls, KeyId *sure, unsigned *n_sure,
-                                               KeyId *bnd, unsigned *n_bnd, long long bnd_cap, SelState *st,
-                                               int next_level, unsigned *s_scan /* 2 * 8 + 2 words */,
-                                               unsigned long long *s_range /* 8 * 4 */) {
-    const long long gtid = (long long)blockIdx.x * kApThreads + threadIdx.x;
-    const long long gsz = (long long)gridDim.x * kApThreads;
-    const int lane = lane_id(), warp = threadIdx.x >> 5;
-    unsigned c0 = 0, c1 = 0;
-    unsigned long long a = 0, b = 0, c = 0, d = 0;      // ~min key, max key, ~min id, max id
-    for (long long i = gtid; i < n; i += gsz) {
-        const KeyId v = load(i);
-        const int k = cls(v);
-        c0 += k == 0;
-        if (k == 1) {
-            ++c1;
-            const unsigned long long id = (unsigned long long)v.id;
-            a = ~v.key > a ? ~v.key : a; b = v.key > b ? v.key : b;
-            c = ~id > c ? ~id : c;       d = id > d ? id : d;
-        }
-    }
-    // block-exclusive scan of (c0, c1)
-    unsigned i0 = c0, i1 = c1;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const unsigned t0 = __shfl_up_sync(0xffffffffu, i0, o), t1 = __shfl_up_sync(0xffffffffu, i1, o);
-        if (lane >= o) { i0 += t0; i1 += t1; }
-    }
-    a = warp_max(a); b = warp_max(b); c = warp_max(c); d = warp_max(d);
-    __syncthreads();
-    if (lane == 31) { s_scan[warp] = i0; s_scan[8 + warp] = i1; }
-    if (lane == 0) { s_range[warp * 4] = a; s_range[warp * 4 + 1] = b; s_range[warp * 4 + 2] = c; s_range[warp * 4 + 3] = d; }
-    __syncthreads();
-    if (threadIdx.x >= 32 && threadIdx.x < 36) {        // one range atomic per CTA and quantity
-        const int q = threadIdx.x - 32;
-        unsigned long long m = 0;
-        for (int w = 0; w < kApThreads / 32; ++w) m = s_range[w * 4 + q] > m ? s_range[w * 4 + q] : m;
-        unsigned long long *dst = q == 0 ? st->inv_kmin : (q == 1 ? st->kmax : (q == 2 ? st->inv_imin : st->imax));
-        if (m) atomicMax(&dst[next_level], m);
-    }
-    if (threadIdx.x == 0) {
-        unsigned t0 = 0, t1 = 0;
-        for (int w = 0; w < kApThreads / 32; ++w) {
-            const unsigned x0 = s_scan[w], x1 = s_scan[8 + w];
-            s_scan[w] = t0; s_scan[8 + w] = t1;
-            t0 += x0; t1 += x1;
-        }
-        s_scan[16] = t0 ? atomicAdd(n_sure, t0) : 0u;
-        s_scan[17] = t1 ? atomicAdd(n_bnd, t1) : 0u;
-    }
-    __syncthreads();
-    unsigned p0 = s_scan[16] + s_scan[warp] + i0 - c0;
-    unsigned p1 = s_scan[17] + s_scan[8 + warp] + i1 - c1;
-    for (long long i = gtid; i < n; i += gsz) {
-        const KeyId v = load(i);
-        const int k = cls(v);
-        if (k == 0) { if (p0 < (unsigned)kSurvCap) sure[p0] = v; ++p0; }
-        else if (k == 1) { if ((long long)p1 < bnd_cap) bnd[p1] = v; ++p1; }
-    }
-}
-
-// The whole selection in ONE cooperative launch (K <= 1024):
-//   level 0   candidates are split by the pricing histogram's final bound b*: bin < b* are "sure"
-//             (there are fewer than K of them), bin == b* form the boundary list, the rest is dropped;
-//   refine    while sure + boundary > kSurvCap: an 11-bit digit of (key, id) taken at the highest bit
-//             in which the boundary list's minimum and maximum differ is histogrammed, the digit d*
-//             that holds the remaining rank is found, digits < d* become sure, == d* the new boundary
-//             list.  Near-ties resolve in one level, exact ties fall through to the id;
-//   rank      all-pairs rank of sure + boundary (<= 8192 elements) gives every output position.
-__global__ void __launch_bounds__(kApThreads)
+// ---- K <= SX_TOPK_MAX_K: select_topk (sx_select.cuh) in ONE cooperative launch ----
+__global__ void __launch_bounds__(kSelThreads)
 topk_select_kernel(const double *__restrict__ cand_rc, const long long *__restrict__ cand_id, long long cand_cap,
-                   SelState *st, sx_price_header *hdr, int K, KeyId *sure, KeyId *listA, KeyId *listB,
-                   double *__restrict__ out_rc, long long *__restrict__ out_id, long long *out_n) {
-    cg::grid_group grid = cg::this_grid();
-    __shared__ unsigned s_hist[kRefBins];
-    __shared__ unsigned s_b[2];
-    __shared__ unsigned s_scan[18];
-    __shared__ unsigned long long s_range[32];
+                   SelState *st, sx_price_header *hdr, int K, SelLists lists, double *__restrict__ out_rc,
+                   long long *__restrict__ out_id, long long *out_n) {
+    __shared__ SelScratch s;
     const unsigned long long n64 = st->n_cand;
     long long n = (long long)n64;
     if (n64 > (unsigned long long)cand_cap) {
@@ -356,124 +235,21 @@ topk_select_kernel(const double *__restrict__ cand_rc, const long long *__restri
     }
     // the candidate list was pruned for the K given to sx_price_pass_begin: a larger K here cannot be served
     if ((unsigned)K > st->K && blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&hdr->status, kStatusKMismatch);
-    const long long gtid = (long long)blockIdx.x * kApThreads + threadIdx.x;
-    const long long gsz = (long long)gridDim.x * kApThreads;
-
-    // ---- level 0: split by the pricing histogram ----
-    if (threadIdx.x < 32) {
-        unsigned below = 0;
-        const unsigned b = warp_find_bound(st, (unsigned)K, &below);
-        if (threadIdx.x == 0) { s_b[0] = b; s_b[1] = below; }
-    }
-    __syncthreads();
-    const unsigned b1 = s_b[0];
-    long long need = (long long)K - (long long)s_b[1];          // rank still to find inside the boundary list
-    partition_step(
-        n, [&](long long i) { return KeyId{f64_to_sort_key(cand_rc[i]), cand_id[i]}; },
-        [&](const KeyId &v) {
-            const unsigned long long kb = v.key >> (64 - 1 - kFineBits);                 // = cand_bin(rc)
-            const unsigned bin = kb < (unsigned long long)kFineBins ? (unsigned)kb : kFineBins - 1u;
-            return bin < b1 ? 0 : (bin == b1 ? 1 : 2);
-        },
-        sure, &st->n_sure, listA, &st->n_list[0], cand_cap, st, 0, s_scan, s_range);
-    grid.sync();
-
-    // ---- refinement levels ----
-    // Each level leaves a list that agrees on every bit from the chosen digit's lowest bit up, so 6 levels
-    // settle the 64-bit key and 6 more the 63-bit id: only copies of one (key, id) can reach kMaxLevels.
-    static_assert(kMaxLevels >= (64 + 10) / 11 + (63 + 10) / 11, "refinement levels cannot settle a (key, id)");
-    int level = 0;
-    bool failed = false;
-    for (;; ++level) {
-        const unsigned n_sure = ld_relaxed_u32(&st->n_sure), n_a = ld_relaxed_u32(&st->n_list[level]);
-        if (n_sure + n_a <= (unsigned)kRankCap) break;
-        if (level == kMaxLevels) { failed = n_sure + n_a > (unsigned)kSurvCap; break; }
-        const unsigned long long kmin = ~__ldcg(&st->inv_kmin[level]), kmax = __ldcg(&st->kmax[level]);
-        const unsigned long long imin = ~__ldcg(&st->inv_imin[level]), imax = __ldcg(&st->imax[level]);
-        const bool by_key = kmin != kmax;
-        const unsigned long long diff = by_key ? (kmin ^ kmax) : (imin ^ imax);
-        if (diff == 0) { failed = n_sure + n_a > (unsigned)kSurvCap; break; }   // duplicates of one (key, id)
-        const int p = 63 - __clzll((long long)diff);
-        const int sh = p > 10 ? p - 10 : 0;
-        auto digit = [&](const KeyId &v) {
-            return (unsigned)(((by_key ? v.key : (unsigned long long)v.id) >> sh) & (kRefBins - 1));
-        };
-        for (int i = threadIdx.x; i < kRefBins; i += kApThreads) s_hist[i] = 0;
-        __syncthreads();
-        {   // digit histogram; lanes holding the same digit add once (near-ties share one digit)
-            const long long na_ceil = ((long long)n_a + 31) / 32 * 32;
-            for (long long i = gtid; i < na_ceil; i += gsz) {
-                const unsigned dg = i < n_a ? digit(ld_keyid(listA + i)) : 0xffffffffu;
-                const unsigned peers = __match_any_sync(0xffffffffu, dg);
-                if (dg != 0xffffffffu && (int)lane_id() == __ffs(peers) - 1) atomicAdd(&s_hist[dg], (unsigned)__popc(peers));
-            }
-        }
-        __syncthreads();
-        for (int i = threadIdx.x; i < kRefBins; i += kApThreads)
-            if (s_hist[i]) atomicAdd(&st->hist2[level][i], s_hist[i]);
-        grid.sync();
-        // digit holding rank `need`: 2048 bins, 64 per lane of warp 0
-        if (threadIdx.x < 32) {
-            const unsigned *h = st->hist2[level] + threadIdx.x * 64;
-            unsigned hv[64];
-#pragma unroll
-            for (int q = 0; q < 64; q += 4) {
-                const uint4 v = __ldcg(reinterpret_cast<const uint4 *>(h + q));
-                hv[q] = v.x; hv[q + 1] = v.y; hv[q + 2] = v.z; hv[q + 3] = v.w;
-            }
-            unsigned local = 0;
-#pragma unroll
-            for (int q = 0; q < 64; ++q) local += hv[q];
-            unsigned incl = local;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const unsigned t = __shfl_up_sync(0xffffffffu, incl, o);
-                if (threadIdx.x >= o) incl += t;
-            }
-            const unsigned cross = __ballot_sync(0xffffffffu, (long long)incl >= need);
-            const int owner = cross ? __ffs(cross) - 1 : 31;
-            if ((int)threadIdx.x == owner) {
-                unsigned cum = incl - local;
-                const int q = find_in_lane(hv, (unsigned)need, cum);
-                s_b[0] = threadIdx.x * 64 + q;
-                s_b[1] = cum;
-            }
-        }
-        __syncthreads();
-        const unsigned dstar = s_b[0];
-        need -= (long long)s_b[1];
-        partition_step(
-            (long long)n_a, [&](long long i) { return ld_keyid(listA + i); },
-            [&](const KeyId &v) {
-                const unsigned dg = digit(v);
-                return dg < dstar ? 0 : (dg == dstar ? 1 : 2);
-            },
-            sure, &st->n_sure, listB, &st->n_list[level + 1], cand_cap, st, level + 1, s_scan, s_range);
-        grid.sync();
-        KeyId *t = listA; listA = listB; listB = t;
-    }
-
-    // ---- all-pairs rank of sure ++ boundary ----
-    const int n_sure = failed ? 0 : (int)ld_relaxed_u32(&st->n_sure);
-    const int n_s = failed ? 0 : n_sure + (int)ld_relaxed_u32(&st->n_list[level]);
-    const int n_out = n_s < K ? n_s : K;
-    if (blockIdx.x == 0) {
-        for (int i = n_out + threadIdx.x; i < K; i += kApThreads) { out_rc[i] = INFINITY; out_id[i] = -1; }
-        if (threadIdx.x == 0) {
-            *out_n = n_out;
-            if (failed) atomicOr(&hdr->status, kStatusDuplicateCandidates);
-        }
-    }
-    if (n_s == 0) return;
-    all_pairs_rank(
-        n_s, [&](int e) { return ld_keyid(e < n_sure ? sure + e : listA + (e - n_sure)); },
-        [&](int e, int rank) {
-            if (rank < K) {
-                const KeyId v = ld_keyid(e < n_sure ? sure + e : listA + (e - n_sure));
+    const SelResult r = select_topk(
+        cand_rc, cand_id, n, cand_cap, st, K, lists, s, [] { cg::this_grid().sync(); },
+        [&](const KeyId &v, int rank, int sub, int) {
+            if (sub == 0 && rank < K) {
                 out_rc[rank] = sort_key_to_f64(v.key);
                 out_id[rank] = v.id;
             }
         });
+    if (blockIdx.x == 0) {
+        for (int i = r.n_out + threadIdx.x; i < K; i += kSelThreads) { out_rc[i] = INFINITY; out_id[i] = -1; }
+        if (threadIdx.x == 0) {
+            *out_n = r.n_out;
+            if (r.duplicates) atomicOr(&hdr->status, kStatusDuplicateCandidates);
+        }
+    }
 }
 
 // Merge of G sorted, padded blocks of K (exchanged between G ranks).  One thread per element: its
@@ -757,17 +533,15 @@ extern "C" int sx_topk_select(const double *cand_rc, const int64_t *cand_id, int
     cudaStream_t st = (cudaStream_t)stream;
     SelState *sst = (SelState *)sel;
     Carver cv(ws);
-    KeyId *sure = cv.take<KeyId>(kSurvCap);
-    KeyId *listA = cv.take<KeyId>(cand_cap > 0 ? cand_cap : 1);
-    KeyId *listB = cv.take<KeyId>(cand_cap > 0 ? cand_cap : 1);
+    SelLists lists = carve_sel_lists(cv, cand_cap);
     if (K > SX_TOPK_MAX_K)
         return topk_select_large_k(cand_rc, cand_id, cand_cap, sst, K, out_rc, out_id, out_n, cv, ws_bytes, st);
     const long long *cid = (const long long *)cand_id;
     int Ki = (int)K;
     long long *oid = (long long *)out_id, *on = (long long *)out_n;
     void *args[] = {(void *)&cand_rc, (void *)&cid, (void *)&cand_cap, (void *)&sst, (void *)&header, (void *)&Ki,
-                    (void *)&sure, (void *)&listA, (void *)&listB, (void *)&out_rc, (void *)&oid, (void *)&on};
-    SX_CUDA(cudaLaunchCooperativeKernel((void *)topk_select_kernel, dim3(num_sms()), dim3(kApThreads), args, 0, st));
+                    (void *)&lists, (void *)&out_rc, (void *)&oid, (void *)&on};
+    SX_CUDA(cudaLaunchCooperativeKernel((void *)topk_select_kernel, dim3(num_sms()), dim3(kSelThreads), args, 0, st));
     return SX_OK;
 }
 

@@ -21,9 +21,8 @@ SX_STATUS_CAND_OVERFLOW = 1
 SX_STATUS_DUPLICATE_CANDIDATES = 2
 SX_STATUS_K_MISMATCH = 4
 SX_STATUS_NAN_RC = 8
-SX_STATUS_NEED_UNFUSED = 16
-SX_STATUS_REPEAT_MASK = 17
-SX_ABI_VERSION = 5
+SX_STATUS_REPEAT_MASK = 1
+SX_ABI_VERSION = 6
 
 
 class SxError(RuntimeError):
@@ -87,7 +86,6 @@ SIGNATURES = {
     "sx_price_set_tuning": (_int, [_int, _int]),
     "sx_price_set_tma_options": (_int, [_int, _int]),
     "sx_fused_state_bytes": (_sz, []),
-    "sx_fused_workspace_bytes": (_sz, []),
     "sx_fused_state_timestamps_offset": (_sz, []),
     "sx_fused_state_init": (_int, [_p, _i64, _p]),
     "sx_fused_merge_fits": (_int, [_i64, _int]),

@@ -220,7 +220,6 @@ class Pricer:
         self._fused_passes, self._last_fused = 0, False
         if self.fused:
             self.fstate = torch.zeros(lib.sx_fused_state_bytes(), dtype=torch.uint8, device=device)
-            self.fws = _ws(lib.sx_fused_workspace_bytes(), device)
             check(lib.sx_fused_state_init(_ptr(self.fstate), Kp, _stream()), "sx_fused_state_init")
 
     def _alloc(self):
@@ -254,8 +253,7 @@ class Pricer:
                                           _ptr(self.fstate), _ptr(self.cand_rc), _ptr(self.cand_id),
                                           self.cap if self.K > 0 else 0, self.Kp, _ptr(self.block),
                                           self.block.numel(), peer_bufs, rank, G, _ptr(merged), _ptr(xstatus),
-                                          _ptr(self.fws),
-                                          self.fws.numel(), _stream()), "sx_price_dense_ot_fused")
+                                          _ptr(self.ws), self.ws.numel(), _stream()), "sx_price_dense_ot_fused")
         self.launches += 1
         self._fused_passes += 1
         self._last_fused = True
@@ -349,12 +347,9 @@ def price_dense_ot(M: torch.Tensor, y: torch.Tensor, K: int = 0, tol: float = TO
             pr.price_dense(M, M.stride(0), 0, S, D, y[:S], y[S:S + D], tol, rc, variant)
             pr.select()
         res = pr.fetch()
-        if pr.overflowed(res):
-            pr.grow(res.n_violating)   # more violators than candidate slots: size exactly, price again
-        elif fused and (pr.status & _native.SX_STATUS_NEED_UNFUSED):
-            fused = False              # too many ties for the in-kernel selection: separate kernels
-        else:
+        if not pr.overflowed(res):
             break
+        pr.grow(res.n_violating)       # more violators than candidate slots: size exactly, price again
     res.rc = rc
     return res
 

@@ -141,10 +141,11 @@ class ShardedDensePricer:
         return self.pricer.launches + self._merge_launches + self._replayed_launches - self._capture_overcount
 
     # -- device-only step: everything stays on the GPU(s) --------------------------------------
-    def enqueue(self, y_dev: torch.Tensor, kernel_events=None, stage_events=None, y_parts=None, unfused: bool = False):
+    def enqueue(self, y_dev: torch.Tensor, kernel_events=None, stage_events=None, y_parts=None):
         """Enqueue one pricing pass; returns device tensors
-        (rc[K], id[K], n_out, count, min key, largest per-rank count, status).  A non-zero status
-        (SX_STATUS_*) means the pass must be repeated (`price` does that).  `kernel_events` =
+        (rc[K], id[K], n_out, count, min key, largest per-rank count, status).  A status with
+        SX_STATUS_CAND_OVERFLOW means the pass must be repeated with larger candidate buffers (`price`
+        does that).  `kernel_events` =
         (start, end) CUDA events recorded around the pricing kernel launch (bench.py's roofline
         measurement); `stage_events` = 5 events recorded at pass start, after pricing, after the
         selection, after the exchange and after the merge (the last two only when world > 1).
@@ -153,9 +154,8 @@ class ShardedDensePricer:
         y_src, y_dst = y_parts if y_parts is not None else (y_dev[self.row0:self.row0 + self.S_loc],
                                                               y_dev[self.S:self.S + self.D])
         mark = (lambda i: stage_events[i].record()) if stage_events is not None else (lambda i: None)
-        fused = self.fused and not unfused
         mark(0)
-        if fused:
+        if self.fused:
             # ONE launch: state clear of the next pass, pricing, selection and (exchange "ll") the push of the
             # selected arcs into every peer's buffer
             if kernel_events is not None:
@@ -186,12 +186,12 @@ class ShardedDensePricer:
             return p.out_rc, p.out_id, p.out_n[0], p.header[0], p.header[1], p.header[0], p.header[3]
         # one exchange: every rank's block (top-K + header) lands in `gathered`, consumed in place
         if self.exchange == "ll":
-            if fused and self.fused_merge:                 # the merge ran inside the pricing kernel too
+            if self.fused_merge:                           # the merge ran inside the pricing kernel too
                 mark(3)
                 mark(4)
                 return (self._m_rc, self._m_id, self._m_n[0], self._m_sum[0], self._m_sum[1], self._m_sum[2],
                         self._m_sum[3])
-            if not fused:
+            if not self.fused:
                 check(lib.sx_exchange_push_ll(dev._ptr(p.block), self.blk, self._hdl.buffer_ptrs_dev, self._rank,
                                               self.world, dev._stream()), "sx_exchange_push_ll")
                 self._merge_launches += 1
@@ -225,12 +225,12 @@ class ShardedDensePricer:
         return self._m_rc, self._m_id, self._m_n[0], self._m_sum[0], self._m_sum[1], self._m_sum[2], self._m_sum[3]
 
     # -- host-facing call: duals in, (count, min, top-K) out --------------------------------------
-    def _step(self, unfused: bool = False):
+    def _step(self):
         """H2D of the duals this rank needs (its rows + every sink), one pass, D2H of the result."""
         r0 = self.row0                                             # y_loc = [this rank's S_loc source duals | D sink duals]
         self.y_loc[:self.S_loc].copy_(self.h_y[r0:r0 + self.S_loc], non_blocking=True)
         self.y_loc[self.S_loc:].copy_(self.h_y[self.S:], non_blocking=True)
-        self.enqueue(None, y_parts=(self.y_loc[:self.S_loc], self.y_loc[self.S_loc:]), unfused=unfused)
+        self.enqueue(None, y_parts=(self.y_loc[:self.S_loc], self.y_loc[self.S_loc:]))
         if self.world == 1:
             self.pricer.h_block.copy_(self.pricer.block, non_blocking=True)
         else:
@@ -301,7 +301,6 @@ class ShardedDensePricer:
         if self._dead:
             raise RuntimeError("this pricer saw a peer-exchange timeout; its epoch counters may be out of step with "
                                "the peers': build a new one")
-        unfused = False
         first = True
         while True:
             if first and self._graph is not None:
@@ -310,20 +309,17 @@ class ShardedDensePricer:
                 if self.fused:
                     self.pricer.note_replayed_fused_passes(1)
             else:
-                self._step(unfused=unfused)
+                self._step()
             first = False
             torch.cuda.current_stream().synchronize()
             res, status, cmax = self._read_result()
-            # Every rank reads the same folded status, so all ranks repeat the pass together: with a larger
-            # candidate buffer after an overflow, with the separate kernels after SX_STATUS_NEED_UNFUSED.
+            # Every rank reads the same folded status, so all ranks repeat the pass together, with a larger
+            # candidate buffer after an overflow.
             res.status = status
-            if self.K == 0 or (status & _native.SX_STATUS_REPEAT_MASK) == 0:
+            if self.K == 0 or (status & _native.SX_STATUS_CAND_OVERFLOW) == 0:
                 return res
-            if status & _native.SX_STATUS_CAND_OVERFLOW:
-                self.pricer.grow(cmax)
-                self._graph, self._capture_tried = None, False      # buffers moved: record again next time
-            else:                                                   # SX_STATUS_NEED_UNFUSED: the separate kernels refine
-                unfused = True
+            self.pricer.grow(cmax)
+            self._graph, self._capture_tried = None, False          # buffers moved: record again next time
 
     @property
     def y_pinned(self) -> np.ndarray:

@@ -28,13 +28,13 @@ def test_header_declares_the_expected_entry_points():
     assert len(names) >= 24
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_abi_6():
     _ensure_built()
     lib = ctypes.CDLL(LIB)
     for name in _declared():
         assert hasattr(lib, name), f"{name} declared in sxcross.h but not exported"
     lib.sx_abi_version.restype = ctypes.c_int
-    assert lib.sx_abi_version() == 5
+    assert lib.sx_abi_version() == 6
     lib.sx_error_string.restype = ctypes.c_char_p
     assert b"spanning" in lib.sx_error_string(-5)
 

@@ -100,8 +100,8 @@ def test_sharded_pricer_on_real_ranks_matches_oracle(exchange, K):
 @pytest.mark.skipif(_n_gpus() < 2, reason="needs at least 2 GPUs")
 @pytest.mark.parametrize("exchange", ["ll", "nccl"])
 def test_sharded_pricer_separate_kernels_on_real_ranks(exchange):
-    """The round-1 path (pass begin, pricing, selection, push and merge as separate launches), which the
-    fused pass falls back to, on real ranks."""
+    """The round-1 path (pass begin, pricing, selection, push and merge as separate launches), which prices
+    slabs the fused pass cannot take (odd leading dimension, unaligned base), on real ranks."""
     _spawn(2, exchange, 301, 517, 256, fused=False)
 
 

@@ -41,6 +41,15 @@ def cu(a, dtype=None):
     return t.cuda()
 
 
+def price_in_one_fused_launch(dev, pr, M, y, K):
+    """price_dense_ot through the fused pricer `pr`; the pass must be one launch of the fused kernel."""
+    assert pr.fused
+    before = pr.launches
+    res = dev.price_dense_ot(cu(M), cu(y), K=K, pricer=pr)
+    assert pr.launches == before + 1
+    return res
+
+
 def u32(t):
     """uint32 bit patterns stored in an int32 tensor -> int64 numpy."""
     return t.cpu().numpy().view(np.uint32).astype(np.int64)
@@ -509,7 +518,10 @@ def test_price_all_equal_reduced_costs(dev, fused_mode):
     M = np.full((S, D), 2.0)
     y = np.concatenate([np.zeros(S), np.full(D, 3.0)])            # rc = -1 everywhere
     pr = dev.Pricer(torch.device("cuda"), K)
-    res = dev.price_dense_ot(cu(M), cu(y), K=K, pricer=pr)
+    if fused_mode == "fused":
+        res = price_in_one_fused_launch(dev, pr, M, y, K)
+    else:
+        res = dev.price_dense_ot(cu(M), cu(y), K=K, pricer=pr)
     assert res.n_violating == S * D and res.min_rc == -1.0
     assert np.array_equal(res.topk_id, np.arange(K)) and np.all(res.topk_rc == -1.0)
     assert pr.status == 0
@@ -573,9 +585,44 @@ def test_price_near_ties_at_the_kth_value(dev, fused_mode):
     cnt, mn, ids, vals = orc.price_summary(rc_ref, K=K)
     assert cnt >= D
     pr = dev.Pricer(torch.device("cuda"), K)
-    res = dev.price_dense_ot(cu(M), cu(y), K=K, pricer=pr)
+    if fused_mode == "fused":
+        res = price_in_one_fused_launch(dev, pr, M, y, K)
+    else:
+        res = dev.price_dense_ot(cu(M), cu(y), K=K, pricer=pr)
     assert pr.status == 0 and res.n_violating == cnt and res.min_rc == mn
     assert np.array_equal(res.topk_id, ids) and np.array_equal(res.topk_rc, vals)
+
+
+@pytest.mark.parametrize("layout", ["ties", "tie_block"])
+def test_fused_selection_refines_on_a_small_grid(dev, layout):
+    """S = 16, D = 2560 is 10 tiles, so the fused kernel runs on 10 CTAs (2 560 selecting threads).  All
+    40 960 reduced costs lie in one histogram bin and rank K falls inside a run of exact ties, next to
+    near-ties that differ from them in low mantissa bits.  "ties": 600 near-ties below a tie of all the
+    other arcs, refined down to the arc id; "tie_block": 900 near-ties below a tie of 3 000 arcs and the
+    rest above it, which leaves 3 900 survivors -- more than the grid has threads -- for the rank.  The
+    oracle's top K must come back from one launch, on both selection states of the pricer."""
+    S, D, K = 16, 2560, 1024
+    rng = np.random.default_rng(16)
+    tie = -(1.0 + 2.0 ** -9)                                      # middle of its 0.4 %-wide histogram bin
+    near = rng.integers(1 << 20, 1 << 30, S * D) * 2.0 ** -52
+    side = np.zeros(S * D)                                        # -1: below the tie (more violating), +1: above
+    pick = rng.permutation(S * D)
+    if layout == "ties":
+        side[pick[:600]] = -1
+    else:
+        side[pick[:900]] = -1
+        side[pick[3900:]] = 1
+    M = (3.0 + tie + side * near).reshape(S, D)
+    y = np.concatenate([np.zeros(S), np.full(D, 3.0)])            # rc = M - 3
+    rc_ref = orc.reduced_costs_ot(M, y)
+    assert np.array_equal(rc_ref, tie + side * near)
+    cnt, mn, ids, vals = orc.price_summary(rc_ref, K=K)
+    assert cnt == S * D and vals[-1] == tie and vals[0] < tie     # rank K lies inside the tie
+    pr = dev.Pricer(torch.device("cuda"), K, fused=True)
+    for _ in range(2):
+        res = price_in_one_fused_launch(dev, pr, M, y, K)
+        assert pr.status == 0 and res.n_violating == cnt and res.min_rc == mn
+        assert np.array_equal(res.topk_id, ids) and res.topk_rc.tobytes() == vals.tobytes()
 
 
 def test_price_bins_are_monotone_over_magnitudes(dev, fused_mode):
@@ -624,11 +671,10 @@ def test_price_tma_stage_release_under_atomic_pressure(dev, fused_mode):
         res = pr.fetch()
         assert res.n_violating == cnt and np.array_equal(res.topk_id, ids)
     if fused_mode == "fused":
-        # the same pressure inside the fused kernel: 8 M survivors are too many for its in-kernel rank, so
-        # every pass raises SX_STATUS_NEED_UNFUSED and is repeated by the separate kernels
-        assert pr.fused
+        # the same pressure inside the fused kernel, whose selection refines the 8 M candidates of the one
+        # bin in the same launch
         for _ in range(3):
-            res = dev.price_dense_ot(cu(M), cu(y), K=K, pricer=pr)
+            res = price_in_one_fused_launch(dev, pr, M, y, K)
             assert pr.status == 0 and res.n_violating == cnt and res.min_rc == mn
             assert np.array_equal(res.topk_id, ids) and np.array_equal(res.topk_rc, vals)
 
