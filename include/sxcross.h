@@ -313,7 +313,12 @@ SX_API int    sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0,
  *   radix argsorts (synchronises the stream once to read the candidate count).
  * sx_topk_merge merges G sorted, padded blocks (as exchanged between G ranks) into one.  Block g
  *   has its rc list at blocks_rc + g * block_stride and its ids at blocks_id + g * block_stride
- *   (strides in 8-byte elements, so the gathered buffer is consumed in place).  Optionally folds
+ *   (strides in 8-byte elements, so the gathered buffer is consumed in place).  A block is sorted by
+ *   (rc, id) as the selection writes it: its real entries, then padding (+inf, -1).  The merges
+ *   (here, sx_topk_merge_ll and the in-kernel merge of sx_price_dense_ot_fused) recognise padding by
+ *   id < 0, or by rc = +inf where they read only rc: a real entry is a violator, never +inf.  rc
+ *   compares by its order-preserving image (-0.0 == +0.0); exact ties go to the smaller id, and ids
+ *   must be distinct across blocks.  Optionally folds
  *   the G pricing headers found at headers + g * block_stride into out_summary =
  *   {total n_violating, min key, largest single n_violating, OR of the status words}.
  *   parity_ctr (device, may be NULL): when the blocks sit in a double-buffered exchange buffer
@@ -352,13 +357,15 @@ SX_API int    sx_exchange_blocks(const int64_t *block, int64_t block_len, void *
 
 /* Low-latency form of the same exchange (default of the package): sx_exchange_push_ll only STORES --
  * every 8-byte word of the block travels as one 16-byte slot {lo32, flag, hi32, flag}, flag = epoch --
- * and sx_topk_merge_ll polls the slots of its local buffer while it stages the G blocks in shared
- * memory, then merges them like sx_topk_merge.  No fence, no flag round trip, no separate wait.
+ * and sx_topk_merge_ll polls the slots of its local buffer while it stages the keys of the G blocks in
+ * shared memory, then merges them like sx_topk_merge.  No fence, no flag round trip, no separate wait.
+ * It runs the same merge as the last CTAs of sx_price_dense_ot_fused (merged_out != NULL).
  *   Buffer: sx_exchange_ll_buffer_bytes() bytes, zeroed, peer-mapped; the epoch counters (one advanced
  *   by the pushing side, one by the merge, each once per pass) sit right after the 2 * G * block_len
  *   slots.  The merge depends on no other kernel of its GPU and is launched with programmatic stream
  *   serialisation: behind sx_price_dense_ot_fused it becomes resident while that kernel drains.  block = [K rc | K ids | 4 header words | ...], block_len >= 2 K + 4.
- *   G * K * 16 bytes must fit in shared memory (200 KB), else SX_ERR_TOO_LARGE.
+ *   G * K * 16 must not exceed 200 KB, else SX_ERR_TOO_LARGE (callers size against this limit; the
+ *   kernel itself stages G * K * 8 bytes).
  *   out_summary (4 words, may be NULL) as in sx_topk_merge; status_dev as in sx_exchange_blocks.
  */
 SX_API size_t sx_exchange_ll_buffer_bytes(int64_t block_len, int G);

@@ -15,7 +15,7 @@
 //
 // Double buffering is enough: a rank can only be one epoch ahead of a peer, because finishing epoch
 // e + 1 needs that peer's flag for e + 1, which the peer raises after its epoch-e merge (stream order).
-#include "sx_common.cuh"
+#include "sx_ll.cuh"
 
 namespace sx {
 
@@ -26,11 +26,6 @@ __device__ __forceinline__ unsigned long long ld_acquire_sys(const unsigned long
     unsigned long long v;
     asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
     return v;
-}
-__device__ __forceinline__ unsigned long long global_timer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
 }
 
 constexpr int kXcThreads = 256;
@@ -64,45 +59,24 @@ exchange_blocks_kernel(const long long *__restrict__ block, long long block_len,
             if (global_timer_ns() - t0 > timeout_ns) { atomicExch(status, SX_ERR_PEER_TIMEOUT); break; }
             __nanosleep(100);
         }
-        // the last CTA to finish advances the epoch for the next launch
-        __threadfence();
-        if (atomicAdd(ctr + 1, 1ull) == (unsigned long long)(G - 1)) {
-            ctr[1] = 0ull;
-            *reinterpret_cast<volatile unsigned long long *>(ctr) = epoch;
-        }
+        advance_epoch_when_last(ctr, G, epoch);   // the last CTA to finish
     }
 }
 
 // ---- low-latency variant: flag-in-data ("LL") push --------------------------------------------
 // Every 8-byte word travels as one 16-byte store {lo32, flag, hi32, flag} with flag = (uint32) epoch,
 // so the receiver needs no separate flag, no fence and no second NVLink round trip: it polls each
-// slot until both flags show the epoch (8-byte units are written atomically; sx_topk_merge_ll does
-// the polling while it stages the blocks in shared memory).  The kernel only stores, it never waits.
+// slot until both flags show the epoch (8-byte units are written atomically; merge_ll of sx_merge.cuh
+// does the polling while it stages the blocks in shared memory).  The kernel only stores, it never waits.
 __global__ void __launch_bounds__(kXcThreads)
 exchange_push_ll_kernel(const unsigned long long *__restrict__ block, long long block_len, char *const *peer_bufs,
                         int rank, int G) {
-    const int p = blockIdx.x;
-    const size_t slots_bytes = (size_t)2 * G * block_len * 16;
-    char *local = peer_bufs[rank];
-    unsigned long long *ctr = reinterpret_cast<unsigned long long *>(local + slots_bytes);
+    unsigned long long *ctr = ll_counters(peer_bufs[rank], G, block_len);
     const unsigned long long epoch = *reinterpret_cast<volatile unsigned long long *>(ctr) + 1ull;
-    const unsigned flag = (unsigned)epoch;
-    uint4 *dst = reinterpret_cast<uint4 *>(peer_bufs[p]) + ((size_t)(epoch & 1ull) * G + rank) * block_len;
-    for (long long i = threadIdx.x; i < block_len; i += kXcThreads) {
-        const unsigned long long v = block[i];
-        const uint4 w = make_uint4((unsigned)v, flag, (unsigned)(v >> 32), flag);
-        asm volatile("st.volatile.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(dst + i), "r"(w.x), "r"(w.y), "r"(w.z),
-                     "r"(w.w)
-                     : "memory");
-    }
+    uint4 *dst = ll_slot(peer_bufs[blockIdx.x], G, block_len, epoch, rank, 0);
+    for (long long i = threadIdx.x; i < block_len; i += kXcThreads) ll_store_slot(dst + i, (unsigned)epoch, block[i]);
     __syncthreads();
-    if (threadIdx.x == 0) {                       // the last CTA to finish advances the epoch for the next launch
-        __threadfence();
-        if (atomicAdd(ctr + 1, 1ull) == (unsigned long long)(G - 1)) {
-            ctr[1] = 0ull;
-            *reinterpret_cast<volatile unsigned long long *>(ctr) = epoch;
-        }
-    }
+    if (threadIdx.x == 0) advance_epoch_when_last(ctr, G, epoch);   // the last CTA to finish
 }
 
 }  // namespace sx

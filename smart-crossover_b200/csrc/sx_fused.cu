@@ -18,16 +18,17 @@
 //            the lanes of an element write it to its position in the local result block AND, with G > 1,
 //            store it as flag-in-data slots straight into every peer's exchange buffer (NVLink; sx_ll.cuh),
 //            so the exchange needs no kernel of its own and starts while other elements are still ranked;
-//   merge    (G > 1) the last CTAs of the grid -- which have no rank work -- stage the keys of all G blocks
-//            out of the local exchange buffer as they land (staging is the wait), rank every element by
-//            G - 1 binary searches in shared memory and write the merged top-K.
+//   merge    the last CTAs of the grid -- which have no rank work -- run merge_ll (sx_merge.cuh), the merge
+//            sx_topk_merge_ll runs too: they stage the keys of all G blocks out of the local exchange buffer
+//            as they land (staging is the wait), rank every element by G - 1 binary searches in shared
+//            memory and write the merged top-K.
 //
 // If the candidate buffer overflowed, the pass raises SX_STATUS_CAND_OVERFLOW in the header -- it still
 // pushes a well-formed block so that no peer waits -- and the caller grows the buffer and repeats the pass.
 #include <stdlib.h>
 
 #include "sx_gridbar.cuh"
-#include "sx_ll.cuh"
+#include "sx_merge.cuh"
 #include "sx_price_tma.cuh"
 
 namespace sx {
@@ -74,11 +75,6 @@ __device__ __forceinline__ void stamp(FusedCtl *ctl, int i) {
     if (blockIdx.x == 0 && threadIdx.x == 0) ctl->ts[i] = global_timer_ns();
 }
 
-// slot `idx` of rank r's block, parity half of `epoch`, in the exchange buffer `buf`
-__device__ __forceinline__ uint4 *ll_slot(char *buf, const FusedParams &f, unsigned long long epoch, int r, long long idx) {
-    return reinterpret_cast<uint4 *>(buf) + ((size_t)(epoch & 1ull) * f.G + r) * f.block_len + idx;
-}
-
 template <int ROWS, int STAGES, int CWARPS, int MINB>
 __global__ void __launch_bounds__((CWARPS + 1) * 32, MINB)
 price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p0, const FusedParams f) {
@@ -86,8 +82,7 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
                   "the stage ring is reused as the selection's shared memory");
     static_assert(CWARPS * 32 == kSelThreads, "the consumer warps select, the producer warp joins the barriers");
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ long long s_hdr[4];
-    __shared__ int s_real;
+    __shared__ MergeFold s_fold;
     const int tid = threadIdx.x, nthr = blockDim.x;
     const int K = (int)f.K;
     FusedCtl *ctl = &f.state->ctl;
@@ -100,7 +95,7 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
     char *ll_local = nullptr;
     if (f.peer_bufs) {
         ll_local = f.peer_bufs[f.rank];
-        ll_ctr = reinterpret_cast<unsigned long long *>(ll_local + (size_t)2 * f.G * f.block_len * 16);
+        ll_ctr = ll_counters(ll_local, f.G, f.block_len);
         epoch = ld_volatile_u64(ll_ctr) + 1ull;
     }
     const unsigned flag = (unsigned)epoch;
@@ -146,8 +141,8 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
             if (sub == 0) { f.block[rank] = (long long)rc_bits; f.block[K + rank] = v.id; }
             if (f.peer_bufs)
                 for (int q = sub; q < f.G; q += L) {
-                    ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, rank), flag, rc_bits);
-                    ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, (long long)K + rank), flag,
+                    ll_store_slot(ll_slot(f.peer_bufs[q], f.G, f.block_len, epoch, f.rank, rank), flag, rc_bits);
+                    ll_store_slot(ll_slot(f.peer_bufs[q], f.G, f.block_len, epoch, f.rank, (long long)K + rank), flag,
                                   (unsigned long long)v.id);
                 }
         });
@@ -161,8 +156,8 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
             f.block[i] = (long long)pad_rc; f.block[K + i] = -1;
             if (f.peer_bufs)
                 for (int q = 0; q < f.G; ++q) {
-                    ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, i), flag, pad_rc);
-                    ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, (long long)K + i), flag, ~0ull);
+                    ll_store_slot(ll_slot(f.peer_bufs[q], f.G, f.block_len, epoch, f.rank, i), flag, pad_rc);
+                    ll_store_slot(ll_slot(f.peer_bufs[q], f.G, f.block_len, epoch, f.rank, (long long)K + i), flag, ~0ull);
                 }
         }
         if (tid < 6) {
@@ -177,125 +172,20 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
             f.block[2 * K + tid] = (long long)w;
             if (f.peer_bufs)
                 for (int q = 0; q < f.G; ++q)
-                    ll_store_slot(ll_slot(f.peer_bufs[q], f, epoch, f.rank, (long long)2 * K + tid), flag, w);
+                    ll_store_slot(ll_slot(f.peer_bufs[q], f.G, f.block_len, epoch, f.rank, (long long)2 * K + tid), flag, w);
         }
     }
 
     if (blockIdx.x == gridDim.x - 1 && tid == 0) ctl->ts[6] = global_timer_ns();   // overwritten at the end of the merge
-    // ---- merge of the G blocks out of the local exchange buffer (replaces sx_topk_merge_ll) ----
+    // ---- merge of the G blocks out of the local exchange buffer (merge_ll, sx_merge.cuh) ----
     if (f.peer_bufs == nullptr || f.merged == nullptr) return;
     const int n_merge = gridDim.x < kMergeCtas ? (int)gridDim.x : kMergeCtas;
     const int mc = (int)blockIdx.x - ((int)gridDim.x - n_merge);           // index among the merge CTAs
     if (mc < 0) return;
-    const int GK = f.G * K;
-    unsigned long long *mkey = reinterpret_cast<unsigned long long *>(smem_raw);   // GK keys; padding = key(+inf)
-    const unsigned long long kPadKey = f64_to_sort_key(INFINITY);
-    const unsigned long long t_start = global_timer_ns();
-    bool ok = true;
-    if (tid == 0) { s_real = 0; s_hdr[0] = 0; s_hdr[1] = 0x7fffffffffffffffll; s_hdr[2] = 0; s_hdr[3] = 0; }
-    __syncthreads();                                                       // the rank tiles are no longer read
-    // elements of this CTA: [e_lo, e_hi), thread t takes e_lo + t, e_lo + t + nthr, ...  The id of the first one
-    // is requested before the keys so that it is in flight with them.
-    const int per_cta = (GK + n_merge - 1) / n_merge;
-    const int e_lo = mc * per_cta, e_hi = (e_lo + per_cta < GK) ? e_lo + per_cta : GK;
-    uint4 w_id = make_uint4(0u, 0u, 0u, 0u);
-    if (e_lo + tid < e_hi) {
-        const int g = (e_lo + tid) / K;
-        w_id = ll_load_slot(ll_slot(ll_local, f, epoch, g, (long long)K + (e_lo + tid - g * K)));
-    }
-    {
-        // kBatch slots are requested together and the whole batch is requested again until every slot carries
-        // this epoch's flag: the merge CTAs start polling while the peers are still ranking, and re-polling the
-        // late slots one by one would cost one L2 round trip each (28 per thread at G = 8: 20 us; measured).
-        constexpr int kBatch = 8;
-        int real = 0;
-        for (int e0 = tid; e0 < GK; e0 += nthr * kBatch) {
-            uint4 w[kBatch];
-            for (;;) {
-                bool all = true;
-#pragma unroll
-                for (int u = 0; u < kBatch; ++u) {
-                    const int e = e0 + u * nthr;
-                    if (e < GK) { const int g = e / K; w[u] = ll_load_slot(ll_slot(ll_local, f, epoch, g, e - g * K)); }
-                }
-#pragma unroll
-                for (int u = 0; u < kBatch; ++u) {
-                    const int e = e0 + u * nthr;
-                    if (e < GK && !ll_ready(w[u], flag)) all = false;
-                }
-                if (all) break;
-                if (global_timer_ns() - t_start > f.timeout_ns) { ok = false; break; }
-            }
-#pragma unroll
-            for (int u = 0; u < kBatch; ++u) {
-                const int e = e0 + u * nthr;
-                if (e >= GK) continue;
-                const unsigned long long bits = ll_ready(w[u], flag) ? ll_value(w[u]) : 0x7ff0000000000000ull;
-                const unsigned long long key = f64_to_sort_key(__longlong_as_double((long long)bits));
-                mkey[e] = key;
-                real += key != kPadKey;
-            }
-        }
-        if (mc == 0) {                                                     // one CTA folds the headers and the count
-            real = warp_sum(real);
-            if (lane_id() == 0 && real) atomicAdd(&s_real, real);
-            for (int g = tid; g < f.G; g += nthr) {
-                unsigned long long h0, h1, h3;
-                ok = ll_poll(ll_slot(ll_local, f, epoch, g, (long long)2 * K), flag, h0, t_start, f.timeout_ns) && ok;
-                ok = ll_poll(ll_slot(ll_local, f, epoch, g, (long long)2 * K + 1), flag, h1, t_start, f.timeout_ns) && ok;
-                ok = ll_poll(ll_slot(ll_local, f, epoch, g, (long long)2 * K + 3), flag, h3, t_start, f.timeout_ns) && ok;
-                atomicAdd((unsigned long long *)&s_hdr[0], h0);
-                atomicMin(&s_hdr[1], (long long)h1);
-                atomicMax(&s_hdr[2], (long long)h0);
-                atomicOr((unsigned long long *)&s_hdr[3], h3);
-            }
-        }
-    }
-    __syncthreads();
-    if (mc == 0) {
-        const int n_tot = s_real < K ? s_real : K;
-        for (int i = n_tot + tid; i < K; i += nthr) { f.merged[i] = 0x7ff0000000000000ll; f.merged[K + i] = -1; }
-        if (tid == 0) {
-            f.merged[2 * K] = n_tot;
-            f.merged[2 * K + 1] = s_hdr[0]; f.merged[2 * K + 2] = s_hdr[1];
-            f.merged[2 * K + 3] = s_hdr[2]; f.merged[2 * K + 4] = s_hdr[3];
-        }
-    }
-    for (int my_e = e_lo + tid; my_e < e_hi; my_e += nthr) {
-        const unsigned long long key = mkey[my_e];
-        if (key == kPadKey) continue;
-        const int my_g = my_e / K, my_i = my_e - my_g * K;
-        unsigned long long id_bits = ll_value(w_id);
-        if (my_e != e_lo + tid || !ll_ready(w_id, flag))
-            ok = ll_poll(ll_slot(ll_local, f, epoch, my_g, (long long)K + my_i), flag, id_bits, t_start, f.timeout_ns) && ok;
-        const long long my_id = (long long)id_bits;
-        int rank = my_i;
-        for (int h = 0; h < f.G && rank < K; ++h) {
-            if (h == my_g) continue;
-            const unsigned long long *kh = mkey + h * K;
-            int lo = 0, hi = K;                                            // first index with key >= mine
-            while (lo < hi) { const int mid = (lo + hi) >> 1; if (kh[mid] < key) lo = mid + 1; else hi = mid; }
-            if (lo < K && kh[lo] == key) {
-                // equal reduced costs in another block: the arc id decides; ids are read from the buffer
-                int ub = lo, hi2 = K;                                      // first index with key > mine
-                while (ub < hi2) { const int mid = (ub + hi2) >> 1; if (kh[mid] <= key) ub = mid + 1; else hi2 = mid; }
-                int a = lo, b = ub;                                        // first index in [lo, ub) with id >= mine
-                while (a < b) {
-                    const int mid = (a + b) >> 1;
-                    unsigned long long ob;
-                    ok = ll_poll(ll_slot(ll_local, f, epoch, h, (long long)K + mid), flag, ob, t_start, f.timeout_ns) && ok;
-                    if ((long long)ob < my_id) a = mid + 1; else b = mid;
-                }
-                lo = a;
-            }
-            rank += lo;
-        }
-        if (rank < K) {
-            f.merged[rank] = __double_as_longlong(sort_key_to_f64(key));
-            f.merged[K + rank] = my_id;
-        }
-    }
-    if (!ok) atomicExch(f.xstatus, SX_ERR_PEER_TIMEOUT);
+    // the stage ring holds the G * K keys: the rank tiles are no longer read
+    if (!merge_ll(ll_local, f.block_len, f.G, K, epoch, mc, n_merge, reinterpret_cast<unsigned long long *>(smem_raw),
+                  s_fold, f.merged, f.merged + K, f.merged + 2 * K, f.merged + 2 * K + 1, f.timeout_ns))
+        atomicExch(f.xstatus, SX_ERR_PEER_TIMEOUT);
     if (mc == n_merge - 1 && tid == 0) ctl->ts[6] = global_timer_ns();      // end of the merge (diagnostics)
 }
 

@@ -1,7 +1,9 @@
-// sx_ll.cuh -- flag-in-data ("LL") slots of the multi-GPU exchange (sx_exchange.cu, sx_topk.cu, sx_fused.cu).
+// sx_ll.cuh -- flag-in-data ("LL") slots of the multi-GPU exchange (sx_exchange.cu, sx_merge.cuh, sx_fused.cu).
 // Every 8-byte word travels as one 16-byte store {lo32, flag, hi32, flag} with flag = (uint32) epoch; the
 // receiver polls a slot until both flags show the epoch (16-byte stores are single transactions, each
 // 8-byte half is written atomically), so no fence, no separate flag and no second NVLink round trip.
+// A buffer is [2][G][block_len] slots (the half is the parity of the epoch) followed by the counters
+// {push epoch, push CTAs done, merge epoch, merge CTAs done}.
 #pragma once
 #include "sx_common.cuh"
 
@@ -11,6 +13,27 @@ __device__ __forceinline__ unsigned long long global_timer_ns() {
     unsigned long long t;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     return t;
+}
+
+// slot `idx` of rank r's block in the half of `epoch` of the exchange buffer `buf`
+__device__ __forceinline__ uint4 *ll_slot(char *buf, int G, long long block_len, unsigned long long epoch, int r,
+                                          long long idx) {
+    return reinterpret_cast<uint4 *>(buf) + ((size_t)(epoch & 1ull) * G + r) * block_len + idx;
+}
+// the counters after the slots
+__device__ __forceinline__ unsigned long long *ll_counters(char *buf, int G, long long block_len) {
+    return reinterpret_cast<unsigned long long *>(buf + (size_t)2 * G * block_len * 16);
+}
+
+// One thread of each of the n_ctas CTAs calls this when its CTA is done with `epoch`; the last one resets the
+// done count ctr[1] and publishes the epoch in ctr[0] for the next launch.
+__device__ __forceinline__ void advance_epoch_when_last(unsigned long long *ctr, unsigned n_ctas,
+                                                        unsigned long long epoch) {
+    __threadfence();
+    if (atomicAdd(ctr + 1, 1ull) == (unsigned long long)(n_ctas - 1)) {
+        ctr[1] = 0ull;
+        *reinterpret_cast<volatile unsigned long long *>(ctr) = epoch;
+    }
 }
 
 __device__ __forceinline__ void ll_store_slot(uint4 *slot, unsigned flag, unsigned long long v) {

@@ -20,57 +20,41 @@
 //   into one pass many times -- can keep the list long; the selection is then void and raises
 //   SX_STATUS_DUPLICATE_CANDIDATES in the pricing header.
 // K > 1024: two stable radix argsorts (by id, then by rc) over the candidates.
-// Merge of G sorted, padded per-GPU lists after the exchange (sx_topk_merge): an element's position is
-// the number of entries below it in every list (binary searches).
+// Merge of G sorted, padded per-GPU lists after the exchange (sx_topk_merge, sx_topk_merge_ll): an element's
+// position is the number of entries below it in every list, by the rank step, header fold and final write of
+// sx_merge.cuh, which the in-kernel merge of the fused pass (sx_fused.cu) runs as well.  Above 2^22 elements a
+// prefix bound over the (key, id) order first limits the elements that are ranked.
 #include <math.h>
 
 #include <cooperative_groups.h>
 
 #include "sx_common.cuh"
 #include "sx_select.cuh"
-#include "sx_ll.cuh"
+#include "sx_merge.cuh"
 
 namespace cg = cooperative_groups;
 
 namespace sx {
 
-struct Cand {
-    double    rc;
-    long long id;
-};
-__device__ __forceinline__ Cand cand_pad() { return Cand{INFINITY, -1}; }
-// padding must sort after every real candidate: compare as (+inf, max id)
-__device__ __forceinline__ bool cand_less_p(const Cand &a, const Cand &b) {
-    const long long ia = a.id < 0 ? 0x7fffffffffffffffll : a.id;
-    const long long ib = b.id < 0 ? 0x7fffffffffffffffll : b.id;
-    return a.rc < b.rc || (a.rc == b.rc && ia < ib);
+// (key, id) of entry `off` of a block; padding (id < 0) sorts last
+__device__ __forceinline__ KeyId merge_load(const double *rc, const long long *id, long long off) {
+    const long long i = id[off];
+    return i < 0 ? KeyId{~0ull, 0x7fffffffffffffffll} : KeyId{f64_to_sort_key(rc[off]), i};
 }
-
-__device__ __forceinline__ Cand shfl_xor_cand(const Cand &c, int mask) {
-    Cand r;
-    r.rc = __shfl_xor_sync(0xffffffffu, c.rc, mask);
-    r.id = __shfl_xor_sync(0xffffffffu, c.id, mask);
-    return r;
-}
-
-// number of elements of a sorted, padded list prefix [0, len) that are  < x  (strict)
-__device__ __forceinline__ int lower_bound_list(const double *rc, const long long *id, int len, const Cand &x) {
+// entries of the sorted block prefix [0, len) below x (or_equal: not above x)
+__device__ __forceinline__ int bound_list(const double *rc, const long long *id, int len, const KeyId &x, bool or_equal) {
     int lo = 0, hi = len;
     while (lo < hi) {
         const int mid = (lo + hi) >> 1;
-        const Cand m{rc[mid], id[mid]};
-        if (cand_less_p(m, x)) lo = mid + 1; else hi = mid;
+        const KeyId m = merge_load(rc, id, mid);
+        if (or_equal ? !keyid_less(x, m) : keyid_less(m, x)) lo = mid + 1; else hi = mid;
     }
     return lo;
 }
-// number of elements <= x
-__device__ __forceinline__ int upper_bound_list(const double *rc, const long long *id, int len, const Cand &x) {
+// real entries of the block prefix [0, len): the index of the first padding entry (ids are -1 from there on)
+__device__ __forceinline__ int real_len(const long long *id, int len) {
     int lo = 0, hi = len;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        const Cand m{rc[mid], id[mid]};
-        if (!cand_less_p(x, m)) lo = mid + 1; else hi = mid;
-    }
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if (id[mid] >= 0) lo = mid + 1; else hi = mid; }
     return lo;
 }
 
@@ -83,18 +67,8 @@ __global__ void __launch_bounds__(1024)
 topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restrict__ lists_id, long long LS, int L,
                  int K, int *__restrict__ plen, int *__restrict__ poff, double *__restrict__ out_rc, long long *__restrict__ out_id,
                  long long *out_n, const long long *headers, long long *out_summary) {
-    // outputs start as padding; the rank kernel (next launch) overwrites the first out_n entries
-    for (int i = threadIdx.x; i < K; i += blockDim.x) { out_rc[i] = INFINITY; out_id[i] = -1; }
-    if (headers && out_summary && threadIdx.x == 0) {
-        // fold the per-rank pricing headers {n_violating, min_rc_key}: total, min, largest single count
-        long long tot = 0, mn = 0x7fffffffffffffffll, mx = 0, stt = 0;
-        for (int l = 0; l < L; ++l) {
-            const long long c = headers[(long long)l * LS], k = headers[(long long)l * LS + 1];
-            tot += c; mn = k < mn ? k : mn; mx = c > mx ? c : mx; stt |= headers[(long long)l * LS + 3];
-        }
-        out_summary[0] = tot; out_summary[1] = mn; out_summary[2] = mx; out_summary[3] = stt;
-    }
-    __shared__ Cand s_thr[32];
+    __shared__ MergeFold s_fold;
+    __shared__ KeyId s_thr[32];
     __shared__ int  s_warp[32];
     __shared__ int  s_carry;
     const int lane = lane_id(), warp = threadIdx.x >> 5;
@@ -108,33 +82,32 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
         for (int w = 0; w < 32; ++w) t += s_red[w];
         return t;
     };
-    auto block_min_cand = [&](Cand c, bool want_max) -> Cand {
+    auto block_min_keyid = [&](KeyId c, bool want_max) -> KeyId {
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
-            const Cand other = shfl_xor_cand(c, o);
-            if (cand_less_p(other, c) != want_max) c = other;
+            const KeyId other{__shfl_xor_sync(0xffffffffu, c.key, o), __shfl_xor_sync(0xffffffffu, c.id, o)};
+            if (keyid_less(other, c) != want_max) c = other;
         }
         __syncthreads();
         if (lane == 0) s_thr[warp] = c;
         __syncthreads();
-        Cand r = s_thr[0];
-        for (int w = 1; w < 32; ++w) if (cand_less_p(s_thr[w], r) != want_max) r = s_thr[w];
+        KeyId r = s_thr[0];
+        for (int w = 1; w < 32; ++w) if (keyid_less(s_thr[w], r) != want_max) r = s_thr[w];
         return r;
     };
+    merge_fold_init(s_fold);
     if (threadIdx.x == 0) s_carry = 0;
-    // bound 1: the smallest "last element of a list" (padding = +inf: no constraint)
-    Cand thr = cand_pad();
+    __syncthreads();
+    // bound 1: the smallest "last element of a list" (padding: no constraint)
+    KeyId thr{~0ull, 0x7fffffffffffffffll};
     long long n_real_lists = 0;
     for (int l = threadIdx.x; l < L; l += blockDim.x) {
-        const long long *ids = lists_id + (long long)l * LS;
-        const Cand c{lists_rc[(long long)l * LS + K - 1], ids[K - 1]};
-        if (cand_less_p(c, thr)) thr = c;
-        int lo = 0, hi = K;                              // real length of the list: first padding entry
-        while (lo < hi) { const int mid = (lo + hi) >> 1; if (ids[mid] >= 0) lo = mid + 1; else hi = mid; }
-        plen[l] = lo;
-        n_real_lists += lo;
+        const KeyId c = merge_load(lists_rc, lists_id, (long long)l * LS + K - 1);
+        if (keyid_less(c, thr)) thr = c;
+        plen[l] = real_len(lists_id + (long long)l * LS, K);
+        n_real_lists += plen[l];
     }
-    thr = block_min_cand(thr, false);
+    thr = block_min_keyid(thr, false);
     // bound 2: the smallest depth i with sum_l min(len_l, i) >= K; the union of the depth-i prefixes
     // already holds K elements, so the global K-th best is <= the largest element among them.  Much
     // tighter than bound 1 when there are many lists.
@@ -147,16 +120,16 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
             for (int l = threadIdx.x; l < L; l += blockDim.x) part += plen[l] < mid ? plen[l] : mid;
             if (block_sum(part) >= K) hi = mid; else lo = mid + 1;
         }
-        Cand deep = Cand{-INFINITY, 0};
+        KeyId deep{0ull, -1};                          // below every entry
         for (int l = threadIdx.x; l < L; l += blockDim.x) {
             const int take = plen[l] < lo ? plen[l] : lo;
             if (take > 0) {
-                const Cand c{lists_rc[(long long)l * LS + take - 1], lists_id[(long long)l * LS + take - 1]};
-                if (cand_less_p(deep, c)) deep = c;
+                const KeyId c = merge_load(lists_rc, lists_id, (long long)l * LS + take - 1);
+                if (keyid_less(deep, c)) deep = c;
             }
         }
-        deep = block_min_cand(deep, true);
-        if (cand_less_p(deep, thr)) thr = deep;
+        deep = block_min_keyid(deep, true);
+        if (keyid_less(deep, thr)) thr = deep;
     }
     __syncthreads();
     // prefix lengths and their exclusive scan, 1024 lists per sweep
@@ -164,13 +137,8 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
     for (int base = 0; base < L; base += blockDim.x) {
         const int l = base + threadIdx.x;
         int len = 0;
-        if (l < L) len = upper_bound_list(lists_rc + (long long)l * LS, lists_id + (long long)l * LS, K, thr);
-        // do not count padding (id < 0) that ties with an all-padding threshold
-        if (l < L && len > 0) {
-            int lo = 0, hi = len;                       // first padding entry within [0, len)
-            while (lo < hi) { const int mid = (lo + hi) >> 1; if (lists_id[(long long)l * LS + mid] >= 0) lo = mid + 1; else hi = mid; }
-            len = lo;
-        }
+        // without padding that ties with an all-padding threshold
+        if (l < L) len = real_len(lists_id + (long long)l * LS, bound_list(lists_rc + (long long)l * LS, lists_id + (long long)l * LS, K, thr, true));
         int incl = len;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
@@ -187,10 +155,15 @@ topk_prep_kernel(const double *__restrict__ lists_rc, const long long *__restric
         __syncthreads();
         real_total = s_carry;
     }
-    if (threadIdx.x == 0) {
-        poff[L] = (int)real_total;
-        *out_n = real_total < K ? real_total : K;
-    }
+    if (headers)
+        for (int l = threadIdx.x; l < L; l += blockDim.x) {
+            const long long *h = headers + (long long)l * LS;
+            merge_fold_header(s_fold, h[0], h[1], h[3]);
+        }
+    if (threadIdx.x == 0) { poff[L] = (int)real_total; s_fold.real = (int)real_total; }
+    __syncthreads();
+    // the rank kernel (next launch) writes the first out_n entries
+    merge_write_tail(s_fold, K, reinterpret_cast<long long *>(out_rc), out_id, out_n, out_summary);
 }
 
 // Rank merge, step 2: one WARP per surviving element; lanes split the lists, each does a binary
@@ -207,17 +180,17 @@ topk_rank_kernel(const double *__restrict__ lists_rc, const long long *__restric
         int lo = 0, hi = L;
         while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (poff[mid] <= w) lo = mid; else hi = mid; }
         const int l = lo, i = (int)(w - poff[l]);
-        const Cand c{lists_rc[(long long)l * LS + i], lists_id[(long long)l * LS + i]};
+        const KeyId c = merge_load(lists_rc, lists_id, (long long)l * LS + i);
         int rank = 0;
         for (int m = lane; m < L; m += 32) {
             if (m == l) rank += i;
             else {
                 const int len = plen[m];
-                if (len) rank += lower_bound_list(lists_rc + (long long)m * LS, lists_id + (long long)m * LS, len, c);
+                if (len) rank += bound_list(lists_rc + (long long)m * LS, lists_id + (long long)m * LS, len, c, false);
             }
         }
         rank = warp_sum(rank);
-        if (lane == 0 && rank < K) { out_rc[rank] = c.rc; out_id[rank] = c.id; }
+        if (lane == 0 && rank < K) { out_rc[rank] = lists_rc[(long long)l * LS + i]; out_id[rank] = c.id; }
     }
 }
 
@@ -252,15 +225,9 @@ topk_select_kernel(const double *__restrict__ cand_rc, const long long *__restri
     }
 }
 
-// Merge of G sorted, padded blocks of K (exchanged between G ranks).  One thread per element: its
-// position in the merged order is its index in its own block plus, for every other block, the number
-// of entries below it (binary search; (rc, id) is a strict total order and ids are distinct across
-// blocks).  G * 10 dependent L1/L2 loads per element instead of an all-pairs pass over G * K.
-__device__ __forceinline__ KeyId merge_load(const double *rc, const long long *id, long long off) {
-    const long long i = id[off];
-    return i < 0 ? KeyId{~0ull, 0x7fffffffffffffffll} : KeyId{f64_to_sort_key(rc[off]), i};
-}
-
+// Merge of G sorted, padded blocks of K (exchanged between G ranks): one thread per element, ranked by
+// merge_rank (sx_merge.cuh).  The keys of every block are staged in shared memory when they fit (coalesced
+// loads, then ~G * 10 shared loads per element); otherwise the blocks are searched in global memory.
 __global__ void __launch_bounds__(1024)
 merge_rank_kernel(const double *blocks_rc, const long long *blocks_id, long long LS, int G,
                   int K, const long long *headers, double *__restrict__ out_rc, long long *__restrict__ out_id,
@@ -272,187 +239,60 @@ merge_rank_kernel(const double *blocks_rc, const long long *blocks_id, long long
         if (headers) headers += off;
     }
     const int n = G * K;
-    // Stage every block's (key, id) in shared memory when it fits (coalesced loads, then ~G * 10 shared
-    // loads per element); otherwise search the blocks in global memory.
     extern __shared__ __align__(16) unsigned char mg_raw[];
-    KeyId *stage = reinterpret_cast<KeyId *>(mg_raw);
-    __shared__ int s_real;
-    __shared__ long long s_hdr[4];
-    if (threadIdx.x == 0) { s_real = 0; s_hdr[0] = 0; s_hdr[1] = 0x7fffffffffffffffll; s_hdr[2] = 0; s_hdr[3] = 0; }
-    __syncthreads();
-    int my_real = 0;
-    if (use_smem) {
+    unsigned long long *mkey = reinterpret_cast<unsigned long long *>(mg_raw);
+    __shared__ MergeFold s_fold;
+    merge_fold_init(s_fold);
+    if (use_smem)
         for (int e = threadIdx.x; e < n; e += blockDim.x) {
             const int g = e / K;
-            const KeyId v = merge_load(blocks_rc, blocks_id, (long long)g * LS + (e - g * K));
-            stage[e] = v;
-            my_real += v.key != ~0ull;
+            mkey[e] = f64_to_sort_key(blocks_rc[(long long)g * LS + (e - g * K)]);
         }
-    }
-    if (blockIdx.x == 0) {
-        if (!use_smem) {
-            // real entries per block = first padding slot (ids are -1 from there on)
-            for (int g = threadIdx.x; g < G; g += blockDim.x) {
-                int lo = 0, hi = K;
-                while (lo < hi) { const int mid = (lo + hi) >> 1; if (blocks_id[(long long)g * LS + mid] >= 0) lo = mid + 1; else hi = mid; }
-                my_real += lo;
-            }
-        }
-        my_real = warp_sum(my_real);
-        if (lane_id() == 0 && my_real) atomicAdd(&s_real, my_real);
-        if (headers && out_summary) {
-            // fold the per-rank pricing headers: total count, min key, largest single count, status bits
-            for (int g = threadIdx.x; g < G; g += blockDim.x) {
-                const long long *h = headers + (long long)g * LS;
-                atomicAdd((unsigned long long *)&s_hdr[0], (unsigned long long)h[0]);
-                atomicMin(&s_hdr[1], h[1]);
-                atomicMax(&s_hdr[2], h[0]);
-                atomicOr((unsigned long long *)&s_hdr[3], (unsigned long long)h[3]);
-            }
-        }
-    }
     __syncthreads();
     if (blockIdx.x == 0) {
-        const int n_out = s_real < K ? s_real : K;             // outputs past the total are padding
-        for (int i = n_out + threadIdx.x; i < K; i += blockDim.x) { out_rc[i] = INFINITY; out_id[i] = -1; }
-        if (threadIdx.x == 0) {
-            *out_n = n_out;
-            if (headers && out_summary) {
-                out_summary[0] = s_hdr[0]; out_summary[1] = s_hdr[1]; out_summary[2] = s_hdr[2]; out_summary[3] = s_hdr[3];
-            }
+        int real = 0;
+        for (int g = threadIdx.x; g < G; g += blockDim.x) {
+            real += real_len(blocks_id + (long long)g * LS, K);
+            if (headers) { const long long *h = headers + (long long)g * LS; merge_fold_header(s_fold, h[0], h[1], h[3]); }
         }
+        merge_fold_real(s_fold, real);
+        __syncthreads();
+        merge_write_tail(s_fold, K, reinterpret_cast<long long *>(out_rc), out_id, out_n, out_summary);
     }
+    const auto key_at = [&](int h, int j) {
+        return use_smem ? mkey[h * K + j] : f64_to_sort_key(blocks_rc[(long long)h * LS + j]);
+    };
+    const auto id_at = [&](int h, int j) { return blocks_id[(long long)h * LS + j]; };
     for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {
         const int g = e / K, i = e - g * K;
-        const KeyId mine = use_smem ? stage[e] : merge_load(blocks_rc, blocks_id, (long long)g * LS + i);
-        if (mine.key == ~0ull) continue;                       // padding
-        int rank = i;
-        for (int h = 0; h < G && rank < K; ++h) {
-            if (h == g) continue;
-            const long long base = (long long)h * LS;
-            int lo = 0, hi = K;
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                const KeyId other = use_smem ? stage[h * K + mid] : merge_load(blocks_rc, blocks_id, base + mid);
-                if (keyid_less(other, mine)) lo = mid + 1; else hi = mid;
-            }
-            rank += lo;
-        }
-        if (rank < K) { out_rc[rank] = blocks_rc[(long long)g * LS + i]; out_id[rank] = mine.id; }
+        const long long id = id_at(g, i);
+        if (id < 0) continue;                                  // padding
+        const int rank = merge_rank(key_at(g, i), id, g, i, G, K, key_at, id_at);
+        if (rank < K) { out_rc[rank] = blocks_rc[(long long)g * LS + i]; out_id[rank] = id; }
     }
 }
 
-// Merge straight out of the LL exchange buffer (sx_exchange_push_ll): staging a block in shared memory
-// IS the wait for it -- every slot is polled until both of its flags show this epoch.
+// Merge straight out of the LL exchange buffer (sx_exchange_push_ll) by merge_ll (sx_merge.cuh), with all CTAs
+// of the grid: staging a block in shared memory IS the wait for it.
 __global__ void __launch_bounds__(1024)
 merge_ll_kernel(char *ll_buf, long long block_len, int G, int K, double *__restrict__ out_rc,
                 long long *__restrict__ out_id, long long *out_n, long long *out_summary, int *status,
                 unsigned long long timeout_ns) {
     extern __shared__ __align__(16) unsigned char mg_raw[];
-    KeyId *stage = reinterpret_cast<KeyId *>(mg_raw);
-    __shared__ int s_real;
-    __shared__ long long s_hdr[4];
-    const size_t slots_bytes = (size_t)2 * G * block_len * 16;
+    __shared__ MergeFold s_fold;
     // The merge keeps an epoch counter of its own ([2], [3] = CTAs done), advanced once per launch like the
     // pushing side's ([0], [1]): it depends on no other kernel of this GPU, so it may be launched with
     // programmatic stream serialisation and become resident while the pricing kernel is still draining.
-    unsigned long long *mctr = reinterpret_cast<unsigned long long *>(ll_buf + slots_bytes) + 2;
+    unsigned long long *mctr = ll_counters(ll_buf, G, block_len) + 2;
     const unsigned long long epoch = *reinterpret_cast<volatile unsigned long long *>(mctr) + 1ull;
-    const unsigned flag = (unsigned)epoch;
-    const uint4 *slots = reinterpret_cast<const uint4 *>(ll_buf) + (size_t)(epoch & 1ull) * G * block_len;
-    if (threadIdx.x == 0) { s_real = 0; s_hdr[0] = 0; s_hdr[1] = 0x7fffffffffffffffll; s_hdr[2] = 0; s_hdr[3] = 0; }
-    __syncthreads();
-    unsigned long long t0;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-    const int n = G * K;
-    int my_real = 0;
-    bool ok = true;
-    // kLlBatch elements per thread are requested before any is examined (one L2 round trip per batch
-    // when the data is already there); a slot that is not ready yet is polled again by ll_poll
-    constexpr int kLlBatch = 4;
-    for (int e0 = threadIdx.x; e0 < n; e0 += blockDim.x * kLlBatch) {
-        uint4 wr[kLlBatch], wi[kLlBatch];
-#pragma unroll
-        for (int u = 0; u < kLlBatch; ++u) {
-            const int e = e0 + u * blockDim.x;
-            if (e < n) {
-                const int g = e / K, i = e - g * K;
-                const uint4 *blk = slots + (size_t)g * block_len;
-                asm volatile("ld.volatile.global.v4.u32 {%0, %1, %2, %3}, [%4];"
-                             : "=r"(wr[u].x), "=r"(wr[u].y), "=r"(wr[u].z), "=r"(wr[u].w) : "l"(blk + i) : "memory");
-                asm volatile("ld.volatile.global.v4.u32 {%0, %1, %2, %3}, [%4];"
-                             : "=r"(wi[u].x), "=r"(wi[u].y), "=r"(wi[u].z), "=r"(wi[u].w) : "l"(blk + K + i) : "memory");
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < kLlBatch; ++u) {
-            const int e = e0 + u * blockDim.x;
-            if (e >= n) continue;
-            const int g = e / K, i = e - g * K;
-            const uint4 *blk = slots + (size_t)g * block_len;
-            unsigned long long rc_bits = (unsigned long long)wr[u].x | ((unsigned long long)wr[u].z << 32);
-            unsigned long long id_bits = (unsigned long long)wi[u].x | ((unsigned long long)wi[u].z << 32);
-            if (wr[u].y != flag || wr[u].w != flag) ok = ll_poll(blk + i, flag, rc_bits, t0, timeout_ns) && ok;
-            if (wi[u].y != flag || wi[u].w != flag) ok = ll_poll(blk + K + i, flag, id_bits, t0, timeout_ns) && ok;
-            const long long id = (long long)id_bits;
-            const KeyId v = (id < 0 || !ok) ? KeyId{~0ull, 0x7fffffffffffffffll}
-                                            : KeyId{f64_to_sort_key(__longlong_as_double((long long)rc_bits)), id};
-            stage[e] = v;
-            my_real += v.key != ~0ull;
-        }
-    }
-    if (blockIdx.x == 0) {
-        my_real = warp_sum(my_real);
-        if (lane_id() == 0 && my_real) atomicAdd(&s_real, my_real);
-        for (int g = threadIdx.x; g < G; g += blockDim.x) {      // fold the per-rank pricing headers
-            const uint4 *hdr = slots + (size_t)g * block_len + 2 * K;
-            unsigned long long h0, h1, h3;
-            ok = ll_poll(hdr, flag, h0, t0, timeout_ns) && ok;
-            ok = ll_poll(hdr + 1, flag, h1, t0, timeout_ns) && ok;
-            ok = ll_poll(hdr + 3, flag, h3, t0, timeout_ns) && ok;
-            atomicAdd((unsigned long long *)&s_hdr[0], h0);
-            atomicMin(&s_hdr[1], (long long)h1);
-            atomicMax(&s_hdr[2], (long long)h0);
-            atomicOr((unsigned long long *)&s_hdr[3], h3);
-        }
-    }
-    if (!ok) atomicExch(status, SX_ERR_PEER_TIMEOUT);
-    __syncthreads();
-    if (blockIdx.x == 0) {
-        const int n_out = s_real < K ? s_real : K;
-        for (int i = n_out + threadIdx.x; i < K; i += blockDim.x) { out_rc[i] = INFINITY; out_id[i] = -1; }
-        if (threadIdx.x == 0) {
-            *out_n = n_out;
-            if (out_summary) { out_summary[0] = s_hdr[0]; out_summary[1] = s_hdr[1]; out_summary[2] = s_hdr[2]; out_summary[3] = s_hdr[3]; }
-        }
-    }
-    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {
-        const int g = e / K, i = e - g * K;
-        const KeyId mine = stage[e];
-        if (mine.key == ~0ull) continue;
-        int rank = i;
-        for (int h = 0; h < G && rank < K; ++h) {
-            if (h == g) continue;
-            int lo = 0, hi = K;
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                if (keyid_less(stage[h * K + mid], mine)) lo = mid + 1; else hi = mid;
-            }
-            rank += lo;
-        }
-        if (rank < K) { out_rc[rank] = sort_key_to_f64(mine.key); out_id[rank] = mine.id; }
-    }
+    if (!merge_ll(ll_buf, block_len, G, K, epoch, blockIdx.x, gridDim.x, reinterpret_cast<unsigned long long *>(mg_raw),
+                  s_fold, reinterpret_cast<long long *>(out_rc), out_id, out_n, out_summary, timeout_ns))
+        atomicExch(status, SX_ERR_PEER_TIMEOUT);
     // not done before the kernel this one was (programmatically) serialised after: what follows in the
     // stream may rely on both
     asm volatile("griddepcontrol.wait;" ::: "memory");
     __syncthreads();
-    if (threadIdx.x == 0) {                       // the last CTA to finish advances the merge epoch
-        __threadfence();
-        if (atomicAdd(mctr + 1, 1ull) == (unsigned long long)(gridDim.x - 1)) {
-            mctr[1] = 0ull;
-            *reinterpret_cast<volatile unsigned long long *>(mctr) = epoch;
-        }
-    }
+    if (threadIdx.x == 0) advance_epoch_when_last(mctr, gridDim.x, epoch);
 }
 
 // ---- large-K path helpers ---------------------------------------------------------------
@@ -561,7 +401,7 @@ extern "C" int sx_topk_merge(const double *blocks_rc, const int64_t *blocks_id, 
     if (!ws || ws_bytes < sx_topk_merge_workspace_bytes(G)) return SX_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     if (G * K <= (1 << 22)) {
-        const size_t stage_bytes = (size_t)G * K * sizeof(KeyId);
+        const size_t stage_bytes = (size_t)G * K * sizeof(unsigned long long);
         const int use_smem = stage_bytes <= 200 * 1024;
         const int threads = use_smem ? 1024 : 256;
         long long mg = (G * K + threads - 1) / threads;
@@ -592,8 +432,8 @@ extern "C" int sx_topk_merge_ll(void *ll_buf_local, int64_t block_len, int64_t G
                                 void *stream) {
     if (!ll_buf_local || G <= 0 || K <= 0 || block_len < 2 * K + 4 || !out_rc || !out_id || !out_n || !status_dev)
         return SX_ERR_INVALID;
-    const size_t stage_bytes = (size_t)G * K * sizeof(KeyId);
-    if (stage_bytes > 200 * 1024) return SX_ERR_TOO_LARGE;
+    if ((size_t)G * K * 16 > 200 * 1024) return SX_ERR_TOO_LARGE;     // the ABI limit (keys and ids once)
+    const size_t stage_bytes = (size_t)G * K * sizeof(unsigned long long);
     SX_CUDA(cudaFuncSetAttribute(merge_ll_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     long long mg = (G * K + 1023) / 1024;
     cudaLaunchConfig_t cfg = {};

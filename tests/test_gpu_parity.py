@@ -707,18 +707,24 @@ def test_price_row_slabs_and_merge(dev):
 def test_topk_merge_above_the_one_thread_per_element_size(dev):
     """sx_topk_merge with G * K > 2^22 (5 blocks of 2^20, 84 MB as an all-gathered (G, 2K + 4) buffer) runs the
     prefix bound + rank merge.  Sorted, padded blocks with many rc ties, tails of padding and one block that is
-    all padding, against a NumPy lexsort of all real entries; the pricing headers fold into the summary."""
+    all padding, against a NumPy lexsort of all real entries; the pricing headers fold into the summary.  In the
+    last case -0.0 and +0.0 (violators when tol < 0) sit in different blocks: they are one sort key, so the arc
+    id orders them, as in the selection and in the merge below 2^22 elements."""
     G, K = 5, 1 << 20
     rng = np.random.default_rng(2024)
-    for n_real in ([K, K - 12345, 0, K // 3, 777], [1000, 0, 0, 5000, 3]):
+    for n_real, zeros in (([K, K - 12345, 0, K // 3, 777], False), ([1000, 0, 0, 5000, 3], False),
+                          ([K // 2, 0, 3000, K, 20000], True)):
         ids_all = rng.permutation(sum(n_real)).astype(np.int64) * 3 + 7      # distinct across blocks
         buf = np.zeros((G, 2 * K + 4), dtype=np.int64)
         rc_real, id_real, off = [], [], 0
         for g, n in enumerate(n_real):
-            rc = -1.0 - np.round(rng.random(n) * 1000) / 1000                # about a thousand distinct values
+            if zeros:
+                rc = rng.choice([-1.0, -0.0, 0.0], n)
+            else:
+                rc = -1.0 - np.round(rng.random(n) * 1000) / 1000            # about a thousand distinct values
             ids = ids_all[off:off + n]
             off += n
-            o = np.lexsort((ids, rc))
+            o = np.lexsort((ids, rc + 0.0))                                  # sort-key image: -0.0 + 0.0 = +0.0
             buf[g, :K] = np.float64(np.inf).view(np.int64)
             buf[g, K:2 * K] = -1
             buf[g, :n] = rc[o].view(np.int64)
@@ -727,7 +733,7 @@ def test_topk_merge_above_the_one_thread_per_element_size(dev):
             rc_real.append(rc)
             id_real.append(ids)
         rc_real, id_real = np.concatenate(rc_real), np.concatenate(id_real)
-        o = np.lexsort((id_real, rc_real))[:K]
+        o = np.lexsort((id_real, rc_real + 0.0))[:K]
         gathered = cu(buf)
         out_rc, out_id, out_n, summary = dev.topk_merge(gathered[:, :K].view(torch.float64), gathered[:, K:2 * K],
                                                         gathered[:, 2 * K:])
@@ -785,6 +791,69 @@ def test_ll_exchange_and_merge_with_emulated_ranks(dev, G, K):
         stack = torch.stack(blocks)
         o_rc, o_id, o_n = dev.topk_merge(stack[:, :K].view(torch.float64), stack[:, K:2 * K])
         assert int(o_n.item()) == k and np.array_equal(o_id[:k].cpu().numpy(), whole.topk_id)
+
+
+@pytest.mark.parametrize("G,K", [(2, 1024), (8, 1024), (5, 33), (3, 1), (8, 4096)])
+def test_merges_break_cross_block_ties_by_arc_id(dev, G, K):
+    """Hand-built blocks whose reduced costs take four values, so most entries tie with entries of other blocks
+    and the arc id decides; tails of padding and one all-padding block.  Pushed with sx_exchange_push_ll into G
+    emulated ranks' buffers, sx_topk_merge_ll out of every buffer and sx_topk_merge on the same blocks (shared
+    memory at 8 x 1024, global memory at 8 x 4096) both equal a NumPy lexsort, bit for bit, over two epochs."""
+    from smart_crossover._native import check, lib
+    blk = 2 * K + dev.Pricer.BLOCK_TAIL
+    ll_fits = G * K * 16 <= 200 * 1024
+    bufs = [torch.zeros(lib.sx_exchange_ll_buffer_bytes(blk, G) // 8, dtype=torch.int64, device="cuda")
+            for _ in range(G)]
+    ptrs = torch.tensor([b.data_ptr() for b in bufs], dtype=torch.int64, device="cuda")
+    status = torch.zeros(1, dtype=torch.int32, device="cuda")
+    rng = np.random.default_rng(G * 10007 + K)
+    for epoch in range(2):
+        n_real = rng.integers(K // 2, K + 1, G)
+        n_real[0] = K
+        n_real[1] = 0
+        ids_all = rng.permutation(int(n_real.sum())).astype(np.int64) * 5 + 3
+        host = np.zeros((G, blk), dtype=np.int64)
+        rc_real, id_real, off = [], [], 0
+        for g, n in enumerate(n_real):
+            rc = -1.0 - rng.integers(0, 4, n) / 8.0
+            ids = ids_all[off:off + n]
+            off += n
+            o = np.lexsort((ids, rc))
+            host[g, :K] = np.float64(np.inf).view(np.int64)
+            host[g, K:2 * K] = -1
+            host[g, :n] = rc[o].view(np.int64)
+            host[g, K:K + n] = ids[o]
+            host[g, 2 * K:2 * K + 5] = [n, rng.integers(-1000, 1000), 0, 8 * (g == 2), n]
+            rc_real.append(rc)
+            id_real.append(ids)
+        rc_real, id_real = np.concatenate(rc_real), np.concatenate(id_real)
+        o = np.lexsort((id_real, rc_real))[:K]
+        hdr = host[:, 2 * K:2 * K + 4]
+        summary = [int(hdr[:, 0].sum()), int(hdr[:, 1].min()), int(hdr[:, 0].max()), int(np.bitwise_or.reduce(hdr[:, 3]))]
+        stack = cu(host)
+
+        def expect(out_rc, out_id, n):
+            assert n == o.size
+            assert np.array_equal(out_id[:n], id_real[o]) and out_rc[:n].tobytes() == rc_real[o].tobytes()
+            assert np.all(out_id[n:] == -1) and np.all(np.isposinf(out_rc[n:]))
+
+        o_rc, o_id, o_n, o_sum = dev.topk_merge(stack[:, :K].view(torch.float64), stack[:, K:2 * K],
+                                                stack[:, 2 * K:2 * K + 4])
+        expect(o_rc.cpu().numpy(), o_id.cpu().numpy(), int(o_n.item()))
+        assert o_sum.cpu().numpy().tolist() == summary
+        for g in range(G):
+            check(lib.sx_exchange_push_ll(dev._ptr(stack[g]), blk, dev._ptr(ptrs), g, G, dev._stream()), "push")
+        for g in range(G):
+            out = torch.zeros(2 * K + 6, dtype=torch.int64, device="cuda")
+            rc = lib.sx_topk_merge_ll(dev._ptr(bufs[g]), blk, G, K, dev._ptr(out[:K]), dev._ptr(out[K:2 * K]),
+                                      dev._ptr(out[2 * K:]), dev._ptr(out[2 * K + 1:]), dev._ptr(status), dev._stream())
+            if not ll_fits:
+                assert rc == -4                         # SX_ERR_TOO_LARGE: G * K * 16 > 200 KB
+                continue
+            check(rc, "merge_ll")
+            h = out.cpu().numpy()
+            expect(h[:K].view(np.float64), h[K:2 * K], int(h[2 * K]))
+            assert h[2 * K + 1:2 * K + 5].tolist() == summary and int(status.item()) == 0
 
 
 @pytest.mark.parametrize("G,K", [(2, 128), (8, 1024), (5, 33), (3, 1)])
