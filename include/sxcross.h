@@ -300,6 +300,33 @@ SX_API int    sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0,
                                int64_t block_len, void *const *peer_bufs_dev, int rank, int G,
                                int64_t *merged_out, int32_t *status_dev, void *ws, size_t ws_bytes, void *stream);
 
+/* ---- lower-bound copy of a cost slab: the fused pass streams 4 B per arc instead of 8 ----------
+ * sx_cost_lb_build writes lb[i * ld_lb + j] = the high 32 bits of the fp64 bit pattern of M[i * ld + j],
+ * rounded toward -inf (one streaming kernel).  Read back as the high half of a double with a zero low half,
+ * L <= M element by element, or L is NaN:
+ *   values whose low half is 0 (+-0, +-inf, and every value with at most 20 mantissa bits) are exact;
+ *   other positive values truncate; other negative values step one unit away from zero (at -DBL_MAX and
+ *   below: -inf); a NaN keeps its sign and exponent and gets the quiet bit (0x00080000), so it stays NaN.
+ *   lb: 16 B aligned device memory, ld_lb >= D and a multiple of 4 (16 B TMA row stride); columns
+ *   [D, ld_lb) are not written.  sx_cost_lb_bytes(S_loc, D) sizes a copy with ld_lb = D rounded up to 4.
+ * sx_price_dense_ot_fused_lb = sx_price_dense_ot_fused (same arguments and results, bit for bit) that may
+ *   stream the copy: each arc whose lower-bound reduced cost L - (v - u) is below max(running min, -tol)
+ *   (or NaN) is re-read from M and priced exactly; no other arc can be a violator or a new minimum.  The
+ *   copy pays off while few arcs violate, so a pass streams M itself when the previous pass on the same
+ *   state had more than a fixed fraction of its arcs violating (the first pass of a state streams the
+ *   copy).  lb == NULL is sx_price_dense_ot_fused.  The copy must be built from the M passed here, and M
+ *   must not change while the copy is in use.
+ */
+SX_API size_t sx_cost_lb_bytes(int64_t S_loc, int64_t D);
+SX_API int    sx_cost_lb_build(const double *M, int64_t ld, int64_t S_loc, int64_t D, uint32_t *lb, int64_t ld_lb,
+                               void *stream);
+SX_API int    sx_price_dense_ot_fused_lb(const double *M, int64_t ld, const uint32_t *lb, int64_t ld_lb, int64_t row0,
+                                         int64_t S_loc, int64_t D, const double *y_src, const double *y_dst,
+                                         double tol, sx_fused_state *state, double *cand_rc, int64_t *cand_id,
+                                         int64_t cand_cap, int64_t K, int64_t *block, int64_t block_len,
+                                         void *const *peer_bufs_dev, int rank, int G, int64_t *merged_out,
+                                         int32_t *status_dev, void *ws, size_t ws_bytes, void *stream);
+
 /* ---- top-k most violating arcs (north_star extension; SURVEY.md section 8 row a9) -------
  * Among the candidates (rc, id) left by a pricing pass select the K smallest by (rc ascending,
  * id ascending).  sel / header are the pass's selection state and header (the candidate count
@@ -397,9 +424,11 @@ SX_API int    sx_sinkhorn_ot(const double *M, int64_t ld, int64_t S, int64_t D, 
  * row-shards the cost matrix over the ndev GPUs it is given: device g prices rows [S g / ndev, S (g+1) / ndev)
  * with ONE kernel per pass (sx_price_dense_ot_fused: price + select + NVLink push + merge).  Single process,
  * plain function calls; not thread-safe (one caller at a time), like the reference's managers.
- *   slabs[g]: DEVICE pointer (on device devs[g], caller-owned, resident for the life of the pricer) to that
- *     row range of M, row-major with leading dimension ld (even ld and 16-byte aligned slabs select the
- *     TMA / fused path; anything else is priced by the scalar-load kernels).
+ *   slabs[g]: DEVICE pointer (on device devs[g], caller-owned, resident and unchanged for the life of the
+ *     pricer) to that row range of M, row-major with leading dimension ld (even ld and 16-byte aligned slabs
+ *     select the TMA / fused path; anything else is priced by the scalar-load kernels).  On the fused path
+ *     the pricer builds and owns a lower-bound copy of each slab (sx_cost_lb_build, half the slab's bytes)
+ *     and prices with sx_price_dense_ot_fused_lb; if that allocation fails it streams the slab itself.
  *   row_bounds (HOST, ndev + 1 entries, may be NULL): shard g holds rows [row_bounds[g], row_bounds[g + 1]);
  *     NULL = the equal partition above.  GPUs of one box stream at rates a few percent apart and a pass ends
  *     when the slowest has delivered its block, so callers may size the shards by measured rate.

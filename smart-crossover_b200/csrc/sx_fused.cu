@@ -7,7 +7,9 @@
 //
 //   start    every CTA clears its slice of the OTHER selection state (the pricer owns two, used by
 //            alternate passes), so no pass ever waits for a clear;
-//   pricing  the TMA pipeline of sx_price_tma.cuh, unchanged: count, min, candidate list + histogram;
+//   pricing  the TMA pipeline of sx_price_tma.cuh: count, min, candidate list + histogram.  With a lower-bound
+//            copy of the slab (sx_cost_lb_build) it streams the copy and re-reads the exact fp64 cost of the
+//            few arcs the copy flags; after a dense pass (many violators) it streams M itself;
 //   barrier  grid-wide (the kernel is launched cooperatively: all CTAs are resident);
 //   select   select_topk (sx_select.cuh), the selection topk_select_kernel runs too: a candidate list of at
 //            most kDirectCap is ranked as it is; a longer one is first split by the histogram's bound b*
@@ -26,6 +28,7 @@
 // If the candidate buffer overflowed, the pass raises SX_STATUS_CAND_OVERFLOW in the header -- it still
 // pushes a well-formed block so that no peer waits -- and the caller grows the buffer and repeats the pass.
 #include <stdlib.h>
+#include <string.h>
 
 #include "sx_gridbar.cuh"
 #include "sx_merge.cuh"
@@ -39,9 +42,12 @@ struct FusedCtl {
     unsigned long long pass;      // passes completed; parity selects the selection state in use
     GridBarrier        bar;       // grid-wide barrier (sx_gridbar.cuh)
     unsigned int       dyn_ctr;   // tail stealing of the pricing walk: next dynamically assigned tile (0 between passes)
-    unsigned int       pad[3];
+    unsigned int       walk;      // diagnostics: 1 = the last pass streamed the lower-bound copy, 0 = fp64 M
+    unsigned long long n_violating_last;   // violators of the last pass on this slab: picks the next pass's walk
     unsigned long long ts[8];     // diagnostics: %globaltimer of CTA 0 at the phase boundaries of the last pass
 };
+// Pricer.fused_walk reads `walk` 12 bytes before the timestamps
+static_assert(offsetof(FusedCtl, ts) - offsetof(FusedCtl, walk) == 12, "");
 struct FusedState {
     SelState sel[2];
     FusedCtl ctl;
@@ -64,6 +70,8 @@ struct FusedParams {
     int             *xstatus;        // SX_ERR_PEER_TIMEOUT lands here
     unsigned long long timeout_ns;
     int              steal;          // 1: the last eighth of the tiles is handed out dynamically
+    int              has_lb;         // 1: the lower-bound copy is there (second tensor map)
+    unsigned long long lb_max_violating;   // walk the copy while the last pass had at most this many violators
 };
 
 __device__ __forceinline__ unsigned long long ld_volatile_u64(const unsigned long long *p) {
@@ -75,11 +83,17 @@ __device__ __forceinline__ void stamp(FusedCtl *ctl, int i) {
     if (blockIdx.x == 0 && threadIdx.x == 0) ctl->ts[i] = global_timer_ns();
 }
 
-template <int ROWS, int STAGES, int CWARPS, int MINB>
+// 2 CTAs per SM hold at most 96 registers per thread: the 18 warps land 5 / 5 / 4 / 4 on the SM's four
+// sub-partitions, whose register files hold 16 384 registers each (112 per thread would pass a whole-SM count
+// but leave one CTA per SM).
+template <int ROWS, int STAGES, int LB_STAGES, int CWARPS, int MINB>
 __global__ void __launch_bounds__((CWARPS + 1) * 32, MINB)
-price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p0, const FusedParams f) {
+price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_lb,
+                   const DenseParams p0, const FusedParams f) {
     static_assert((size_t)STAGES * ROWS * kBoxCols * sizeof(double) >= sizeof(SelScratch),
                   "the stage ring is reused as the selection's shared memory");
+    static_assert((size_t)LB_STAGES * ROWS * kBoxCols * sizeof(uint32_t) == (size_t)STAGES * ROWS * kBoxCols * sizeof(double),
+                  "both walks use the same ring (the barriers follow it)");
     static_assert(CWARPS * 32 == kSelThreads, "the consumer warps select, the producer warp joins the barriers");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ MergeFold s_fold;
@@ -111,7 +125,13 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
     p.sink.hdr = &sel->hdr;
     p.sink.sel = sel;
     p.dyn_ctr = f.steal ? &ctl->dyn_ctr : nullptr;
-    price_tiles<ROWS, STAGES, CWARPS, false>(tmap, p, smem_raw);
+    // The walk of this pass: the lower-bound copy (4 B per arc, flagged arcs re-read from M) unless the last
+    // pass on this state was dense, where the re-reads would cost more than the fp64 walk (DESIGN.md 5).
+    // n_violating_last is written after barrier 1 of a pass, so every CTA reads the same value here.
+    const bool lb_walk = f.has_lb && ld_volatile_u64(&ctl->n_violating_last) <= f.lb_max_violating;
+    if (lb_walk) price_tiles<uint32_t, ROWS, LB_STAGES, CWARPS, false>(tmap_lb, p, smem_raw);
+    else         price_tiles<double, ROWS, STAGES, CWARPS, false>(tmap, p, smem_raw);
+    if (blockIdx.x == 0 && tid == 0) ctl->walk = lb_walk ? 1u : 0u;
     stamp(ctl, 1);
 
     grid_barrier(&ctl->bar);      // header, histogram and candidate list of this pass are complete
@@ -162,7 +182,7 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p
         }
         if (tid < 6) {
             unsigned long long w = 0;
-            if (tid == 0) w = __ldcg(&sel->hdr.n_violating);
+            if (tid == 0) { w = __ldcg(&sel->hdr.n_violating); ctl->n_violating_last = w; }
             if (tid == 1) w = (unsigned long long)__ldcg(&sel->hdr.min_rc_key);
             if (tid == 2) w = __ldcg(&sel->hdr.n_priced);
             if (tid == 3)
@@ -200,8 +220,15 @@ __global__ void __launch_bounds__(256) fused_init_kernel(FusedState *st, unsigne
     if (blockIdx.x == 0 && threadIdx.x < sizeof(FusedCtl) / 4) reinterpret_cast<unsigned *>(&st->ctl)[threadIdx.x] = 0u;
 }
 
-// the one pipeline shape the fused kernel is built for: 16 rows x 3 stages, 8 consumer warps, 2 CTAs per SM
-constexpr int kFRows = 16, kFStages = 3, kFWarps = 8, kFMinB = 2;
+// the one pipeline shape the fused kernel is built for: 16 rows x 3 stages (fp64; 6 stages of the 4-byte copy: the
+// same 96 KB ring), 8 consumer warps, 2 CTAs per SM
+constexpr int kFRows = 16, kFStages = 3, kFLbStages = 6, kFWarps = 8, kFMinB = 2;
+
+// The lower-bound walk is chosen while the last pass had at most this fraction of the slab's arcs violating.
+// Measured at 20 000^2 on a B200 (DESIGN.md 5): the copy walk takes 0.37 / 0.42 / 0.57 / 1.07 ms at 1e-5 /
+// 1e-4 / 1e-3 / 1e-2 violating, the fp64 walk 0.46 / 0.46 / 0.48 / 0.64 ms: they cross near 5e-4.
+// SX_FUSED_LB_MAX_FRAC overrides it (to measure the crossover).
+constexpr double kLbMaxViolatingFrac = 1.0 / 2048;
 
 }  // namespace sx
 
@@ -229,6 +256,17 @@ extern "C" int sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0
                                        int64_t K, int64_t *block, int64_t block_len, void *const *peer_bufs_dev,
                                        int rank, int G, int64_t *merged_out, int32_t *status_dev, void *ws,
                                        size_t ws_bytes, void *stream) {
+    return sx_price_dense_ot_fused_lb(M, ld, nullptr, 0, row0, S_loc, D, y_src, y_dst, tol, state, cand_rc, cand_id,
+                                      cand_cap, K, block, block_len, peer_bufs_dev, rank, G, merged_out, status_dev, ws,
+                                      ws_bytes, stream);
+}
+
+extern "C" int sx_price_dense_ot_fused_lb(const double *M, int64_t ld, const uint32_t *lb, int64_t ld_lb, int64_t row0,
+                                          int64_t S_loc, int64_t D, const double *y_src, const double *y_dst,
+                                          double tol, sx_fused_state *state, double *cand_rc, int64_t *cand_id,
+                                          int64_t cand_cap, int64_t K, int64_t *block, int64_t block_len,
+                                          void *const *peer_bufs_dev, int rank, int G, int64_t *merged_out,
+                                          int32_t *status_dev, void *ws, size_t ws_bytes, void *stream) {
     if (!M || !y_src || !y_dst || !state || !block || S_loc <= 0 || D <= 0 || ld < D || row0 < 0 || cand_cap < 0)
         return SX_ERR_INVALID;
     if (K < 1 || K > SX_TOPK_MAX_K || block_len < 2 * K + 6) return SX_ERR_INVALID;
@@ -238,19 +276,23 @@ extern "C" int sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0
     if (merged_out && !sx_fused_merge_fits(K, G)) return SX_ERR_TOO_LARGE;
     if (!ws || ws_bytes < sx_topk_workspace_bytes(cand_cap, K)) return SX_ERR_WORKSPACE;
     if (((uintptr_t)M % 16) != 0 || (ld % 2) != 0) return SX_ERR_UNALIGNED;
+    if (lb && ld_lb < D) return SX_ERR_INVALID;
+    if (lb && (((uintptr_t)lb % 16) != 0 || (ld_lb % 4) != 0)) return SX_ERR_UNALIGNED;   // 16 B TMA row stride
     if (D >= (1ll << 31) || S_loc >= (1ll << 31)) return SX_ERR_TOO_LARGE;
     cudaStream_t st = (cudaStream_t)stream;
 
     DenseParams p;
-    p.y_src = y_src; p.y_dst = y_dst; p.S_loc = S_loc; p.D = D; p.row0 = row0; p.thr = -tol;
+    p.y_src = y_src; p.y_dst = y_dst; p.M = M; p.ld = ld; p.S_loc = S_loc; p.D = D; p.row0 = row0; p.thr = -tol;
     p.sink.hdr = nullptr; p.sink.sel = nullptr;                   // set on the device from the pass parity
     p.sink.rc = cand_rc; p.sink.id = (int64_t *)cand_id; p.sink.cap = cand_cap;
     p.rc_out = nullptr; p.ld_out = 0; p.zero = 0; p.evict_first = 1; p.dyn_ctr = nullptr;
     p.n_col_blocks = (D + kBoxCols - 1) / kBoxCols;
     p.n_row_tiles = (S_loc + kFRows - 1) / kFRows;
-    CUtensorMap map;
+    CUtensorMap map, map_lb;
     int rc = encode_slab_map(&map, M, ld, S_loc, D, kFRows, /*l2_promotion=*/3);
     if (rc != SX_OK) return rc;
+    memset(&map_lb, 0, sizeof(map_lb));
+    if (lb && (rc = encode_slab_map(&map_lb, lb, ld_lb, S_loc, D, kFRows, /*l2_promotion=*/3)) != SX_OK) return rc;
 
     FusedParams f;
     f.state = (FusedState *)state; f.cand_rc = cand_rc; f.cand_id = (const long long *)cand_id; f.cand_cap = cand_cap;
@@ -261,9 +303,15 @@ extern "C" int sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0
     static int steal = -1;
     if (steal < 0) { const char *e = getenv("SX_FUSED_STEAL"); steal = (e && e[0] == '0') ? 0 : 1; }
     f.steal = steal;
+    static double lb_frac = -1.0;
+    if (lb_frac < 0) { const char *e = getenv("SX_FUSED_LB_MAX_FRAC"); lb_frac = e ? atof(e) : kLbMaxViolatingFrac; }
+    f.has_lb = lb ? 1 : 0;
+    f.lb_max_violating = (unsigned long long)(lb_frac * (double)S_loc * (double)D);
 
-    auto kern = price_fused_kernel<kFRows, kFStages, kFWarps, kFMinB>;
-    constexpr size_t smem = tma_smem_bytes(kFRows, kFStages, kFWarps);
+    auto kern = price_fused_kernel<kFRows, kFStages, kFLbStages, kFWarps, kFMinB>;
+    constexpr size_t smem_f64 = tma_smem_bytes(kFRows, kFStages, kFWarps),
+                     smem_lb = tma_smem_bytes(kFRows, kFLbStages, kFWarps, sizeof(uint32_t));
+    constexpr size_t smem = smem_f64 > smem_lb ? smem_f64 : smem_lb;
     constexpr int threads = (kFWarps + 1) * 32;
     static int occ_cached[64] = {0};
     int dev = 0;
@@ -279,7 +327,7 @@ extern "C" int sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0
     const long long total = p.n_row_tiles * p.n_col_blocks;
     long long grid = (long long)num_sms() * occ_cached[dev];
     if (grid > total) grid = total;
-    void *args[] = {(void *)&map, (void *)&p, (void *)&f};
+    void *args[] = {(void *)&map, (void *)&map_lb, (void *)&p, (void *)&f};
     // cooperative: the grid-wide barriers need every CTA resident (a plain launch measured the same speed)
     SX_CUDA(cudaLaunchCooperativeKernel((void *)kern, dim3((unsigned)grid), dim3(threads), args, smem, st));
     return SX_OK;

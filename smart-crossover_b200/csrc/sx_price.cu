@@ -21,7 +21,7 @@ template <int ROWS, int STAGES, int CWARPS, int MINB, bool WRITE_RC>
 __global__ void __launch_bounds__((CWARPS + 1) * 32, MINB)
 price_dense_tma_kernel(const __grid_constant__ CUtensorMap tmap, const DenseParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    price_tiles<ROWS, STAGES, CWARPS, WRITE_RC>(tmap, p, smem_raw);
+    price_tiles<double, ROWS, STAGES, CWARPS, WRITE_RC>(tmap, p, smem_raw);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -334,9 +334,47 @@ static int dispatch_tma(int shape, const CUtensorMap &map, const DenseParams &p,
     }
 }
 
+// High word of x's fp64 bit pattern, rounded toward -inf: as the high half of a double (low half 0) it is
+// <= x, or NaN when x is NaN.  Positive values and exact ones (low half 0: +-0, +-inf) truncate; a negative
+// value with a nonzero low half steps one unit away from zero (-DBL_MAX and below become -inf); a NaN keeps
+// its sign and exponent and gets the quiet bit, so its payload cannot vanish into the dropped half.
+__device__ __forceinline__ uint32_t cost_lb_word(double x) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(x);
+    const uint32_t hi = (uint32_t)(b >> 32), lo = (uint32_t)b;
+    if (x != x) return hi | 0x00080000u;
+    return (lo != 0 && (hi >> 31)) ? hi + 1u : hi;
+}
+
+// Lower-bound copy of a slab (sx_cost_lb_build): one streaming pass, coalesced rows.
+__global__ void __launch_bounds__(256) cost_lb_kernel(const double *__restrict__ M, long long ld, long long S_loc,
+                                                      long long D, uint32_t *__restrict__ lb, long long ld_lb) {
+    for (long long i = blockIdx.x; i < S_loc; i += gridDim.x) {
+        const double *src = M + i * ld;
+        uint32_t *dst = lb + i * ld_lb;
+        for (long long j = threadIdx.x; j < D; j += blockDim.x) dst[j] = cost_lb_word(__ldcs(src + j));
+    }
+}
+
 }  // namespace sx
 
 using namespace sx;
+
+extern "C" size_t sx_cost_lb_bytes(int64_t S_loc, int64_t D) {
+    if (S_loc <= 0 || D <= 0) return 0;
+    return (size_t)S_loc * (size_t)((D + 3) & ~(int64_t)3) * sizeof(uint32_t);
+}
+
+extern "C" int sx_cost_lb_build(const double *M, int64_t ld, int64_t S_loc, int64_t D, uint32_t *lb, int64_t ld_lb,
+                                void *stream) {
+    if (!M || !lb || S_loc < 0 || D <= 0 || ld < D || ld_lb < D) return SX_ERR_INVALID;
+    if (((uintptr_t)lb % 16) != 0 || (ld_lb % 4) != 0) return SX_ERR_UNALIGNED;
+    if (S_loc == 0) return SX_OK;
+    long long grid = (long long)num_sms() * 8;
+    if (grid > S_loc) grid = S_loc;
+    cost_lb_kernel<<<(int)grid, 256, 0, (cudaStream_t)stream>>>(M, ld, S_loc, D, lb, ld_lb);
+    SX_LAUNCH_CHECK();
+    return SX_OK;
+}
 
 extern "C" int sx_price_set_tma_options(int l2_promotion, int evict_first) {
     if (l2_promotion > 3) return SX_ERR_INVALID;
@@ -379,7 +417,7 @@ extern "C" int sx_price_dense_ot(const double *M, int64_t ld, int64_t row0, int6
     if (variant == 0 && (D >= (1ll << 31) || S_loc >= (1ll << 31))) variant = 1;
 
     DenseParams p;
-    p.y_src = y_src; p.y_dst = y_dst; p.S_loc = S_loc; p.D = D; p.row0 = row0; p.thr = -tol;
+    p.y_src = y_src; p.y_dst = y_dst; p.M = M; p.ld = ld; p.S_loc = S_loc; p.D = D; p.row0 = row0; p.thr = -tol;
     p.sink.hdr = header; p.sink.sel = (SelState *)sel; p.sink.rc = cand_rc; p.sink.id = (int64_t *)cand_id;
     p.sink.cap = cand_cap;
     p.rc_out = rc_out; p.ld_out = ld_out; p.zero = 0; p.evict_first = (uint32_t)g_tma_evict_first;

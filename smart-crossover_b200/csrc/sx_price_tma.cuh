@@ -6,6 +6,8 @@
 #include <cuda.h>
 #include <math.h>
 
+#include <type_traits>
+
 #include "sx_common.cuh"
 #include "sx_select.cuh"
 
@@ -179,11 +181,13 @@ __device__ __forceinline__ void block_min_commit(double tmin, sx_price_header *h
 // ---------------------------------------------------------------------------------------
 // K4a, variant 0: TMA pipeline
 // ---------------------------------------------------------------------------------------
-constexpr int kBoxCols = 256;   // fp64 elements per box row (TMA max box dim)
+constexpr int kBoxCols = 256;   // elements per box row (TMA max box dim)
 
 struct DenseParams {
     const double *y_src;   // S_loc
     const double *y_dst;   // D
+    const double *M;       // the slab itself: the lower-bound walk re-reads flagged arcs from it
+    long long     ld;
     long long     S_loc, D, row0;
     double        thr;     // -tol
     CandSink      sink;
@@ -227,15 +231,31 @@ __device__ __forceinline__ void tile_epilogue(const DenseParams &p, WarpTally &t
 }
 
 // CWARPS consumer warps: 4 warps span the 256 box columns (2 adjacent columns per thread, so a
-// warp reads 512 contiguous bytes of a box row: conflict-free LDS.128), CWARPS/4 row groups.
+// warp reads 512 (fp64) / 256 (fp32) contiguous bytes of a box row: conflict-free), CWARPS/4 row groups.
 // The whole pricing pass of one CTA as a device function (shared by price_dense_tma_kernel and the fused
 // price + select + push kernel, sx_fused.cu).  Returns after a __syncthreads(): every TMA load of this CTA
 // has been consumed, so the caller may reuse the shared memory.
-template <int ROWS, int STAGES, int CWARPS, bool WRITE_RC>
+//
+// T = double: the map streams M itself (8 B per arc).
+// T = uint32_t: the map streams the lower-bound copy (sx_cost_lb_build, 4 B per arc): the high word of each
+//   fp64 cost rounded toward -inf, so L = that word as the high half of a double (low half 0) -- a register
+//   move, not a conversion -- and M is re-read from global memory only for the arcs L flags.  Why that is
+//   exact: L <= M elementwise (or L is NaN), and fp64 subtraction of the same w = fl(v - u) is monotone, so
+//   rc_lb = fl(L - w) <= fl(M - w) = rc.  The filter flags an arc when !(rc_lb >= lim), lim = max(running min, -tol); an arc it does not
+//   flag has rc >= rc_lb >= lim, so it is neither a violator (rc >= -tol) nor below the running minimum,
+//   and it is not NaN (a NaN rc needs M or w NaN, or M and w infinite of one sign -- L keeps NaN and
+//   infinities, so rc_lb is NaN then too).  Flagged arcs get rc = M - (v - u) from the exact M, the same
+//   operations as the fp64 walk, and unflagged ones enter the epilogue as +inf.  The running minimum is
+//   only ever updated from exact values, so count, minimum, NaN status and candidates are those of the
+//   fp64 walk, bit for bit.
+template <class T, int ROWS, int STAGES, int CWARPS, bool WRITE_RC>
 __device__ __forceinline__ void price_tiles(const CUtensorMap &tmap, const DenseParams &p, unsigned char *smem_raw) {
+    static_assert(sizeof(T) == 8 || !WRITE_RC, "the lower-bound walk does not write reduced costs");
+    static_assert(std::is_same<T, double>::value || std::is_same<T, uint32_t>::value, "fp64 M or its lower-bound words");
+    using T2 = typename std::conditional<sizeof(T) == 8, double2, uint2>::type;
     constexpr int      RPT         = ROWS / (CWARPS / 4);      // rows per consumer thread
-    constexpr uint32_t kStageBytes = ROWS * kBoxCols * sizeof(double);
-    double   *stage_base = reinterpret_cast<double *>(smem_raw);
+    constexpr uint32_t kStageBytes = ROWS * kBoxCols * sizeof(T);
+    T        *stage_base = reinterpret_cast<T *>(smem_raw);
     uint64_t *full_bar   = reinterpret_cast<uint64_t *>(smem_raw + (size_t)STAGES * kStageBytes);
     uint64_t *empty_bar  = full_bar + STAGES;
     long long *scratch   = reinterpret_cast<long long *>(empty_bar + STAGES);
@@ -325,9 +345,9 @@ __device__ __forceinline__ void price_tiles(const CUtensorMap &tmap, const Dense
                 for (int r = 0; r < RPT; ++r) u[r] = (i0 + r < p.S_loc) ? __ldg(p.y_src + i0 + r) : 0.0;
             }
             if (!waited) mbar_wait(&full_bar[s], (it / STAGES) & 1);
-            const double2 *tile = reinterpret_cast<const double2 *>(stage_base + (size_t)s * ROWS * kBoxCols) +
-                                  (size_t)rg * RPT * (kBoxCols / 2) + c;
-            double2 m[RPT];
+            const T2 *tile = reinterpret_cast<const T2 *>(stage_base + (size_t)s * ROWS * kBoxCols) +
+                             (size_t)rg * RPT * (kBoxCols / 2) + c;
+            T2 m[RPT];
 #pragma unroll
             for (int r = 0; r < RPT; ++r) m[r] = tile[(size_t)r * (kBoxCols / 2)];
             // Release the slot once the data has ARRIVED in registers: the vote below cannot issue before
@@ -335,10 +355,48 @@ __device__ __forceinline__ void price_tiles(const CUtensorMap &tmap, const Dense
             // address depends on the vote.
             uint32_t landed = 0;
 #pragma unroll
-            for (int r = 0; r < RPT; ++r) landed ^= (uint32_t)__double2loint(m[r].x);
+            for (int r = 0; r < RPT; ++r) {
+                if constexpr (sizeof(T) == 8) landed ^= (uint32_t)__double2loint(m[r].x);
+                else landed ^= m[r].x;
+            }
             const bool rel = __any_sync(0xffffffffu, landed == 0x5a5a5a5au);
             if (lane_id() == 0) mbar_arrive_after(&empty_bar[s], (uint32_t)rel * p.zero);
 
+            if constexpr (sizeof(T) == 4) {
+                // lower-bound filter: two fp64 subtractions and one compare per arc, as the fp64 walk
+                auto L = [](uint32_t w) { return __hiloint2double((int)w, 0); };
+                const bool ok0 = j0 < p.D, ok1 = j0 + 1 < p.D;
+                bool hit = false;
+                if (interior) {
+#pragma unroll
+                    for (int r = 0; r < RPT; ++r)
+                        hit = lt_or(L(m[r].y) - (v1 - u[r]), lim, lt_or(L(m[r].x) - (v0 - u[r]), lim, hit));
+                } else {
+#pragma unroll
+                    for (int r = 0; r < RPT; ++r) {
+                        const bool rok = i0 + r < p.S_loc;
+                        const bool f0 = lt_or(L(m[r].x) - (v0 - u[r]), lim, false);
+                        const bool f1 = lt_or(L(m[r].y) - (v1 - u[r]), lim, false);
+                        hit = hit || (rok && ((f0 && ok0) || (f1 && ok1)));
+                    }
+                }
+                if (!__any_sync(0xffffffffu, hit)) return;
+                // rare path: the exact fp64 M of the flagged arcs, the reduced costs rebuilt as the fp64 walk
+                // builds them, +inf for the others
+                double rc0[RPT], rc1[RPT];
+                const double *row = p.M + i0 * p.ld + j0;
+#pragma unroll
+                for (int r = 0; r < RPT; ++r) {
+                    const bool rok = interior || i0 + r < p.S_loc;
+                    const double w0 = v0 - u[r], w1 = v1 - u[r];
+                    const bool f0 = rok && (interior || ok0) && lt_or(L(m[r].x) - w0, lim, false);
+                    const bool f1 = rok && (interior || ok1) && lt_or(L(m[r].y) - w1, lim, false);
+                    rc0[r] = f0 ? __ldg(row + (long long)r * p.ld) - w0 : INFINITY;
+                    rc1[r] = f1 ? __ldg(row + (long long)r * p.ld + 1) - w1 : INFINITY;
+                }
+                tile_epilogue<RPT>(p, tally, tmin, lim, rc0, rc1, hit, (p.row0 + i0) * p.D + j0, p.D);
+                return;
+            }
             double rc0[RPT], rc1[RPT];
             bool   hit = false;
             if (interior) {
@@ -407,8 +465,8 @@ __device__ __forceinline__ void price_tiles(const CUtensorMap &tmap, const Dense
     __syncthreads();
 }
 
-constexpr size_t tma_smem_bytes(int rows, int stages, int cwarps) {
-    return (size_t)stages * rows * kBoxCols * sizeof(double) + 2 * (size_t)stages * sizeof(uint64_t) +
+constexpr size_t tma_smem_bytes(int rows, int stages, int cwarps, size_t elem_bytes = sizeof(double)) {
+    return (size_t)stages * rows * kBoxCols * elem_bytes + 2 * (size_t)stages * sizeof(uint64_t) +
            2 * (size_t)cwarps * sizeof(long long) + (size_t)stages * sizeof(long long) + 64;   // + tickets, counts
 }
 
@@ -433,16 +491,19 @@ inline EncodeTiledFn get_encode_fn() {
     return fn;
 }
 
-// 2-D fp64 map {D columns, S_loc rows}, box {256, rows}.  l2_promotion 0..3 = none / 64 / 128 / 256 B.
-inline int encode_slab_map(CUtensorMap *map, const double *M, int64_t ld, int64_t S_loc, int64_t D, int rows,
+// 2-D map {D columns, S_loc rows}, box {256, rows}, over fp64 M or (T = uint32_t) its lower-bound copy.
+// l2_promotion 0..3 = none / 64 / 128 / 256 B.
+template <class T>
+inline int encode_slab_map(CUtensorMap *map, const T *M, int64_t ld, int64_t S_loc, int64_t D, int rows,
                            int l2_promotion) {
     EncodeTiledFn enc = get_encode_fn();
     if (!enc) return SX_ERR_NO_DEVICE;
     cuuint64_t gdim[2]    = {(cuuint64_t)D, (cuuint64_t)S_loc};
-    cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(double)};
+    cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(T)};
     cuuint32_t box[2]     = {(cuuint32_t)kBoxCols, (cuuint32_t)rows};
     cuuint32_t estr[2]    = {1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, (void *)M, gdim, gstride, box, estr,
+    const CUtensorMapDataType dt = sizeof(T) == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_UINT32;
+    CUresult r = enc(map, dt, 2, (void *)M, gdim, gstride, box, estr,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
                      (CUtensorMapL2promotion)l2_promotion, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { g_last_cuda_error = (int)r; return SX_ERR_CUDA; }

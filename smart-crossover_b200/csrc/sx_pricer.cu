@@ -10,7 +10,9 @@
 // ONE kernel (sx_price_dense_ot_fused: price + select + NVLink push + merge) and reads the merged result
 // back; the threads run concurrently, so the GPUs start within microseconds of each other and the caller
 // sees a plain function call (SURVEY.md section 8e "process model").
-// The cost-matrix slabs are caller-owned device memory (the managers upload M once per problem).
+// The cost-matrix slabs are caller-owned device memory (the managers upload M once per problem).  On the fused
+// path the pricer builds one lower-bound copy per slab at create (sx_cost_lb_build: high words rounded toward
+// -inf, half the slab's bytes) and the fused pass streams it while few arcs violate.
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -32,6 +34,8 @@ struct DevCtx {
     int dev = 0, g = 0;
     cudaStream_t st = nullptr;
     const double *M = nullptr;
+    uint32_t *lb = nullptr;                            // lower-bound copy of M (owned), or nullptr: stream M itself
+    int64_t ld_lb = 0;
     int64_t row0 = 0, S_loc = 0;
     double *y_loc = nullptr;
     double *cand_rc = nullptr;
@@ -108,11 +112,11 @@ int run_pass(sx_ot_pricer *p, DevCtx *c) {
     const int64_t cap = p->K > 0 ? p->cap : 0;
     int32_t *xstatus = reinterpret_cast<int32_t *>(c->merged + 2 * Kp + 5);
     if (p->fusable) {
-        SXP(sx_price_dense_ot_fused(c->M, p->ld, c->row0, c->S_loc, D, c->y_loc, c->y_loc + c->S_loc, p->tol,
-                                    (sx_fused_state *)c->fstate, c->cand_rc, c->cand_id, cap, Kp, c->block, p->blk,
-                                    p->G > 1 ? c->peer_bufs_dev : nullptr, c->g, p->G,
-                                    (p->G > 1 && p->merge_in_kernel) ? c->merged : nullptr, xstatus, c->topk_ws,
-                                    c->topk_ws_bytes, c->st));
+        SXP(sx_price_dense_ot_fused_lb(c->M, p->ld, c->lb, c->ld_lb, c->row0, c->S_loc, D, c->y_loc,
+                                       c->y_loc + c->S_loc, p->tol, (sx_fused_state *)c->fstate, c->cand_rc,
+                                       c->cand_id, cap, Kp, c->block, p->blk, p->G > 1 ? c->peer_bufs_dev : nullptr,
+                                       c->g, p->G, (p->G > 1 && p->merge_in_kernel) ? c->merged : nullptr, xstatus,
+                                       c->topk_ws, c->topk_ws_bytes, c->st));
     } else {
         sx_price_header *hdr = reinterpret_cast<sx_price_header *>(c->block + 2 * Kp);
         SXP(sx_price_pass_begin(hdr, (sx_select_state *)c->sel, p->K, c->st));
@@ -202,7 +206,7 @@ void free_ctx(DevCtx *c) {
     cudaSetDevice(c->dev);
     if (c->st) cudaStreamSynchronize(c->st);
     void *dev_ptrs[] = {c->y_loc, c->cand_rc, c->cand_id, c->fstate, c->sel, c->topk_ws, c->block, c->merged, c->ll_buf,
-                        c->peer_bufs_dev};
+                        c->peer_bufs_dev, c->lb};
     for (void *q : dev_ptrs) if (q) cudaFree(q);
     if (c->h_y) cudaFreeHost(c->h_y);
     if (c->h_out) cudaFreeHost(c->h_out);
@@ -228,8 +232,11 @@ extern "C" int sx_ot_pricer_destroy(sx_ot_pricer *p) {
     return SX_OK;
 }
 
-extern "C" int sx_ot_pricer_create(int ndev, const int *devs, const double *const *slabs, const int64_t *row_bounds,
-                                   int64_t ld, int64_t S, int64_t D, int64_t K, double tol, sx_ot_pricer **out) {
+namespace {
+
+// want_lb: build the lower-bound copies (a pricer that prices once, sx_price_dense_ot_h, would only pay for them)
+int ot_pricer_create(int ndev, const int *devs, const double *const *slabs, const int64_t *row_bounds, int64_t ld,
+                     int64_t S, int64_t D, int64_t K, double tol, bool want_lb, sx_ot_pricer **out) {
     if (!out) return SX_ERR_INVALID;
     *out = nullptr;
     if (ndev < 1 || ndev > 64 || !devs || !slabs || S < 1 || D < 1 || ld < D || K < 0) return SX_ERR_INVALID;
@@ -286,6 +293,15 @@ extern "C" int sx_ot_pricer_create(int ndev, const int *devs, const double *cons
             SXA(cudaMalloc(&c->fstate, sx_fused_state_bytes()));
             if ((rc = sx_fused_state_init((sx_fused_state *)c->fstate, Kp, c->st)) != SX_OK) return fail(rc);
         }
+        if (p->fusable && want_lb) {
+            c->ld_lb = (D + 3) & ~(int64_t)3;
+            if (cudaMalloc((void **)&c->lb, sx_cost_lb_bytes(c->S_loc, D)) != cudaSuccess) {
+                cudaGetLastError();                                    // no room for the copy: stream M itself
+                c->lb = nullptr;
+            } else if ((rc = sx_cost_lb_build(c->M, ld, c->S_loc, D, c->lb, c->ld_lb, c->st)) != SX_OK) {
+                return fail(rc);
+            }
+        }
         if (ndev > 1) {
             const size_t nb = sx_exchange_ll_buffer_bytes(p->blk, ndev);
             SXA(cudaMalloc((void **)&c->ll_buf, nb));
@@ -309,6 +325,13 @@ extern "C" int sx_ot_pricer_create(int ndev, const int *devs, const double *cons
     cudaSetDevice(prev);
     *out = p;
     return SX_OK;
+}
+
+}  // namespace
+
+extern "C" int sx_ot_pricer_create(int ndev, const int *devs, const double *const *slabs, const int64_t *row_bounds,
+                                   int64_t ld, int64_t S, int64_t D, int64_t K, double tol, sx_ot_pricer **out) {
+    return ot_pricer_create(ndev, devs, slabs, row_bounds, ld, S, D, K, tol, /*want_lb=*/true, out);
 }
 
 extern "C" int sx_ot_pricer_info(const sx_ot_pricer *p, int g, int *dev, int64_t *row0, int64_t *S_loc) {
@@ -401,7 +424,7 @@ extern "C" int sx_price_dense_ot_h(const double *M_h, const double *M_dev, int64
     }
     sx_ot_pricer *p = nullptr;
     const double *slabs[1] = {M_dev};
-    int rc = sx_ot_pricer_create(1, &dev, slabs, nullptr, ld, S, D, K, tol, &p);
+    int rc = ot_pricer_create(1, &dev, slabs, nullptr, ld, S, D, K, tol, /*want_lb=*/false, &p);
     if (rc == SX_OK) {
         rc = sx_ot_pricer_price_h(p, y_h, y_h + S, n_violating_h, min_rc_h, topk_rc_h, topk_id_h, topk_n_h, nullptr);
         sx_ot_pricer_destroy(p);

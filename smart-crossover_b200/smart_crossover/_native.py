@@ -91,6 +91,10 @@ SIGNATURES = {
     "sx_fused_merge_fits": (_int, [_i64, _int]),
     "sx_price_dense_ot_fused": (_int, [_p, _i64, _i64, _i64, _i64, _p, _p, _dbl, _p, _p, _p, _i64, _i64, _p, _i64,
                                        _p, _int, _int, _p, _p, _p, _sz, _p]),
+    "sx_cost_lb_bytes": (_sz, [_i64, _i64]),
+    "sx_cost_lb_build": (_int, [_p, _i64, _i64, _i64, _p, _i64, _p]),
+    "sx_price_dense_ot_fused_lb": (_int, [_p, _i64, _p, _i64, _i64, _i64, _i64, _p, _p, _dbl, _p, _p, _p, _i64, _i64,
+                                          _p, _i64, _p, _int, _int, _p, _p, _p, _sz, _p]),
     "sx_topk_workspace_bytes": (_sz, [_i64, _i64]),
     "sx_topk_select": (_int, [_p, _p, _i64, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
     "sx_topk_merge_workspace_bytes": (_sz, [_i64]),

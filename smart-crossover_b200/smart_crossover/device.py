@@ -246,14 +246,23 @@ class Pricer:
         return M.data_ptr() % 16 == 0 and ld % 2 == 0
 
     def price_dense_fused(self, M, ld, row0, S_loc, D, y_src, y_dst, tol=TOL_RC, peer_bufs=None, rank=0, G=1,
-                          merged=None, xstatus=None):
+                          merged=None, xstatus=None, lb=None):
         """begin + pricing + selection (+ push of the block to `peer_bufs`, + merge of the G blocks into
-        `merged`) as one launch."""
-        check(lib.sx_price_dense_ot_fused(_ptr(M), ld, row0, S_loc, D, _ptr(y_src), _ptr(y_dst), float(tol),
-                                          _ptr(self.fstate), _ptr(self.cand_rc), _ptr(self.cand_id),
-                                          self.cap if self.K > 0 else 0, self.Kp, _ptr(self.block),
-                                          self.block.numel(), peer_bufs, rank, G, _ptr(merged), _ptr(xstatus),
-                                          _ptr(self.ws), self.ws.numel(), _stream()), "sx_price_dense_ot_fused")
+        `merged`) as one launch.  `lb`: the lower-bound copy of M (`cost_lb`); the pass may then stream it
+        instead of M, with the same results."""
+        if lb is not None:
+            check(lib.sx_price_dense_ot_fused_lb(_ptr(M), ld, _ptr(lb), lb.stride(0), row0, S_loc, D, _ptr(y_src),
+                                                 _ptr(y_dst), float(tol), _ptr(self.fstate), _ptr(self.cand_rc),
+                                                 _ptr(self.cand_id), self.cap if self.K > 0 else 0, self.Kp,
+                                                 _ptr(self.block), self.block.numel(), peer_bufs, rank, G, _ptr(merged),
+                                                 _ptr(xstatus), _ptr(self.ws), self.ws.numel(), _stream()),
+                  "sx_price_dense_ot_fused_lb")
+        else:
+            check(lib.sx_price_dense_ot_fused(_ptr(M), ld, row0, S_loc, D, _ptr(y_src), _ptr(y_dst), float(tol),
+                                              _ptr(self.fstate), _ptr(self.cand_rc), _ptr(self.cand_id),
+                                              self.cap if self.K > 0 else 0, self.Kp, _ptr(self.block),
+                                              self.block.numel(), peer_bufs, rank, G, _ptr(merged), _ptr(xstatus),
+                                              _ptr(self.ws), self.ws.numel(), _stream()), "sx_price_dense_ot_fused")
         self.launches += 1
         self._fused_passes += 1
         self._last_fused = True
@@ -267,6 +276,11 @@ class Pricer:
         out["last_cta_end_(after_merge_if_any)_minus_cta0_rank_end"] = round(float(t[6] - t[5]) * 1e-3, 2)
         out["gap_since_previous_pass_end"] = round(float(t[0] - t[7]) * 1e-3, 2)
         return out
+
+    def fused_walk(self) -> int:
+        """What the last fused pass streamed: 1 = the lower-bound copy, 0 = M itself (diagnostics; synchronises)."""
+        off = lib.sx_fused_state_timestamps_offset() - 12
+        return int(self.fstate[off:off + 4].view(torch.int32).item())
 
     def note_replayed_fused_passes(self, n: int = 1):
         """A captured CUDA graph holding a fused pass was replayed n times (keeps `n_candidates` right)."""
@@ -395,6 +409,17 @@ def topk_merge(blocks_rc: torch.Tensor, blocks_id: torch.Tensor, headers: torch.
     if headers is not None:
         return out_rc, out_id, out_n, summary
     return out_rc, out_id, out_n
+
+
+def cost_lb(M: torch.Tensor) -> torch.Tensor:
+    """Lower-bound copy of a device cost matrix for the fused pass (`sx_cost_lb_build`): the high 32 bits of each
+    fp64 cost rounded toward -inf (int32 bit patterns; as the high half of a double they are <= M element by
+    element), row stride a multiple of 4 words.  Raises torch.OutOfMemoryError when it does not fit."""
+    S, D = M.shape
+    ld_lb = (D + 3) // 4 * 4
+    lb = torch.empty(S, ld_lb, dtype=torch.int32, device=M.device)
+    check(lib.sx_cost_lb_build(_ptr(M), M.stride(0), S, D, _ptr(lb), ld_lb, _stream()), "sx_cost_lb_build")
+    return lb
 
 
 # ---- persistent, row-sharded pricer behind the managers (sx_ot_pricer) --------------------------------

@@ -41,7 +41,9 @@ def block_views(gathered: torch.Tensor, K: int):
 
 class ShardedDensePricer:
     """Pricing of one row slab per rank + global top-K.  `M_loc` is this rank's slab (S_loc x D,
-    row-major, device resident for the life of the problem, like the reference keeps `ot.M`)."""
+    row-major, device resident for the life of the problem, like the reference keeps `ot.M`).  It must not be
+    modified after construction: the fused pass keeps a lower-bound copy of it (`lb`, half its bytes, built
+    here) and streams that copy instead of M while few arcs violate."""
 
     def __init__(self, M_loc: torch.Tensor, S: int, row0: int, K: int, tol: float = dev.TOL_RC,
                  group=None, variant: int = -1, exchange: str = "ll", use_graph: bool = True, fused: bool | None = None,
@@ -55,6 +57,12 @@ class ShardedDensePricer:
         self.fused = bool(dev.FUSED_DEFAULT if fused is None else fused) and variant in (-1, 0) and dev.Pricer.fusable(M_loc, M_loc.stride(0)) \
             and max(self.K, 1) <= _native.SX_TOPK_MAX_K and self.S_loc > 0
         self.pricer = dev.Pricer(M_loc.device, self.K, fused=self.fused)
+        self.lb = None
+        if self.fused:
+            try:
+                self.lb = dev.cost_lb(M_loc)
+            except torch.OutOfMemoryError:              # no room for the copy: every pass streams M itself
+                self.lb = None
         self._merge_launches = 0
         self._dead = False
         self.use_graph = bool(use_graph)
@@ -164,9 +172,10 @@ class ShardedDensePricer:
                 p.price_dense_fused(self.M, self.M.stride(0), self.row0, self.S_loc, self.D, y_src, y_dst, self.tol,
                                     self._hdl.buffer_ptrs_dev, self._rank, self.world,
                                     merged=self.d_out if self.fused_merge else None,
-                                    xstatus=self._xstatus if self.fused_merge else None)
+                                    xstatus=self._xstatus if self.fused_merge else None, lb=self.lb)
             else:
-                p.price_dense_fused(self.M, self.M.stride(0), self.row0, self.S_loc, self.D, y_src, y_dst, self.tol)
+                p.price_dense_fused(self.M, self.M.stride(0), self.row0, self.S_loc, self.D, y_src, y_dst, self.tol,
+                                    lb=self.lb)
             if kernel_events is not None:
                 kernel_events[1].record()
             mark(1)
