@@ -417,6 +417,28 @@ SX_API int    sx_sinkhorn_ot(const double *M, int64_t ld, int64_t S, int64_t D, 
                       int64_t check_every, double *f, double *g, double *x_out, int64_t *iters_h,
                       double *err_h, void *ws, size_t ws_bytes, void *stream);
 
+/* sx_sinkhorn_ot_sharded_h: the same iteration (same order, stopping rule and check_every) over a cost matrix
+ * held as row slabs on several devices, as sx_ot_pricer holds it; one process, one host thread.  Rank g runs
+ * the kernels of sx_sinkhorn_ot on rows [row_bounds[g], row_bounds[g + 1]) of its slab and keeps f for them;
+ * the column half-step exchanges one (max, scaled sum) log-sum-exp pair per column and rank through NVLink
+ * peer stores (two 16-byte flag-in-data slots: 32 B x D from each rank into each of the G buffers per iteration),
+ * and every rank merges the G pairs in rank order, so every rank computes the same g bit for bit.  The stopping
+ * error is summed in a fixed order, so the iteration count does not depend on kernel timing either.  With ndev = 1 the results are those of sx_sinkhorn_ot bit for bit.
+ *   devs / slabs / row_bounds / ld: as sx_ot_pricer_create (row_bounds NULL = equal partition).  A device may
+ *     appear more than once: its ranks then run one after the other on one stream of that device (same
+ *     results as ranks on distinct devices with the same row bounds).  Distinct devices need peer access
+ *     (SX_ERR_NO_DEVICE otherwise).
+ *   a_h (S), b_h (D): HOST marginals.  f_h (S), g_h (D): HOST outputs (g from rank 0).
+ *   x_out (may be NULL): x_out[g] is an S_loc x D DEVICE buffer on devs[g] that receives rank g's rows of X.
+ *   iters_h / err_h (HOST, may be NULL): as sx_sinkhorn_ot; the error of rank 0 decides for every rank.
+ * Blocking; allocates and frees its buffers per call.  SX_ERR_PEER_TIMEOUT when a rank's pair did not arrive
+ * within 10 s. */
+SX_API int    sx_sinkhorn_ot_sharded_h(int ndev, const int *devs, const double *const *slabs,
+                                const int64_t *row_bounds, int64_t ld, int64_t S, int64_t D, const double *a_h,
+                                const double *b_h, double reg, int64_t max_iter, double stop_thr,
+                                int64_t check_every, double *f_h, double *g_h, double *const *x_out,
+                                int64_t *iters_h, double *err_h);
+
 /* ---- host-buffer entry points (what a reference-side binding calls with NumPy arrays) ----
  * sx_ot_pricer: persistent pricer of one dense OT problem for `OTManager.check_optimality_condition`
  * (net_manager.py:485-497, called once per column-generation round from algorithms.py:132).  It owns every

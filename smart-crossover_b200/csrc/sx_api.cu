@@ -17,6 +17,18 @@ int num_sms() {
     }
     return cached[dev];
 }
+
+int enable_peer_access(int dev, int ndev, const int *devs) {
+    for (int h = 0; h < ndev; ++h) {
+        if (devs[h] == dev) continue;
+        int can = 0;
+        if (cudaDeviceCanAccessPeer(&can, dev, devs[h]) != cudaSuccess || !can) return SX_ERR_NO_DEVICE;
+        cudaError_t e = cudaDeviceEnablePeerAccess(devs[h], 0);
+        if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+        else if (e != cudaSuccess) return cuda_fail(e);
+    }
+    return SX_OK;
+}
 }
 using namespace sx;
 

@@ -26,6 +26,10 @@ inline int cuda_fail(cudaError_t e) {
 // persistent / cooperative kernels are sized from it.  Defined in sx_api.cu.
 int num_sms();
 
+// Lets the current device `dev` access the memory of every other distinct device in devs[0..ndev) (entries equal
+// to `dev` are skipped).  SX_ERR_NO_DEVICE when a pair has no peer access.  Defined in sx_api.cu.
+int enable_peer_access(int dev, int ndev, const int *devs);
+
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // Bump allocator over a caller-provided workspace.

@@ -270,14 +270,9 @@ int ot_pricer_create(int ndev, const int *devs, const double *const *slabs, cons
         if (((uintptr_t)c->M & 15) != 0) p->fusable = false;
         if (cudaSetDevice(c->dev) != cudaSuccess) return fail(SX_ERR_NO_DEVICE);
         if (ndev > 1) {
-            for (int h = 0; h < ndev; ++h) {
-                if (h == g) continue;
-                int can = 0;
-                if (cudaDeviceCanAccessPeer(&can, c->dev, devs[h]) != cudaSuccess || !can) return fail(SX_ERR_NO_DEVICE);
-                cudaError_t e = cudaDeviceEnablePeerAccess(devs[h], 0);
-                if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
-                else if (e != cudaSuccess) return fail(cuda_fail(e));
-            }
+            // one GPU per shard: the ranks of a pass wait for each other inside one kernel
+            for (int h = 0; h < ndev; ++h) if (h != g && devs[h] == c->dev) return fail(SX_ERR_NO_DEVICE);
+            if ((rc = enable_peer_access(c->dev, ndev, devs)) != SX_OK) return fail(rc);
         }
 #define SXA(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) return fail(cuda_fail(_e)); } while (0)
         SXA(cudaStreamCreateWithFlags(&c->st, cudaStreamNonBlocking));

@@ -16,10 +16,17 @@
 // The column-marginal error of POT's test is free: with the new f and the old g the column sums of X
 // are b_j exp((g_old_j - g_new_j) / reg), so the error of iteration k is known during the column pass
 // of iteration k + 1 (the loop then stops with that pass's g, one half-step further than POT).
+// sx_sinkhorn_ot_sharded_h runs the same kernels on row slabs spread over several GPUs (the shards sx_ot_pricer
+// prices): the row half-step reads only a slab's own rows; the column half-step exchanges one log-sum-exp pair
+// per column and rank over NVLink (push / fold kernels below) and merges the pairs in rank order on every rank.
 #include <math.h>
+#include <string.h>
+
+#include <vector>
 
 #include "sx_common.cuh"
 #include "sx_expm.cuh"
+#include "sx_ll.cuh"
 
 namespace sx {
 
@@ -63,6 +70,10 @@ __device__ __forceinline__ void lse_add_group(Lse &a, double &wm, const double (
 __device__ __forceinline__ void lse_merge(Lse &a, const Lse &b) {
     if (b.m <= a.m) a.s += b.s * exp(b.m - a.m);
     else { a.s = a.s * exp(a.m - b.m) + b.s; a.m = b.m; }
+}
+// merge of partial accumulators; an empty one (s = 0: masked slots only, or every term underflowed) is skipped
+__device__ __forceinline__ void lse_fold(Lse &acc, const Lse &other) {
+    if (other.s > 0.0) { if (acc.s > 0.0) lse_merge(acc, other); else acc = other; }
 }
 
 // f update: one warp per row, lanes stride the columns (coalesced), kSkGroup * 32 columns per step.
@@ -155,33 +166,94 @@ sk_col_partial_kernel(const double *__restrict__ M, long long ld, long long S, l
     ps[chunk * D + j] = acc.s;
 }
 
+// g update, stage 2, first job: the chunk partials of column j merged in chunk order (empty partials, s = 0, skipped).
+__device__ __forceinline__ Lse sk_merge_chunks(long long D, long long n_chunks, const double *__restrict__ pm,
+                                               const double *__restrict__ ps, long long j) {
+    Lse acc{-INFINITY, 0.0};
+    for (long long c = 0; c < n_chunks; ++c) lse_fold(acc, Lse{pm[c * D + j], ps[c * D + j]});
+    return acc;
+}
+
+// g update, stage 2, second job: g_j = reg (log b_j - LSE_j); returns the term (b_j (exp((g_old - g_new)/reg) - 1))^2
+// of POT's error.
+__device__ __forceinline__ double sk_col_finish(const Lse &acc, double log_b, double b, double reg, double &g) {
+    const double g_new = reg * (log_b - (acc.m + log(acc.s)));
+    const double e = b * (exp((g - g_new) / reg) - 1.0);
+    g = g_new;
+    return e * e;
+}
+
+// Sum of the error terms of a 256-thread CTA, in a fixed order; valid in thread 0.  Every thread of the CTA calls it.
+__device__ __forceinline__ double sk_err_block_sum(double e2) {
+    __shared__ double s_err[8];
+    e2 = warp_sum(e2);
+    if (lane_id() == 0) s_err[threadIdx.x >> 5] = e2;
+    __syncthreads();
+    double t = 0.0;
+    if (threadIdx.x == 0)
+        for (int w = 0; w < 8; ++w) t += s_err[w];
+    return t;
+}
+
 // g update, stage 2: merge the chunks of a column; accumulate POT's error sum_j (b_j (exp((g_old - g_new)/reg) - 1))^2.
 __global__ void __launch_bounds__(256)
 sk_col_merge_kernel(long long D, long long n_chunks, const double *__restrict__ pm, const double *__restrict__ ps,
                     const double *__restrict__ log_b, const double *__restrict__ b, double reg,
                     double *__restrict__ g, double *err2) {
-    __shared__ double s_err[8];
     const long long j = (long long)blockIdx.x * 256 + threadIdx.x;
     double e2 = 0.0;
-    if (j < D) {
+    if (j < D) e2 = sk_col_finish(sk_merge_chunks(D, n_chunks, pm, ps, j), log_b[j], b[j], reg, g[j]);
+    const double t = sk_err_block_sum(e2);
+    if (threadIdx.x == 0 && err2 != nullptr && t != 0.0) atomicAdd(err2, t);
+}
+
+// ---- row-sharded form (sx_sinkhorn_ot_sharded_h) ------------------------------------------------------------
+// Rank r holds rows [row0_r, row0_r + S_loc_r) of M and runs the kernels above on them; f is local to the rank,
+// g is computed by every rank.  The column half-step needs one (m, s) pair per column from every rank: the push
+// kernel merges the rank's chunk partials and stores the pair into every rank's exchange buffer as two LL slots
+// (sx_ll.cuh; block_len = 2 D slots per rank, flag = iteration + 1, half = flag & 1); the fold kernel polls the
+// G pairs of its column in the local buffer and merges them in rank order, so every rank computes the same g.
+// Double buffering suffices: a rank pushes iteration e + 1 only after its own fold of e, which needed every
+// peer's push of e, which that peer enqueued after its fold of e - 1 -- the last reader of the same half.
+__global__ void __launch_bounds__(256)
+sk_col_push_kernel(long long D, long long n_chunks, const double *__restrict__ pm, const double *__restrict__ ps,
+                   char *const *peer_bufs, int rank, int G, unsigned flag) {
+    const long long j = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (j >= D) return;
+    const Lse acc = sk_merge_chunks(D, n_chunks, pm, ps, j);
+    for (int p = 0; p < G; ++p) {
+        uint4 *dst = ll_slot(peer_bufs[p], G, 2 * D, flag, rank, 2 * j);
+        ll_store_slot(dst, flag, (unsigned long long)__double_as_longlong(acc.m));
+        ll_store_slot(dst + 1, flag, (unsigned long long)__double_as_longlong(acc.s));
+    }
+}
+
+// err_part (may be null): CTA c writes the sum of its columns' error terms to err_part[c], and the host adds them
+// in CTA order -- unlike an atomic sum, the error (and so the iteration a run stops at) does not depend on the
+// order in which CTAs finish, which differs between ranks sharing a GPU and ranks waiting on NVLink peers.
+// status: SX_ERR_PEER_TIMEOUT when some pair did not arrive within timeout_ns; once it is set, later folds return
+// at once (g is then stale and the host reports the error).
+__global__ void __launch_bounds__(256)
+sk_col_fold_kernel(long long D, char *ll_local, int G, unsigned flag, const double *__restrict__ log_b,
+                   const double *__restrict__ b, double reg, double *__restrict__ g, double *err_part, int *status,
+                   unsigned long long timeout_ns) {
+    const long long j = (long long)blockIdx.x * 256 + threadIdx.x;
+    double e2 = 0.0;
+    if (j < D && *reinterpret_cast<volatile int *>(status) == 0) {
+        const unsigned long long t0 = global_timer_ns();
         Lse acc{-INFINITY, 0.0};
-        for (long long c = 0; c < n_chunks; ++c) {
-            const Lse other{pm[c * D + j], ps[c * D + j]};
-            if (other.s > 0.0) { if (acc.s > 0.0) lse_merge(acc, other); else acc = other; }
+        bool ok = true;
+        for (int r = 0; r < G && ok; ++r) {
+            const uint4 *src = ll_slot(ll_local, G, 2 * D, flag, r, 2 * j);
+            unsigned long long m = 0, s = 0;
+            ok = ll_poll(src, flag, m, t0, timeout_ns) && ll_poll(src + 1, flag, s, t0, timeout_ns);
+            if (ok) lse_fold(acc, Lse{__longlong_as_double((long long)m), __longlong_as_double((long long)s)});
         }
-        const double g_new = reg * (log_b[j] - (acc.m + log(acc.s)));
-        const double e = b[j] * (exp((g[j] - g_new) / reg) - 1.0);
-        e2 = e * e;
-        g[j] = g_new;
+        if (ok) e2 = sk_col_finish(acc, log_b[j], b[j], reg, g[j]);
+        else atomicExch(status, SX_ERR_PEER_TIMEOUT);
     }
-    e2 = warp_sum(e2);
-    if (lane_id() == 0) s_err[threadIdx.x >> 5] = e2;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double t = 0.0;
-        for (int w = 0; w < 8; ++w) t += s_err[w];
-        if (err2 != nullptr && t != 0.0) atomicAdd(err2, t);
-    }
+    const double t = sk_err_block_sum(e2);
+    if (threadIdx.x == 0 && err_part != nullptr) err_part[blockIdx.x] = t;
 }
 
 __global__ void sk_log_kernel(const double *__restrict__ a, long long n, double *__restrict__ out) {
@@ -267,6 +339,185 @@ extern "C" int sx_sinkhorn_ot(const double *M, int64_t ld, int64_t S, int64_t D,
         sk_plan_kernel<<<num_sms() * 8, 256, 0, st>>>(M, ld, S, D, f, g, reg, x_out);
         SX_LAUNCH_CHECK();
     }
+    if (iters_h) *iters_h = it;
+    if (err_h) *err_h = err;
+    return SX_OK;
+}
+
+namespace {
+
+// Buffers of one rank of sx_sinkhorn_ot_sharded_h, carved from one allocation on the rank's device.
+struct SkRank {
+    int dev = 0;
+    cudaStream_t st = nullptr;                 // the stream of this rank's device (ranks of one device share it)
+    const double *M = nullptr;
+    int64_t row0 = 0, S_loc = 0, n_chunks = 0;
+    void *mem = nullptr;
+    double *a = nullptr, *log_a = nullptr, *b = nullptr, *log_b = nullptr, *f = nullptr, *g = nullptr;
+    double *pm = nullptr, *ps = nullptr;
+    double *ctl = nullptr;                     // {status (int32), error part of each fold CTA}: one copy reads both
+    char *ll_buf = nullptr;
+    char **peer_bufs = nullptr;
+    int *status() const { return reinterpret_cast<int *>(ctl); }
+    double *err_part() const { return ctl + 1; }
+};
+
+struct SkSharded {
+    std::vector<SkRank> r;
+    std::vector<std::pair<int, cudaStream_t>> streams;   // one per distinct device
+    int prev = 0;
+    ~SkSharded() {
+        for (auto &ds : streams) {
+            cudaSetDevice(ds.first);
+            cudaStreamSynchronize(ds.second);
+            cudaStreamDestroy(ds.second);
+        }
+        for (SkRank &k : r) {
+            if (!k.mem) continue;
+            cudaSetDevice(k.dev);
+            cudaFree(k.mem);
+        }
+        cudaSetDevice(prev);
+    }
+};
+
+size_t sk_rank_bytes(int64_t S_loc, int64_t D, int64_t n_chunks, int G, unsigned col_blocks) {
+    return 3 * carve_bytes((size_t)S_loc, 8) + 3 * carve_bytes((size_t)D, 8) +
+           2 * carve_bytes((size_t)n_chunks * D, 8) + carve_bytes(1 + (size_t)col_blocks, 8) +
+           carve_bytes((size_t)4 * G * D, 16) + carve_bytes((size_t)G, sizeof(void *));
+}
+
+}  // namespace
+
+extern "C" int sx_sinkhorn_ot_sharded_h(int ndev, const int *devs, const double *const *slabs,
+                                        const int64_t *row_bounds, int64_t ld, int64_t S, int64_t D,
+                                        const double *a_h, const double *b_h, double reg, int64_t max_iter,
+                                        double stop_thr, int64_t check_every, double *f_h, double *g_h,
+                                        double *const *x_out, int64_t *iters_h, double *err_h) {
+    if (ndev < 1 || ndev > 64 || !devs || !slabs || !a_h || !b_h || !f_h || !g_h || S < 1 || D < 1 || ld < D ||
+        !(reg > 0.0) || max_iter < 0)
+        return SX_ERR_INVALID;
+    if (ndev > S) return SX_ERR_INVALID;                      // every rank needs at least one row
+    if (row_bounds) {
+        if (row_bounds[0] != 0 || row_bounds[ndev] != S) return SX_ERR_INVALID;
+        for (int g = 0; g < ndev; ++g) if (row_bounds[g + 1] <= row_bounds[g]) return SX_ERR_INVALID;
+    }
+    for (int g = 0; g < ndev; ++g) if (!slabs[g] || (x_out && !x_out[g])) return SX_ERR_INVALID;
+    if (check_every <= 0) check_every = 10;
+    const int G = ndev;
+    const unsigned col_blocks = (unsigned)((D + 255) / 256);
+    SkSharded sh;
+    SX_CUDA(cudaGetDevice(&sh.prev));
+    sh.r.resize(G);
+    for (int g = 0; g < G; ++g) {
+        SkRank &k = sh.r[g];
+        k.dev = devs[g];
+        k.M = slabs[g];
+        k.row0 = row_bounds ? row_bounds[g] : S * g / G;
+        k.S_loc = (row_bounds ? row_bounds[g + 1] : S * (g + 1) / G) - k.row0;
+        k.n_chunks = (k.S_loc + kSkRowsPerChunk - 1) / kSkRowsPerChunk;
+        if (cudaSetDevice(k.dev) != cudaSuccess) return SX_ERR_NO_DEVICE;
+        for (auto &ds : sh.streams) if (ds.first == k.dev) k.st = ds.second;
+        if (!k.st) {                                          // first rank on this device
+            int rc = enable_peer_access(k.dev, G, devs);
+            if (rc != SX_OK) return rc;
+            SX_CUDA(cudaStreamCreateWithFlags(&k.st, cudaStreamNonBlocking));
+            sh.streams.emplace_back(k.dev, k.st);
+        }
+        const size_t bytes = sk_rank_bytes(k.S_loc, D, k.n_chunks, G, col_blocks);
+        SX_CUDA(cudaMalloc(&k.mem, bytes));
+        Carver cv(k.mem);
+        k.a = cv.take<double>(k.S_loc); k.log_a = cv.take<double>(k.S_loc); k.f = cv.take<double>(k.S_loc);
+        k.b = cv.take<double>(D); k.log_b = cv.take<double>(D); k.g = cv.take<double>(D);
+        k.pm = cv.take<double>((size_t)k.n_chunks * D); k.ps = cv.take<double>((size_t)k.n_chunks * D);
+        k.ctl = cv.take<double>(1 + (size_t)col_blocks);
+        k.ll_buf = cv.take<char>((size_t)4 * G * D * 16);
+        k.peer_bufs = cv.take<char *>(G);
+        SX_CUDA(cudaMemsetAsync(k.ctl, 0, sizeof(double), k.st));
+        SX_CUDA(cudaMemsetAsync(k.ll_buf, 0, (size_t)4 * G * D * 16, k.st));
+        SX_CUDA(cudaMemcpyAsync(k.a, a_h + k.row0, (size_t)k.S_loc * 8, cudaMemcpyHostToDevice, k.st));
+        SX_CUDA(cudaMemcpyAsync(k.b, b_h, (size_t)D * 8, cudaMemcpyHostToDevice, k.st));
+        sk_log_kernel<<<num_sms(), 256, 0, k.st>>>(k.a, k.S_loc, k.log_a);
+        sk_log_kernel<<<num_sms(), 256, 0, k.st>>>(k.b, D, k.log_b);
+        SX_LAUNCH_CHECK();
+        SX_CUDA(cudaMemsetAsync(k.g, 0, sizeof(double) * (size_t)D, k.st));
+        sk_fill_kernel<<<num_sms(), 256, 0, k.st>>>(k.f, k.S_loc, -reg * log((double)S));     // u = 1 / S (global S)
+        SX_LAUNCH_CHECK();
+    }
+    std::vector<char *> bufs(G);                              // every rank learns every exchange buffer
+    for (int g = 0; g < G; ++g) bufs[g] = sh.r[g].ll_buf;
+    for (SkRank &k : sh.r) {
+        SX_CUDA(cudaSetDevice(k.dev));
+        SX_CUDA(cudaMemcpyAsync(k.peer_bufs, bufs.data(), sizeof(void *) * G, cudaMemcpyHostToDevice, k.st));
+    }
+    for (auto &ds : sh.streams) {                             // buffers zeroed everywhere before any push
+        SX_CUDA(cudaSetDevice(ds.first));
+        SX_CUDA(cudaStreamSynchronize(ds.second));
+    }
+    const unsigned long long timeout_ns = 10ull * 1000 * 1000 * 1000;
+    std::vector<double> ctl_h(1 + (size_t)col_blocks);
+    SkRank &k0 = sh.r[0];
+    int64_t it = 0;
+    double err = INFINITY;
+    // Enqueue order per iteration: partial + push of every rank, fold of every rank, row pass of every rank.  Ranks
+    // that share a device share its stream, so there every push precedes every fold and no kernel waits on a later
+    // one; ranks on distinct devices poll each other's pushes over NVLink.
+    for (; it < max_iter; ++it) {
+        const bool check = stop_thr > 0.0 && it > 0 && ((it - 1) % check_every == 0);
+        const unsigned flag = (unsigned)(it + 1);
+        for (int g = 0; g < G; ++g) {
+            SkRank &k = sh.r[g];
+            SX_CUDA(cudaSetDevice(k.dev));
+            sk_col_partial_kernel<<<dim3(col_blocks, (unsigned)k.n_chunks), 256, 0, k.st>>>(
+                k.M, ld, k.S_loc, D, k.f, reg, kSkRowsPerChunk, k.pm, k.ps);
+            sk_col_push_kernel<<<col_blocks, 256, 0, k.st>>>(D, k.n_chunks, k.pm, k.ps, k.peer_bufs, g, G, flag);
+            SX_LAUNCH_CHECK();
+        }
+        for (int g = 0; g < G; ++g) {
+            SkRank &k = sh.r[g];
+            SX_CUDA(cudaSetDevice(k.dev));
+            sk_col_fold_kernel<<<col_blocks, 256, 0, k.st>>>(D, k.ll_buf, G, flag, k.log_b, k.b, reg, k.g,
+                                                             (check && g == 0) ? k.err_part() : nullptr, k.status(),
+                                                             timeout_ns);
+            SX_LAUNCH_CHECK();
+        }
+        if (check) {                                          // rank 0's error decides for every rank
+            SX_CUDA(cudaSetDevice(k0.dev));
+            SX_CUDA(cudaMemcpyAsync(ctl_h.data(), k0.ctl, ctl_h.size() * 8, cudaMemcpyDeviceToHost, k0.st));
+            SX_CUDA(cudaStreamSynchronize(k0.st));
+            int status = 0;
+            memcpy(&status, ctl_h.data(), sizeof(int));
+            if (status != 0) return status;
+            double e2 = 0.0;
+            for (unsigned c = 0; c < col_blocks; ++c) e2 += ctl_h[1 + c];        // CTA order: deterministic
+            err = sqrt(e2);
+            if (err < stop_thr) break;
+        }
+        for (int g = 0; g < G; ++g) {
+            SkRank &k = sh.r[g];
+            SX_CUDA(cudaSetDevice(k.dev));
+            long long row_grid = (k.S_loc * 32 + 255) / 256;
+            if (row_grid > num_sms() * 16) row_grid = num_sms() * 16;
+            sk_row_kernel<<<(int)row_grid, 256, 0, k.st>>>(k.M, ld, k.S_loc, D, k.g, k.log_a, reg, k.f);
+            SX_LAUNCH_CHECK();
+        }
+    }
+    int status = SX_OK;
+    for (int g = 0; g < G; ++g) {
+        SkRank &k = sh.r[g];
+        SX_CUDA(cudaSetDevice(k.dev));
+        if (x_out) {
+            sk_plan_kernel<<<num_sms() * 8, 256, 0, k.st>>>(k.M, ld, k.S_loc, D, k.f, k.g, reg, x_out[g]);
+            SX_LAUNCH_CHECK();
+        }
+        SX_CUDA(cudaMemcpyAsync(f_h + k.row0, k.f, (size_t)k.S_loc * 8, cudaMemcpyDeviceToHost, k.st));
+        if (g == 0) SX_CUDA(cudaMemcpyAsync(g_h, k.g, (size_t)D * 8, cudaMemcpyDeviceToHost, k.st));
+        int s = 0;
+        SX_CUDA(cudaMemcpyAsync(&s, k.status(), sizeof(int), cudaMemcpyDeviceToHost, k.st));
+        SX_CUDA(cudaStreamSynchronize(k.st));
+        if (status == SX_OK) status = s;
+    }
+    if (status != SX_OK) return status;
     if (iters_h) *iters_h = it;
     if (err_h) *err_h = err;
     return SX_OK;

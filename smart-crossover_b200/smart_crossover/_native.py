@@ -107,6 +107,8 @@ SIGNATURES = {
     "sx_topk_merge_ll": (_int, [_p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _p]),
     "sx_sinkhorn_workspace_bytes": (_sz, [_i64, _i64]),
     "sx_sinkhorn_ot": (_int, [_p, _i64, _i64, _i64, _p, _p, _dbl, _i64, _dbl, _i64, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "sx_sinkhorn_ot_sharded_h": (_int, [_int, _p, _p, _p, _i64, _i64, _i64, _p, _p, _dbl, _i64, _dbl, _i64, _p, _p,
+                                        _p, _p, _p]),
     "sx_price_dense_ot_h": (_int, [_p, _p, _i64, _i64, _p, _dbl, _i64, _p, _p, _p, _p, _p]),
     "sx_ot_pricer_create": (_int, [_int, _p, _p, _p, _i64, _i64, _i64, _i64, _dbl, _p]),
     "sx_ot_pricer_destroy": (_int, [_p]),

@@ -5,6 +5,8 @@ numItermax=1000)` (`scripts/run_network_crossover.py:96`), and hands the flatten
 `network_crossover`.  POT is not part of the reference tree; `sinkhorn` below keeps its call shape
 (marginals, cost matrix, `reg`, `numItermax`, `stopThr`; returns the S x D plan) and runs the same
 Sinkhorn-Knopp iteration in the log domain on the device (`sx_sinkhorn_ot`, csrc/sx_sinkhorn.cu).
+A cost matrix held as `device.CostSlabs` (row shards on several GPUs, e.g. the slabs of
+`OTManager.from_device_cost`) runs the same iteration on every shard's GPU (`sx_sinkhorn_ot_sharded_h`).
 """
 from __future__ import annotations
 
@@ -21,6 +23,8 @@ def sinkhorn(a, b, M, reg: float, numItermax: int = 1000, stopThr: float = 1e-9,
     from smart_crossover._native import check, lib
 
     dev._require_cuda()
+    if isinstance(M, dev.CostSlabs):
+        return _sinkhorn_slabs(a, b, M, reg, numItermax, stopThr, log)
     a_t, b_t = dev._f64(np.asarray(a, dtype=np.float64)), dev._f64(np.asarray(b, dtype=np.float64))
     M_t = dev._f64(M) if not (isinstance(M, torch.Tensor) and M.is_cuda) else M.contiguous()
     S, D = M_t.shape
@@ -38,4 +42,35 @@ def sinkhorn(a, b, M, reg: float, numItermax: int = 1000, stopThr: float = 1e-9,
     plan = X.cpu().numpy()
     if log:
         return plan, {"niter": iters.value, "err": err.value, "f": f.cpu().numpy(), "g": g.cpu().numpy()}
+    return plan
+
+
+def _sinkhorn_slabs(a, b, slabs, reg, numItermax, stopThr, log):
+    """`sinkhorn` over the row shards of a `device.CostSlabs`: shard g's rows on its device, the plan assembled on
+    the host shard by shard.  The cost matrix is never read on the host."""
+    import torch
+    from smart_crossover import device as dev
+    from smart_crossover._native import check, lib
+
+    S, D, G = slabs.S, slabs.D, len(slabs.devices)
+    a = np.ascontiguousarray(a, dtype=np.float64).ravel()
+    b = np.ascontiguousarray(b, dtype=np.float64).ravel()
+    if a.size != S or b.size != D:
+        raise ValueError("marginals do not match the cost matrix")
+    X = [torch.empty(slabs.rows[g], D, dtype=torch.float64, device=slabs.t[g].device) for g in range(G)]
+    f, g_pot = np.empty(S), np.empty(D)
+    slabs.sync()
+    iters, err = ctypes.c_int64(0), ctypes.c_double(0.0)
+    check(lib.sx_sinkhorn_ot_sharded_h(G, (ctypes.c_int * G)(*slabs.devices),
+                                       (ctypes.c_void_p * G)(*[t.data_ptr() for t in slabs.t]),
+                                       (ctypes.c_int64 * (G + 1))(*slabs.row_bounds), slabs.ld, S, D,
+                                       a.ctypes.data, b.ctypes.data, float(reg), int(numItermax), float(stopThr), 10,
+                                       f.ctypes.data, g_pot.ctypes.data,
+                                       (ctypes.c_void_p * G)(*[x.data_ptr() for x in X]),
+                                       ctypes.byref(iters), ctypes.byref(err)), "sx_sinkhorn_ot_sharded_h")
+    plan = np.empty((S, D))
+    for g in range(G):
+        plan[slabs.row0[g]:slabs.row0[g] + slabs.rows[g]] = dev.to_host(X[g])
+    if log:
+        return plan, {"niter": iters.value, "err": err.value, "f": f, "g": g_pot}
     return plan
