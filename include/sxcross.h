@@ -95,7 +95,7 @@ SX_API double      sx_key_to_f64(long long key);        /* decode sx_price_heade
  *   x (S*D), s (S), d (D) -> score_out (S*D).  Correctly rounded IEEE divisions; NumPy
  *   `maximum` semantics (NaN propagates).  hist12_out (may be NULL; 4096 uint32, zeroed by the
  *   caller): histogram of the scores' top 12 key bits, accumulated while the scores are written,
- *   which sx_kruskal_prefix accepts instead of taking it with a pass of its own.
+ *   which sx_kruskal_prefix and sx_order_head_sharded_h accept instead of taking it with a pass of their own.
  * sx_score_mcf replaces net_manager.py:165-182: reversal of arcs with x > u/2, per-node
  *   out/in sums in ascending arc id (SciPy csr_matvec order), f_inv = 1/max(f1,f2),
  *   indicator = max over the two end nodes of |f_inv * x_hat|.  node_ptr (N+1) /
@@ -162,6 +162,28 @@ SX_API int    sx_hist12_f64(const double *weight, int64_t n, uint32_t *hist12, v
 SX_API int    sx_kruskal_prefix(const double *weight, int64_t n, int64_t T, int64_t T_cap,
                          const uint32_t *hist12, uint32_t *korder_out, int64_t *n_prefix_h,
                          void *ws, size_t ws_bytes, void *stream);
+
+/* sx_order_head_sharded_h: the same head over S x D weights held as row slabs on several devices (the flow
+ * scores of a row-sharded OT problem, with the row bounds of its cost slabs); one process, one host thread.
+ * Every shard streams only its own weights on its own GPU; the host adds the shards' 4096-bin histograms of
+ * both levels (two small round trips per shard), so every shard selects against the same threshold, and only
+ * the candidates (at most T_cap arcs) are copied to devs[0], where they are sorted and ordered.
+ *   devs / row_bounds: as sx_sinkhorn_ot_sharded_h (row_bounds NULL = equal partition; a device may appear more
+ *     than once: its shards then run one after the other on one stream of that device, with the same results).
+ *   weights[g]: DEVICE pointer on devs[g] to shard g's rows x D weights, contiguous.  Arc ids are global:
+ *     row_bounds[g] * D + position in the shard; S * D >= 2^32 is SX_ERR_TOO_LARGE.
+ *   hist12 (may be NULL, as may any entry): hist12[g] is shard g's level-0 histogram (sx_score_ot).
+ *   mode SX_ORDER_KRUSKAL: out = uint32 ids, descending weight, ties by ascending id (sx_kruskal's input);
+ *   mode SX_ORDER_QUEUE:   out = int64 ids, descending weight, ties by descending id, i.e. the head of
+ *     np.argsort(w, kind="stable")[::-1] (net_manager.py:379).
+ *   out: DEVICE buffer on devs[0], capacity T_cap >= T.  *n_out_h (HOST): arcs written (>= min(T, S * D)), or -1
+ *     when more than T_cap arcs tie at the threshold, as sx_kruskal_prefix.
+ * Blocking; allocates and frees its buffers per call (per shard 80 B x T_cap, on devs[0] ~48 B x T_cap more). */
+#define SX_ORDER_KRUSKAL 0
+#define SX_ORDER_QUEUE   1
+SX_API int    sx_order_head_sharded_h(int ndev, const int *devs, const double *const *weights,
+                               const int64_t *row_bounds, int64_t S, int64_t D, int64_t T, int64_t T_cap,
+                               const uint32_t *const *hist12, int mode, void *out, int64_t *n_out_h);
 
 /* ---- K2: spanning-tree basis identification -------------------------------------------
  * Replaces `sp.csgraph.minimum_spanning_tree(-w)` + flatnonzero, tree_BI.py:32-59.

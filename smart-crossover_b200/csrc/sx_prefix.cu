@@ -16,6 +16,9 @@
 //   3. the few candidates are sorted by id, then stably by weight (radix argsort, sx_sort.cu), and
 //      the tie runs are flipped into the Kruskal order (sx_kruskal_order).
 // HBM-bound: 8-16 B per arc (24 B in the crowded-bin case) instead of the ~256 B per arc of the full 8-pass argsort.
+#include <utility>
+#include <vector>
+
 #include "sx_common.cuh"
 
 namespace sx {
@@ -129,8 +132,9 @@ constexpr int kPfBatch = 4;
 constexpr int kPfStage = 2048;                 // staged candidates per CTA (32 KB)
 
 __global__ void __launch_bounds__(kPfThreads)
-pf_filter_kernel(const double *__restrict__ w, const unsigned long long *__restrict__ ids_in, long long n,
-                 PrefixCtl *ctl, double *__restrict__ cand_w, unsigned long long *__restrict__ cand_id, long long cap) {
+pf_filter_kernel(const double *__restrict__ w, const unsigned long long *__restrict__ ids_in, unsigned long long id_base,
+                 long long n, PrefixCtl *ctl, double *__restrict__ cand_w, unsigned long long *__restrict__ cand_id,
+                 long long cap) {
     __shared__ double             s_w[kPfStage];
     __shared__ unsigned long long s_id[kPfStage];
     __shared__ unsigned           s_cnt;
@@ -150,7 +154,7 @@ pf_filter_kernel(const double *__restrict__ w, const unsigned long long *__restr
         base = __shfl_sync(0xffffffffu, base, 0);
         const unsigned slot = base + __popc(m & lt);
         if (!keep) return;
-        const unsigned long long gid = ids_in ? ids_in[id] : (unsigned long long)id;     // position -> arc id
+        const unsigned long long gid = ids_in ? ids_in[id] : id_base + (unsigned long long)id;   // position -> arc id
         if (slot < (unsigned)kPfStage) { s_w[slot] = v; s_id[slot] = gid; }
         else {                                                   // stage full (dense selection): straight to global
             const unsigned long long g = atomicAdd(&ctl->n_sel, 1ull);
@@ -224,9 +228,9 @@ __device__ __forceinline__ unsigned pf_image32(double v) {
 constexpr int kPfHalf = kPfStage / 2;
 
 __global__ void __launch_bounds__(kPfThreads)
-pf_split_kernel(const double *__restrict__ w, long long n, PrefixCtl *ctl, double *__restrict__ cand_w,
-                unsigned long long *__restrict__ cand_id, long long cap, double *__restrict__ bnd_w,
-                unsigned long long *__restrict__ bnd_id, long long bnd_cap) {
+pf_split_kernel(const double *__restrict__ w, unsigned long long id_base, long long n, PrefixCtl *ctl,
+                double *__restrict__ cand_w, unsigned long long *__restrict__ cand_id, long long cap,
+                double *__restrict__ bnd_w, unsigned long long *__restrict__ bnd_id, long long bnd_cap) {
     __shared__ double             s_w[2][kPfHalf];
     __shared__ unsigned long long s_id[2][kPfHalf];
     __shared__ unsigned           s_cnt[2];
@@ -247,11 +251,12 @@ pf_split_kernel(const double *__restrict__ w, long long n, PrefixCtl *ctl, doubl
         base = __shfl_sync(0xffffffffu, base, 0);
         const unsigned slot = base + __popc(m & lt);
         if (!keep) return;
-        if (slot < (unsigned)kPfHalf) { s_w[which][slot] = v; s_id[which][slot] = (unsigned long long)id; }
+        const unsigned long long gid = id_base + (unsigned long long)id;
+        if (slot < (unsigned)kPfHalf) { s_w[which][slot] = v; s_id[which][slot] = gid; }
         else {                                                   // stage full: straight to global
             const unsigned long long g = atomicAdd(which ? &ctl->n_bnd : &ctl->n_sel, 1ull);
-            if (which == 0) { if ((long long)g < cap) { cand_w[g] = v; cand_id[g] = (unsigned long long)id; } }
-            else { if ((long long)g < bnd_cap) { bnd_w[g] = v; bnd_id[g] = (unsigned long long)id; } }
+            if (which == 0) { if ((long long)g < cap) { cand_w[g] = v; cand_id[g] = gid; } }
+            else { if ((long long)g < bnd_cap) { bnd_w[g] = v; bnd_id[g] = gid; } }
         }
     };
     auto flush = [&]() {                                         // whole CTA, both stages
@@ -280,11 +285,12 @@ pf_split_kernel(const double *__restrict__ w, long long n, PrefixCtl *ctl, doubl
     const bool     none_above = b1 >= (unsigned)kPfBins - 1;
     const unsigned sel_lo = none_above ? 0xffffffffu : (b1 + 1) << 20;             // image32 >= sel_lo: bin > b1
     auto put = [&](int which, unsigned slot, double v, long long id) {
-        if (slot < (unsigned)kPfHalf) { s_w[which][slot] = v; s_id[which][slot] = (unsigned long long)id; }
+        const unsigned long long gid = id_base + (unsigned long long)id;
+        if (slot < (unsigned)kPfHalf) { s_w[which][slot] = v; s_id[which][slot] = gid; }
         else {                                                   // stage full: straight to global
             const unsigned long long g = atomicAdd(which ? &ctl->n_bnd : &ctl->n_sel, 1ull);
-            if (which == 0) { if ((long long)g < cap) { cand_w[g] = v; cand_id[g] = (unsigned long long)id; } }
-            else { if ((long long)g < bnd_cap) { bnd_w[g] = v; bnd_id[g] = (unsigned long long)id; } }
+            if (which == 0) { if ((long long)g < cap) { cand_w[g] = v; cand_id[g] = gid; } }
+            else { if ((long long)g < bnd_cap) { bnd_w[g] = v; bnd_id[g] = gid; } }
         }
     };
     const long long n2_blocks = (n2 + kPfThreads - 1) / kPfThreads;
@@ -390,6 +396,54 @@ static int pf_grid(long long n, int per_thread) {
     return (int)g;
 }
 
+// Grids of the split and filter passes over cnt weights on the current device: one wave of resident CTAs at most.
+static int pf_pass_grid(const void *kernel, long long cnt) {
+    int occ = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, kPfThreads, 0) != cudaSuccess || occ < 1) occ = 1;
+    const long long ctas = (long long)num_sms() * occ;
+    long long need = (cnt / 2 + (long long)kPfThreads * kPfBatch - 1) / ((long long)kPfThreads * kPfBatch);
+    if (need < 1) need = 1;
+    return (int)(need < ctas ? need : ctas);
+}
+
+// The sort-and-order tail shared by sx_kruskal_prefix and sx_order_head_sharded_h: the m <= cap candidates
+// (weight, arc id) are sorted by id, then stably by weight (ascending weight, ties by ascending id), and the
+// ascending order is turned into the Kruskal order (uint32 ids, descending weight, ties by ascending id) or
+// reversed into the queue order (int64 ids, descending weight, ties by descending id).
+static size_t pf_tail_bytes(int64_t cap) {
+    const size_t c = (size_t)cap;
+    return 2 * carve_bytes(c, 8) + 4 * carve_bytes(c, 4) + align_up(sx_argsort_workspace_bytes(cap), 256) +
+           sx_kruskal_order_workspace_bytes(cap);
+}
+
+static int pf_order_tail(const double *cand_w, const unsigned long long *cand_id, long long m, int64_t cap, int mode,
+                         void *out, void *ws, cudaStream_t st) {
+    if (m == 0) return SX_OK;
+    Carver cv(ws);
+    double *w1 = cv.take<double>(cap);
+    double *sorted_w = cv.take<double>(cap);
+    uint32_t *id1 = cv.take<uint32_t>(cap);
+    uint32_t *perm = cv.take<uint32_t>(cap);
+    uint32_t *perm2 = cv.take<uint32_t>(cap);
+    uint32_t *order_asc = cv.take<uint32_t>(cap);
+    void *sort_ws = cv.base + cv.off;
+    const size_t sort_ws_bytes = sx_argsort_workspace_bytes(cap);
+    void *ko_ws = (char *)sort_ws + align_up(sort_ws_bytes, 256);
+    const size_t ko_ws_bytes = sx_kruskal_order_workspace_bytes(cap);
+    // (weight, id) is a strict total order: sort by id, then stably by weight
+    int rc = sx_argsort_u64(cand_id, m, 32, perm, nullptr, sort_ws, sort_ws_bytes, st);
+    if (rc != SX_OK) return rc;
+    const int g2 = pf_grid(m, 1);
+    pf_gather_kernel<<<g2, kPfThreads, 0, st>>>(cand_w, cand_id, perm, m, w1, id1);
+    SX_LAUNCH_CHECK();
+    rc = sx_argsort_f64(w1, m, perm2, sorted_w, sort_ws, sort_ws_bytes, st);
+    if (rc != SX_OK) return rc;
+    pf_gather_ids_kernel<<<g2, kPfThreads, 0, st>>>(id1, perm2, m, order_asc);
+    SX_LAUNCH_CHECK();
+    if (mode == SX_ORDER_QUEUE) return sx_queue_from_order(order_asc, m, (int64_t *)out, st);
+    return sx_kruskal_order(sorted_w, order_asc, m, (uint32_t *)out, ko_ws, ko_ws_bytes, st);
+}
+
 }  // namespace sx
 
 using namespace sx;
@@ -397,9 +451,8 @@ using namespace sx;
 extern "C" size_t sx_kruskal_prefix_workspace_bytes(int64_t T_cap) {
     if (T_cap < 0) return 0;
     const size_t c = (size_t)T_cap;
-    return carve_bytes(1, sizeof(PrefixCtl)) + 3 * carve_bytes(c, 8) + 4 * carve_bytes(c, 4) + carve_bytes(c, 8) +
-           2 * carve_bytes(kPfBndFactor * c, 8) + sx_argsort_workspace_bytes(T_cap) +
-           sx_kruskal_order_workspace_bytes(T_cap) + 256;
+    return carve_bytes(1, sizeof(PrefixCtl)) + carve_bytes(c, 8) + carve_bytes(c, 8) +
+           2 * carve_bytes(kPfBndFactor * c, 8) + pf_tail_bytes(T_cap) + 256;
 }
 
 // hist[bin] += number of weights whose order-preserving image has top 12 bits == bin (4096 bins).
@@ -421,18 +474,9 @@ extern "C" int sx_kruskal_prefix(const double *weight, int64_t n, int64_t T, int
     PrefixCtl *ctl = cv.take<PrefixCtl>(1);
     double *cand_w = cv.take<double>(T_cap);
     unsigned long long *cand_id = cv.take<unsigned long long>(T_cap);
-    double *w1 = cv.take<double>(T_cap);
-    uint32_t *id1 = cv.take<uint32_t>(T_cap);
-    uint32_t *perm = cv.take<uint32_t>(T_cap);
-    uint32_t *perm2 = cv.take<uint32_t>(T_cap);
-    uint32_t *order_asc = cv.take<uint32_t>(T_cap);
-    double *sorted_w = cv.take<double>(T_cap);
     double *bnd_w = cv.take<double>(kPfBndFactor * (size_t)T_cap);
     unsigned long long *bnd_id = cv.take<unsigned long long>(kPfBndFactor * (size_t)T_cap);
-    void *sort_ws = cv.base + cv.off;
-    const size_t sort_ws_bytes = sx_argsort_workspace_bytes(T_cap);
-    void *ko_ws = (char *)sort_ws + align_up(sort_ws_bytes, 256);
-    const size_t ko_ws_bytes = sx_kruskal_order_workspace_bytes(T_cap);
+    void *tail_ws = cv.base + cv.off;
 
     SX_CUDA(cudaMemsetAsync(ctl, 0, sizeof(PrefixCtl), st));
     const int grid = pf_grid(n, 16);
@@ -447,24 +491,14 @@ extern "C" int sx_kruskal_prefix(const double *weight, int64_t n, int64_t T, int
     // level 1.  Preferred: ONE more pass over the weights that selects everything above bin b1 and sets
     // the arcs of bin b1 aside; the second histogram and the filter then run on that short list.  If the
     // threshold bin is too crowded for the list, both run over all the weights instead.
-    int occ = 1;
-    SX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pf_split_kernel, kPfThreads, 0));
-    long long fgrid = (long long)num_sms() * (occ > 0 ? occ : 1);
-    const long long fneed = (n / 2 + (long long)kPfThreads * kPfBatch - 1) / ((long long)kPfThreads * kPfBatch);
-    if (fgrid > fneed) fgrid = fneed > 0 ? fneed : 1;
     const long long bnd_cap = (long long)(kPfBndFactor * (size_t)T_cap);
-    pf_split_kernel<<<(int)fgrid, kPfThreads, 0, st>>>(weight, n, ctl, cand_w, cand_id, T_cap, bnd_w, bnd_id, bnd_cap);
+    pf_split_kernel<<<pf_pass_grid((const void *)pf_split_kernel, n), kPfThreads, 0, st>>>(
+        weight, 0, n, ctl, cand_w, cand_id, T_cap, bnd_w, bnd_id, bnd_cap);
     SX_LAUNCH_CHECK();
     unsigned long long n_bnd = 0;
     SX_CUDA(cudaMemcpyAsync(&n_bnd, &ctl->n_bnd, sizeof(n_bnd), cudaMemcpyDeviceToHost, st));
     SX_CUDA(cudaStreamSynchronize(st));
-    SX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pf_filter_kernel, kPfThreads, 0));
-    const long long filter_ctas = (long long)num_sms() * (occ > 0 ? occ : 1);
-    auto filter_grid = [&](long long cnt) {
-        long long need = (cnt / 2 + (long long)kPfThreads * kPfBatch - 1) / ((long long)kPfThreads * kPfBatch);
-        if (need < 1) need = 1;
-        return (int)(need < filter_ctas ? need : filter_ctas);
-    };
+    const void *filter = (const void *)pf_filter_kernel;
     if (n_bnd <= (unsigned long long)bnd_cap) {
         const long long mb = (long long)n_bnd;
         if (mb > 0) {
@@ -474,7 +508,8 @@ extern "C" int sx_kruskal_prefix(const double *weight, int64_t n, int64_t T, int
         pf_bound_kernel<1><<<1, 1024, 0, st>>>(ctl, (unsigned long long)T);
         SX_LAUNCH_CHECK();
         if (mb > 0) {
-            pf_filter_kernel<<<filter_grid(mb), kPfThreads, 0, st>>>(bnd_w, bnd_id, mb, ctl, cand_w, cand_id, T_cap);
+            pf_filter_kernel<<<pf_pass_grid(filter, mb), kPfThreads, 0, st>>>(bnd_w, bnd_id, 0, mb, ctl, cand_w,
+                                                                               cand_id, T_cap);
             SX_LAUNCH_CHECK();
         }
     } else {
@@ -483,7 +518,8 @@ extern "C" int sx_kruskal_prefix(const double *weight, int64_t n, int64_t T, int
         SX_LAUNCH_CHECK();
         pf_bound_kernel<1><<<1, 1024, 0, st>>>(ctl, (unsigned long long)T);
         SX_LAUNCH_CHECK();
-        pf_filter_kernel<<<filter_grid(n), kPfThreads, 0, st>>>(weight, nullptr, n, ctl, cand_w, cand_id, T_cap);
+        pf_filter_kernel<<<pf_pass_grid(filter, n), kPfThreads, 0, st>>>(weight, nullptr, 0, n, ctl, cand_w, cand_id,
+                                                                          T_cap);
         SX_LAUNCH_CHECK();
     }
     unsigned long long n_sel = 0;
@@ -493,18 +529,204 @@ extern "C" int sx_kruskal_prefix(const double *weight, int64_t n, int64_t T, int
         *n_prefix_h = -1;
         return SX_OK;
     }
-    const long long m = (long long)n_sel;
-    *n_prefix_h = m;
-    if (m == 0) return SX_OK;
-    // (weight, id) is a strict total order: sort by id, then stably by weight
-    int rc = sx_argsort_u64(cand_id, m, 32, perm, nullptr, sort_ws, sort_ws_bytes, st);
+    *n_prefix_h = (long long)n_sel;
+    return pf_order_tail(cand_w, cand_id, (long long)n_sel, T_cap, SX_ORDER_KRUSKAL, korder_out, tail_ws, st);
+}
+
+// ---- row-sharded form (sx_order_head_sharded_h) ------------------------------------------------------------------
+namespace {
+
+// One shard of sx_order_head_sharded_h: its weights, control block and candidate / boundary lists, carved from
+// one allocation on the shard's device.
+struct PfShard {
+    int dev = 0;
+    cudaStream_t st = nullptr;                 // the stream of this shard's device (shards of one device share it)
+    const double *w = nullptr;
+    long long n = 0;
+    unsigned long long id0 = 0;                // global id of the shard's first weight
+    void *mem = nullptr;
+    PrefixCtl *ctl = nullptr;
+    double *cand_w = nullptr, *bnd_w = nullptr;
+    unsigned long long *cand_id = nullptr, *bnd_id = nullptr;
+    unsigned long long n_bnd = 0, n_sel = 0;
+};
+
+struct PfSharded {
+    std::vector<PfShard> r;
+    std::vector<std::pair<int, cudaStream_t>> streams;   // one per distinct device
+    void *mem0 = nullptr;                                // gathered candidates + tail workspace, on r[0].dev
+    int prev = 0;
+    ~PfSharded() {
+        for (auto &ds : streams) {
+            cudaSetDevice(ds.first);
+            cudaStreamSynchronize(ds.second);
+            cudaStreamDestroy(ds.second);
+        }
+        for (PfShard &k : r) {
+            if (!k.mem) continue;
+            cudaSetDevice(k.dev);
+            cudaFree(k.mem);
+        }
+        if (mem0) { cudaSetDevice(r[0].dev); cudaFree(mem0); }
+        cudaSetDevice(prev);
+    }
+    int sync() {
+        for (auto &ds : streams) {
+            SX_CUDA(cudaSetDevice(ds.first));
+            SX_CUDA(cudaStreamSynchronize(ds.second));
+        }
+        return SX_OK;
+    }
+    // Sums the shards' level-LEVEL histograms on the host (S * D < 2^32: uint32 bins hold every count), writes the
+    // sum back into every shard's control block and finds the threshold bin there: every shard sees the same bound.
+    template <int LEVEL> int merge_hist(int64_t T, std::vector<unsigned> &h) {
+        const size_t G = r.size(), bytes = sizeof(unsigned) * kPfBins;
+        h.assign((G + 1) * kPfBins, 0u);
+        for (size_t g = 0; g < G; ++g) {
+            SX_CUDA(cudaSetDevice(r[g].dev));
+            SX_CUDA(cudaMemcpyAsync(&h[(g + 1) * kPfBins], r[g].ctl->hist[LEVEL], bytes, cudaMemcpyDeviceToHost, r[g].st));
+        }
+        int rc = sync();
+        if (rc != SX_OK) return rc;
+        for (size_t g = 0; g < G; ++g)
+            for (int b = 0; b < kPfBins; ++b) h[b] += h[(g + 1) * kPfBins + b];
+        for (PfShard &k : r) {
+            SX_CUDA(cudaSetDevice(k.dev));
+            SX_CUDA(cudaMemcpyAsync(k.ctl->hist[LEVEL], h.data(), bytes, cudaMemcpyHostToDevice, k.st));
+            pf_bound_kernel<LEVEL><<<1, 1024, 0, k.st>>>(k.ctl, (unsigned long long)T);
+            SX_LAUNCH_CHECK();
+        }
+        return SX_OK;
+    }
+};
+
+}  // namespace
+
+extern "C" int sx_order_head_sharded_h(int ndev, const int *devs, const double *const *weights,
+                                       const int64_t *row_bounds, int64_t S, int64_t D, int64_t T, int64_t T_cap,
+                                       const uint32_t *const *hist12, int mode, void *out, int64_t *n_out_h) {
+    if (ndev < 1 || ndev > 64 || !devs || !weights || S < 1 || D < 1 || ndev > S || T < 1 || T_cap < T || !out ||
+        !n_out_h || (mode != SX_ORDER_KRUSKAL && mode != SX_ORDER_QUEUE))
+        return SX_ERR_INVALID;
+    if (row_bounds) {
+        if (row_bounds[0] != 0 || row_bounds[ndev] != S) return SX_ERR_INVALID;
+        for (int g = 0; g < ndev; ++g) if (row_bounds[g + 1] <= row_bounds[g]) return SX_ERR_INVALID;
+    }
+    for (int g = 0; g < ndev; ++g) if (!weights[g]) return SX_ERR_INVALID;
+    if (S >= (1ll << 32) || D >= (1ll << 32) || (unsigned long long)S * (unsigned long long)D >= (1ull << 32))
+        return SX_ERR_TOO_LARGE;
+    const long long n = S * D;
+    if (T > n) T = n;
+    const int G = ndev;
+    const long long bnd_cap = (long long)(kPfBndFactor * (size_t)T_cap);
+    PfSharded sh;
+    SX_CUDA(cudaGetDevice(&sh.prev));
+    sh.r.resize(G);
+    for (int g = 0; g < G; ++g) {
+        PfShard &k = sh.r[g];
+        k.dev = devs[g];
+        k.w = weights[g];
+        const long long row0 = row_bounds ? row_bounds[g] : S * g / G;
+        k.n = ((row_bounds ? row_bounds[g + 1] : S * (g + 1) / G) - row0) * D;
+        k.id0 = (unsigned long long)(row0 * D);
+        if (cudaSetDevice(k.dev) != cudaSuccess) return SX_ERR_NO_DEVICE;
+        for (auto &ds : sh.streams) if (ds.first == k.dev) k.st = ds.second;
+        if (!k.st) {
+            SX_CUDA(cudaStreamCreateWithFlags(&k.st, cudaStreamNonBlocking));
+            sh.streams.emplace_back(k.dev, k.st);
+        }
+        SX_CUDA(cudaMalloc(&k.mem, carve_bytes(1, sizeof(PrefixCtl)) + 2 * carve_bytes((size_t)T_cap, 8) +
+                                       2 * carve_bytes((size_t)bnd_cap, 8)));
+        Carver cv(k.mem);
+        k.ctl = cv.take<PrefixCtl>(1);
+        k.cand_w = cv.take<double>(T_cap);
+        k.cand_id = cv.take<unsigned long long>(T_cap);
+        k.bnd_w = cv.take<double>(bnd_cap);
+        k.bnd_id = cv.take<unsigned long long>(bnd_cap);
+        // level 0: the shard's histogram (or the one sx_score_ot took while writing the scores)
+        SX_CUDA(cudaMemsetAsync(k.ctl, 0, sizeof(PrefixCtl), k.st));
+        if (hist12 && hist12[g]) {
+            SX_CUDA(cudaMemcpyAsync(k.ctl->hist[0], hist12[g], sizeof(unsigned) * kPfBins, cudaMemcpyDeviceToDevice,
+                                    k.st));
+        } else {
+            pf_hist_kernel<0><<<pf_grid(k.n, 16), kPfThreads, 0, k.st>>>(k.w, k.n, k.ctl, k.ctl->hist[0]);
+            SX_LAUNCH_CHECK();
+        }
+    }
+    std::vector<unsigned> h;
+    int rc = sh.merge_hist<0>(T, h);
     if (rc != SX_OK) return rc;
-    const int g2 = pf_grid(m, 1);
-    pf_gather_kernel<<<g2, kPfThreads, 0, st>>>(cand_w, cand_id, perm, m, w1, id1);
-    SX_LAUNCH_CHECK();
-    rc = sx_argsort_f64(w1, m, perm2, sorted_w, sort_ws, sort_ws_bytes, st);
+    // split pass on every shard, then each shard's level-1 histogram: on its boundary list, or on all its weights
+    // when the list overflowed (each shard decides for itself; the filter then selects that shard from scratch)
+    for (PfShard &k : sh.r) {
+        SX_CUDA(cudaSetDevice(k.dev));
+        pf_split_kernel<<<pf_pass_grid((const void *)pf_split_kernel, k.n), kPfThreads, 0, k.st>>>(
+            k.w, k.id0, k.n, k.ctl, k.cand_w, k.cand_id, T_cap, k.bnd_w, k.bnd_id, bnd_cap);
+        SX_LAUNCH_CHECK();
+    }
+    for (PfShard &k : sh.r) {
+        SX_CUDA(cudaSetDevice(k.dev));
+        SX_CUDA(cudaMemcpyAsync(&k.n_bnd, &k.ctl->n_bnd, sizeof(k.n_bnd), cudaMemcpyDeviceToHost, k.st));
+    }
+    if ((rc = sh.sync()) != SX_OK) return rc;
+    for (PfShard &k : sh.r) {
+        SX_CUDA(cudaSetDevice(k.dev));
+        if (k.n_bnd <= (unsigned long long)bnd_cap) {
+            if (k.n_bnd > 0)
+                pf_hist_kernel<1><<<pf_grid((long long)k.n_bnd, 16), kPfThreads, 0, k.st>>>(k.bnd_w, (long long)k.n_bnd,
+                                                                                          k.ctl, k.ctl->hist[1]);
+        } else {
+            SX_CUDA(cudaMemsetAsync(&k.ctl->n_sel, 0, sizeof(unsigned long long), k.st));
+            pf_hist_kernel<1><<<pf_grid(k.n, 16), kPfThreads, 0, k.st>>>(k.w, k.n, k.ctl, k.ctl->hist[1]);
+        }
+        SX_LAUNCH_CHECK();
+    }
+    if ((rc = sh.merge_hist<1>(T, h)) != SX_OK) return rc;
+    const void *filter = (const void *)pf_filter_kernel;
+    for (PfShard &k : sh.r) {
+        SX_CUDA(cudaSetDevice(k.dev));
+        if (k.n_bnd <= (unsigned long long)bnd_cap) {
+            const long long mb = (long long)k.n_bnd;
+            if (mb > 0)
+                pf_filter_kernel<<<pf_pass_grid(filter, mb), kPfThreads, 0, k.st>>>(k.bnd_w, k.bnd_id, 0, mb, k.ctl,
+                                                                                     k.cand_w, k.cand_id, T_cap);
+        } else {
+            pf_filter_kernel<<<pf_pass_grid(filter, k.n), kPfThreads, 0, k.st>>>(k.w, nullptr, k.id0, k.n, k.ctl,
+                                                                                  k.cand_w, k.cand_id, T_cap);
+        }
+        SX_LAUNCH_CHECK();
+        SX_CUDA(cudaMemcpyAsync(&k.n_sel, &k.ctl->n_sel, sizeof(k.n_sel), cudaMemcpyDeviceToHost, k.st));
+    }
+    if ((rc = sh.sync()) != SX_OK) return rc;
+    unsigned long long m = 0;
+    for (PfShard &k : sh.r) m += k.n_sel;          // a shard over T_cap puts the sum over T_cap too
+    if (m > (unsigned long long)T_cap) {           // too many ties at the threshold for this capacity
+        *n_out_h = -1;
+        return SX_OK;
+    }
+    // the candidates of every shard go to devs[0] (at most T_cap of them), where they are sorted and ordered
+    PfShard &k0 = sh.r[0];
+    SX_CUDA(cudaSetDevice(k0.dev));
+    SX_CUDA(cudaMalloc(&sh.mem0, 2 * carve_bytes((size_t)T_cap, 8) + pf_tail_bytes(T_cap) + 256));
+    Carver cv(sh.mem0);
+    double *all_w = cv.take<double>(T_cap);
+    unsigned long long *all_id = cv.take<unsigned long long>(T_cap);
+    void *tail_ws = cv.base + cv.off;
+    unsigned long long off = 0;
+    for (PfShard &k : sh.r) {
+        if (k.n_sel == 0) continue;
+        if (k.dev == k0.dev) {
+            SX_CUDA(cudaMemcpyAsync(all_w + off, k.cand_w, k.n_sel * 8, cudaMemcpyDeviceToDevice, k0.st));
+            SX_CUDA(cudaMemcpyAsync(all_id + off, k.cand_id, k.n_sel * 8, cudaMemcpyDeviceToDevice, k0.st));
+        } else {
+            SX_CUDA(cudaMemcpyPeerAsync(all_w + off, k0.dev, k.cand_w, k.dev, k.n_sel * 8, k0.st));
+            SX_CUDA(cudaMemcpyPeerAsync(all_id + off, k0.dev, k.cand_id, k.dev, k.n_sel * 8, k0.st));
+        }
+        off += k.n_sel;
+    }
+    rc = pf_order_tail(all_w, all_id, (long long)m, T_cap, mode, out, tail_ws, k0.st);
     if (rc != SX_OK) return rc;
-    pf_gather_ids_kernel<<<g2, kPfThreads, 0, st>>>(id1, perm2, m, order_asc);
-    SX_LAUNCH_CHECK();
-    return sx_kruskal_order(sorted_w, order_asc, m, korder_out, ko_ws, ko_ws_bytes, st);
+    SX_CUDA(cudaStreamSynchronize(k0.st));
+    *n_out_h = (long long)m;
+    return SX_OK;
 }

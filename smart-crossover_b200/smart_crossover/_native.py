@@ -23,6 +23,8 @@ SX_STATUS_K_MISMATCH = 4
 SX_STATUS_NAN_RC = 8
 SX_STATUS_REPEAT_MASK = 1
 SX_ABI_VERSION = 6
+SX_ORDER_KRUSKAL = 0
+SX_ORDER_QUEUE = 1
 
 
 class SxError(RuntimeError):
@@ -74,6 +76,7 @@ SIGNATURES = {
     "sx_kruskal_prefix_workspace_bytes": (_sz, [_i64]),
     "sx_hist12_f64": (_int, [_p, _i64, _p, _p]),
     "sx_kruskal_prefix": (_int, [_p, _i64, _i64, _i64, _p, _p, _p, _p, _sz, _p]),
+    "sx_order_head_sharded_h": (_int, [_int, _p, _p, _p, _i64, _i64, _i64, _i64, _p, _int, _p, _p]),
     "sx_kruskal_workspace_bytes": (_sz, [_i64, _i64]),
     "sx_kruskal": (_int, [_p, _i64, _p, _p, _i64, _i64, _i64, _p, _p, _p, _sz, _p]),
     "sx_tree_potentials_workspace_bytes": (_sz, [_i64]),

@@ -46,11 +46,12 @@ def _f64(t, device=None):
 
 
 # ---- K1 ------------------------------------------------------------------------------------
-def score_ot(x: torch.Tensor, s: torch.Tensor, d: torch.Tensor, want_hist: bool = False):
+def score_ot(x: torch.Tensor, s: torch.Tensor, d: torch.Tensor, want_hist: bool = False, out=None):
     """Flow indicators max(x_ij/s_i, x_ij/d_j); reference net_manager.py:377-378.  With want_hist also
-    returns the 4096-bin histogram of the scores' top key bits (input of `kruskal_prefix`)."""
+    returns the 4096-bin histogram of the scores' top key bits (input of `kruskal_prefix`).  `out`: a
+    contiguous S * D float64 tensor to write the scores into."""
     S, D = s.numel(), d.numel()
-    out = torch.empty(S * D, dtype=torch.float64, device=x.device)
+    out = torch.empty(S * D, dtype=torch.float64, device=x.device) if out is None else out
     hist = torch.zeros(4096, dtype=torch.int32, device=x.device) if want_hist else None
     check(lib.sx_score_ot(_ptr(x), _ptr(s), _ptr(d), S, D, _ptr(out), _ptr(hist), _stream()), "sx_score_ot")
     return (out, hist) if want_hist else out
@@ -460,15 +461,16 @@ def balanced_row_bounds(S: int, seconds_per_row, multiple: int = 16):
 
 
 class CostSlabs:
-    """Row shards of a dense S x D cost matrix, one per device, resident for the life of the problem (as the
-    reference keeps `ot.M` in its manager).  Leading dimension rounded up to even (TMA path)."""
+    """Row shards of a dense S x D matrix, one per device, resident for the life of the problem (as the
+    reference keeps `ot.M` in its manager).  A cost matrix has its leading dimension rounded up to even (TMA
+    path); a flow or its scores (`pad_ld=False`) has contiguous rows, which `sx_score_ot` needs."""
 
-    def __init__(self, S: int, D: int, devices, row_bounds=None):
+    def __init__(self, S: int, D: int, devices, row_bounds=None, pad_ld: bool = True):
         """`row_bounds` (G + 1 increasing row indices from 0 to S): shard g = rows [row_bounds[g], row_bounds[g+1]);
         default = equal shares.  See `balanced_row_bounds`."""
         _require_cuda()
         self.S, self.D, self.devices = int(S), int(D), list(devices)
-        self.ld = self.D + (self.D & 1)
+        self.ld = self.D + (self.D & 1) if pad_ld else self.D
         G = len(self.devices)
         if row_bounds is None:
             row_bounds = [self.S * g // G for g in range(G + 1)]
@@ -486,15 +488,39 @@ class CostSlabs:
         """(rows_g, D) view of shard g."""
         return self.t[g][:, :self.D]
 
+    def same_shards(self, other: "CostSlabs") -> bool:
+        """Whether `other` has this matrix's shape, devices and row bounds."""
+        return (self.S, self.D, self.devices, self.row_bounds) == (other.S, other.D, other.devices, other.row_bounds)
+
+    def take_flat(self, ids) -> np.ndarray:
+        """Entries at row-major ids (host int64 array), gathered shard by shard on the devices."""
+        ids = np.asarray(ids, dtype=np.int64)
+        out = np.empty(ids.shape)
+        i, j = np.divmod(ids, self.D)
+        for g, d in enumerate(self.devices):
+            r0, rows = self.row0[g], self.rows[g]
+            m = (i >= r0) & (i < r0 + rows)
+            if m.any():
+                ii = torch.from_numpy(i[m] - r0).to(torch.device("cuda", d))
+                jj = torch.from_numpy(j[m]).to(torch.device("cuda", d))
+                out[m] = self.t[g][ii, jj].cpu().numpy()
+        return out
+
     @classmethod
-    def from_host(cls, M, devices, border=None, row_bounds=None):
+    def from_host(cls, M, devices=None, border=None, row_bounds=None, like: "CostSlabs | None" = None):
         """Upload a host matrix.  `border` = (bigM, corner): the device matrix is the (S+1) x (D+1) big-M
         extension of M (net_manager.py:390-393) -- last row / column = bigM, corner = `corner` -- built on the
-        device, so the extended matrix never exists on the host."""
+        device, so the extended matrix never exists on the host.  `like`: a flow (S x D, or S * D flat) for the
+        problem whose cost slabs `like` are -- same devices and row bounds, contiguous rows."""
         M = np.asarray(M, dtype=np.float64)
+        if like is not None:
+            M = M.reshape(like.S, like.D)
         S0, D0 = M.shape
         S, D = (S0 + 1, D0 + 1) if border is not None else (S0, D0)
-        self = cls(S, D, devices, row_bounds)
+        if like is not None:
+            self = cls(S, D, like.devices, like.row_bounds, pad_ld=False)
+        else:
+            self = cls(S, D, devices, row_bounds)
         for g in range(len(self.devices)):
             r0, r1 = self.row0[g], self.row0[g] + self.rows[g]
             h1 = min(r1, S0)
@@ -565,6 +591,51 @@ class OTPricer:
             self.close()
         except Exception:
             pass
+
+
+def score_ot_slabs(x: CostSlabs, s: np.ndarray, d: np.ndarray):
+    """`score_ot` on every shard of a row-sharded flow, each on its own device: (score slabs with x's devices and
+    row bounds, each shard's level-0 histogram).  The scores never leave their devices."""
+    if x.ld != x.D:
+        raise ValueError("a sharded flow needs contiguous rows (CostSlabs(..., pad_ld=False) / from_host(like=))")
+    s = np.ascontiguousarray(s, dtype=np.float64)
+    d = np.ascontiguousarray(d, dtype=np.float64)
+    if s.size != x.S or d.size != x.D:
+        raise ValueError("marginals do not match the flow")
+    out = CostSlabs(x.S, x.D, x.devices, x.row_bounds, pad_ld=False)
+    hists = []
+    for g, dv in enumerate(x.devices):
+        with torch.cuda.device(dv):
+            r0 = x.row0[g]
+            s_g = torch.from_numpy(s[r0:r0 + x.rows[g]]).cuda()
+            d_g = torch.from_numpy(d).cuda()
+            hists.append(score_ot(x.t[g], s_g, d_g, want_hist=True, out=out.t[g].view(-1))[1])
+    return out, hists
+
+
+def order_head_sharded(w: CostSlabs, T: int, T_cap: int | None = None, hists=None, queue: bool = False):
+    """Head of the order of row-sharded weights (`sx_order_head_sharded_h`), on w.devices[0]: queue=False gives the
+    Kruskal order (descending weight, ties by ascending id; int32 tensor of uint32 ids), queue=True the queue order
+    (descending weight, ties by descending id; int64).  At least min(T, n) arcs, whole tie runs; None when more
+    than T_cap arcs tie at the threshold.  `hists`: the shards' level-0 histograms (`score_ot_slabs`)."""
+    if w.ld != w.D:
+        raise ValueError("sharded weights need contiguous rows")
+    G, n = len(w.devices), w.S * w.D
+    T = int(min(T, n))
+    T_cap = int(min(n, T_cap or max(2 * T, T + 65536)))
+    d0 = torch.device("cuda", w.devices[0])
+    out = torch.empty(T_cap, dtype=torch.int64 if queue else torch.int32, device=d0)
+    w.sync()                      # the weights (and `out`'s memory) are ready before the library's own streams run
+    hist_ptrs = (ctypes.c_void_p * G)(*[h.data_ptr() for h in hists]) if hists is not None else None
+    n_out = ctypes.c_int64(0)
+    check(lib.sx_order_head_sharded_h(G, (ctypes.c_int * G)(*w.devices),
+                                      (ctypes.c_void_p * G)(*[t.data_ptr() for t in w.t]),
+                                      (ctypes.c_int64 * (G + 1))(*w.row_bounds), w.S, w.D, T, T_cap, hist_ptrs,
+                                      _native.SX_ORDER_QUEUE if queue else _native.SX_ORDER_KRUSKAL, _ptr(out),
+                                      ctypes.byref(n_out)), "sx_order_head_sharded_h")
+    if n_out.value < 0:
+        return None
+    return out[:n_out.value]
 
 
 # ---- large device -> host downloads (get_sorted_flows returns two n-sized NumPy arrays) -----------------

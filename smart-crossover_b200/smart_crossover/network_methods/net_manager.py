@@ -125,18 +125,7 @@ class DeviceResidentCost:
 
     def take_flat(self, ids: np.ndarray) -> np.ndarray:
         """Entries at row-major arc ids, gathered from the device shards (the restricted master's costs)."""
-        import torch
-        ids = np.asarray(ids, dtype=np.int64)
-        out = np.empty(ids.size)
-        i, j = np.divmod(ids, self.slabs.D)
-        for g, d in enumerate(self.slabs.devices):
-            r0, rows = self.slabs.row0[g], self.slabs.rows[g]
-            m = (i >= r0) & (i < r0 + rows)
-            if m.any():
-                ii = torch.from_numpy(i[m] - r0).to(torch.device("cuda", d))
-                jj = torch.from_numpy(j[m]).to(torch.device("cuda", d))
-                out[m] = self.slabs.t[g][ii, jj].cpu().numpy()
-        return out
+        return self.slabs.take_flat(ids)
 
     def __array__(self, dtype=None, copy=None):
         raise TypeError("this cost matrix is device resident; it has no host copy")
@@ -181,6 +170,94 @@ class _SortedFlows:
                                              and np.shares_memory(weights, self.scores_np))
 
 
+NAN_WEIGHTS_MSG = "flow weights contain NaN (a zero marginal?): the spanning tree is undefined"
+
+
+class ShardedScores:
+    """Flow indicators of a row-sharded flow, left on the devices that hold its shards: the sharded counterpart of
+    `_SortedFlows`, and what `OTManager.get_sorted_flows` returns as the scores of a flow given as slabs.  Nothing
+    sorts all n arcs: `head` selects the first arcs of either order across the shards (`sx_order_head_sharded_h`).
+    A handle, not an array: `shape`, `len`, `take(ids)`; converting it to a host array raises."""
+
+    ndim = 1
+    dtype = np.dtype(np.float64)
+
+    def __init__(self, slabs, hists=None) -> None:
+        self.slabs, self.hists = slabs, hists
+        self.size = slabs.S * slabs.D
+        self.shape = (self.size,)
+        self._nan = None
+
+    def __len__(self) -> int:
+        return self.size
+
+    def __array__(self, dtype=None, copy=None):
+        raise TypeError("these flow scores are device resident; they have no host copy")
+
+    def take(self, ids: np.ndarray) -> np.ndarray:
+        """Scores of the arcs `ids` (host float64)."""
+        return self.slabs.take_flat(ids)
+
+    def has_nan(self) -> bool:
+        """Whether any score is NaN.  NaN and +inf share the top bin of the level-0 histograms, so only shards with
+        something there are scanned."""
+        if self._nan is None:
+            nan = False
+            for g, t in enumerate(self.slabs.t):
+                if self.hists is None or int(self.hists[g][4095].item()) != 0:
+                    nan = nan or bool(t.isnan().any().item())
+            self._nan = nan
+        return self._nan
+
+    def head(self, T: int, kruskal: bool, T_cap: int | None = None):
+        """At least min(T, n) arcs at the head of the Kruskal order (kruskal=True: uint32 ids as int32) or of the
+        queue (int64), on the first shard's device.  When the tie runs at the threshold do not fit T_cap the call
+        is repeated with 4 x T_cap; beyond the first device's memory it raises MemoryError."""
+        from smart_crossover import device as dev
+        from smart_crossover._native import SxError, lib
+        import torch
+        if self.has_nan():
+            raise ValueError(NAN_WEIGHTS_MSG)
+        n = self.size
+        T = int(min(T, n))
+        T_cap = int(min(n, T_cap or max(2 * T, T + 65536)))
+        while True:
+            try:
+                out = dev.order_head_sharded(self.slabs, T, T_cap, self.hists, queue=not kruskal)
+            except (torch.OutOfMemoryError, SxError) as e:
+                if isinstance(e, SxError) and not (e.code == -2 and lib.sx_last_cuda_error() == 2):
+                    raise
+                raise MemoryError(f"the head of {T} arcs (capacity {T_cap}) of the flow order does not fit on "
+                                  f"device {self.slabs.devices[0]}") from e
+            if out is not None:
+                return out
+            T_cap = min(n, 4 * T_cap)
+
+
+class ShardedQueue:
+    """The arcs of a sharded flow sorted by score, largest first (ties by descending arc id), as `column_generation`
+    reads it: `len(queue) == n` and `queue[a:b]` is the int64 host array the host path's queue gives.  Only the
+    head that slices have reached is materialised (`ShardedScores.head` in queue mode), grown geometrically."""
+
+    def __init__(self, scores: ShardedScores) -> None:
+        self.scores = scores
+        self._head = np.empty(0, dtype=np.int64)
+
+    def __len__(self) -> int:
+        return self.scores.size
+
+    def __getitem__(self, key) -> np.ndarray:
+        if not isinstance(key, slice):
+            raise TypeError("a sharded queue is read in slices")
+        a, b, step = key.indices(len(self))
+        if step != 1:
+            raise ValueError("a sharded queue is read in slices of step 1")
+        if b > self._head.size:
+            T = min(len(self), max(b, 2 * self._head.size, 1 << 16))
+            self._head = self.scores.head(T, kruskal=False).cpu().numpy()
+        return self._head[a:max(a, b)].copy()
+
+
 # =================================================================================================
 class OTManager:
     """Optimal-transport manager (reference `net_manager.py:322-509`).
@@ -202,16 +279,16 @@ class OTManager:
         self._mcf = None
         self._sorted = None
         self._bigM = None
+        if isinstance(ot.M, DeviceResidentCost):
+            self._slabs = ot.M.slabs
 
     @classmethod
     def from_device_cost(cls, s: np.ndarray, d: np.ndarray, slabs) -> "OTManager":
         """Manager over a cost matrix that already sits on the device(s) as `device.CostSlabs` (generated or
         uploaded there by the caller).  Scoring, the tree build, pricing and the restricted master work as
         usual; `to_MCF` / `get_mcf` / `extend_by_bigM` need the host matrix and are not available."""
-        mgr = cls(OptTransport(np.asarray(s, dtype=np.float64), np.asarray(d, dtype=np.float64),
-                               DeviceResidentCost(slabs)))
-        mgr._slabs = slabs
-        return mgr
+        return cls(OptTransport(np.asarray(s, dtype=np.float64), np.asarray(d, dtype=np.float64),
+                                DeviceResidentCost(slabs)))
 
     # ---- lazily built host / device state ---------------------------------------------------------
     @property
@@ -265,8 +342,19 @@ class OTManager:
     # ---- K1: scores + sorted queue --------------------------------------------------------------------
     def get_sorted_flows(self, x: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
         """Flow indicators max(x_ij/s_i, x_ij/d_j) and the arcs sorted by them, largest first
-        (stable sort: ties by descending arc id).  Reference :368-379."""
+        (stable sort: ties by descending arc id).  Reference :368-379.
+
+        `x` may also be the flow as row slabs (`device.CostSlabs`, e.g. `warm_start.sinkhorn(..., as_slabs=True)`)
+        with the devices and row bounds of the manager's cost slabs.  Each shard is then scored on its own GPU and
+        the call returns a lazy `ShardedQueue` and the device-resident `ShardedScores`: no n-sized array is sorted
+        or crosses PCIe."""
         dev = _dev()
+        if isinstance(x, dev.CostSlabs):
+            # (compared with the slabs already on the devices: a host cost matrix is not uploaded just to refuse x)
+            if self._slabs is None or not x.same_shards(self._slabs):
+                raise ValueError("the flow slabs must have the cost slabs' shape, devices and row bounds")
+            self._sorted = ShardedScores(*dev.score_ot_slabs(x, self.ot.s, self.ot.d))
+            return ShardedQueue(self._sorted), self._sorted
         scores_t = dev.score_ot(_cuda(np.asarray(x, dtype=np.float64).ravel()),
                                 _cuda(np.asarray(self.ot.s, dtype=np.float64)),
                                 _cuda(np.asarray(self.ot.d, dtype=np.float64)))

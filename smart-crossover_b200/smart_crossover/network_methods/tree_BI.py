@@ -1,7 +1,9 @@
 """Tree basis identification for optimal transport (TNET), reference `network_methods/tree_BI.py`.
 
   max_weight_spanning_tree  -> device: stable radix argsort of the weights, Kruskal order,
-                               chunked Kruskal with a lock-free union-find (sx_kruskal)
+                               chunked Kruskal with a lock-free union-find (sx_kruskal); scores of a
+                               row-sharded flow (`ShardedScores`): the head of the Kruskal order selected
+                               across the shards (sx_order_head_sharded_h), Kruskal on the first shard's GPU
   tree_potentials           -> device: Euler tour + list ranking (sx_tree_potentials); new, the
                                reference reads duals from the LP solver instead
   push_tree_to_bfs          -> device: the tree primal flows (`B x = b[:-1]`, tree_BI.py:74-76, SuperLU in
@@ -18,7 +20,8 @@ from typing import Tuple
 import numpy as np
 
 from smart_crossover.formats import OptTransport
-from smart_crossover.network_methods.net_manager import OTManager, _SortedFlows, _cuda, _dev
+from smart_crossover.network_methods.net_manager import (NAN_WEIGHTS_MSG, OTManager, ShardedScores, _SortedFlows,
+                                                         _cuda, _dev)
 from smart_crossover.output import Basis
 
 
@@ -56,11 +59,13 @@ def _device_tree(ot: OptTransport, flow_weights: np.ndarray, _sorted: _SortedFlo
     (`sx_kruskal_order_head`).  If the forest is incomplete the whole order is used.  All give the same
     tree: a prefix of a strict total order is unique."""
     dev = _dev()
-    S, D = np.asarray(ot.M).shape
+    S, D = np.shape(ot.M)                 # (.shape of the matrix object: a device-resident one has no host copy)
     N, n = S + D, S * D
+    if isinstance(flow_weights, ShardedScores):
+        return _sharded_tree(flow_weights, S, D)
     flow_weights = np.asarray(flow_weights, dtype=np.float64)
-    have_sort = _sorted is not None and _sorted.matches(flow_weights)
-    nan_msg = "flow weights contain NaN (a zero marginal?): the spanning tree is undefined"
+    have_sort = isinstance(_sorted, _SortedFlows) and _sorted.matches(flow_weights)
+    nan_msg = NAN_WEIGHTS_MSG
     if have_sort:
         # NaN keys sort last (NumPy order): one device read instead of an O(n) host scan
         if bool(_sorted.sorted_key[-1:].isnan().item()):
@@ -91,13 +96,32 @@ def _device_tree(ot: OptTransport, flow_weights: np.ndarray, _sorted: _SortedFlo
     return tree_t, int(n_t.item())
 
 
+def _sharded_tree(scores: ShardedScores, S: int, D: int):
+    """`_device_tree` for scores held as row shards on several GPUs: the head of the Kruskal order (16 N arcs) is
+    selected across the shards and Kruskal runs on the first shard's GPU.  An incomplete forest, or tie runs too
+    long for the head's capacity, repeat with 4 x the head until the whole order has been seen."""
+    import torch
+    dev = _dev()
+    N, n = S + D, S * D
+    T = PREFIX_FACTOR * N
+    with torch.cuda.device(scores.slabs.devices[0]):
+        while True:
+            head = scores.head(T, kruskal=True)
+            tree_t, n_t = dev.kruskal(head, N, S=S, D=D)
+            nt = int(n_t.item())
+            if nt == N - 1 or head.numel() >= n:
+                return tree_t, nt
+            T = min(n, 4 * T)
+
+
 def max_weight_spanning_tree(ot: OptTransport, flow_weights: np.ndarray, _sorted: _SortedFlows = None) -> np.ndarray:
     """Arc ids (ascending) of the maximum-weight spanning tree of K_{S,D}: Kruskal in the order
     'descending weight, ties by ascending arc id'.  Like the reference, tree arcs whose weight is
     exactly zero are dropped from the result (`np.flatnonzero` on the dense tree, tree_BI.py:56)."""
     tree_t, nt = _device_tree(ot, flow_weights, _sorted)
     tree = tree_t[:nt].cpu().numpy()
-    return tree[np.asarray(flow_weights)[tree] != 0]
+    w = flow_weights.take(tree) if isinstance(flow_weights, ShardedScores) else np.asarray(flow_weights)[tree]
+    return tree[w != 0]
 
 
 def tree_potentials(ot: OptTransport, tree: np.ndarray) -> np.ndarray:

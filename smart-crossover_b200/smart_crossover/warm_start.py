@@ -15,16 +15,21 @@ import ctypes
 import numpy as np
 
 
-def sinkhorn(a, b, M, reg: float, numItermax: int = 1000, stopThr: float = 1e-9, log: bool = False):
+def sinkhorn(a, b, M, reg: float, numItermax: int = 1000, stopThr: float = 1e-9, log: bool = False,
+             as_slabs: bool = False):
     """Entropic-regularised OT plan gamma = diag(u) exp(-M / reg) diag(v) between marginals a (S,)
-    and b (D,).  With log=True also returns {'niter', 'err', 'f', 'g'} (potentials reg*log u, reg*log v)."""
+    and b (D,).  With log=True also returns {'niter', 'err', 'f', 'g'} (potentials reg*log u, reg*log v).
+    as_slabs (M a `device.CostSlabs` only): return the plan as row slabs on M's devices (`CostSlabs` with
+    contiguous rows, the flow `OTManager.get_sorted_flows` scores shard by shard) instead of a host array."""
     import torch
     from smart_crossover import device as dev
     from smart_crossover._native import check, lib
 
     dev._require_cuda()
     if isinstance(M, dev.CostSlabs):
-        return _sinkhorn_slabs(a, b, M, reg, numItermax, stopThr, log)
+        return _sinkhorn_slabs(a, b, M, reg, numItermax, stopThr, log, as_slabs)
+    if as_slabs:
+        raise ValueError("as_slabs needs the cost matrix as device.CostSlabs")
     a_t, b_t = dev._f64(np.asarray(a, dtype=np.float64)), dev._f64(np.asarray(b, dtype=np.float64))
     M_t = dev._f64(M) if not (isinstance(M, torch.Tensor) and M.is_cuda) else M.contiguous()
     S, D = M_t.shape
@@ -45,10 +50,9 @@ def sinkhorn(a, b, M, reg: float, numItermax: int = 1000, stopThr: float = 1e-9,
     return plan
 
 
-def _sinkhorn_slabs(a, b, slabs, reg, numItermax, stopThr, log):
+def _sinkhorn_slabs(a, b, slabs, reg, numItermax, stopThr, log, as_slabs):
     """`sinkhorn` over the row shards of a `device.CostSlabs`: shard g's rows on its device, the plan assembled on
-    the host shard by shard.  The cost matrix is never read on the host."""
-    import torch
+    the host shard by shard (or left in place with as_slabs).  The cost matrix is never read on the host."""
     from smart_crossover import device as dev
     from smart_crossover._native import check, lib
 
@@ -57,7 +61,7 @@ def _sinkhorn_slabs(a, b, slabs, reg, numItermax, stopThr, log):
     b = np.ascontiguousarray(b, dtype=np.float64).ravel()
     if a.size != S or b.size != D:
         raise ValueError("marginals do not match the cost matrix")
-    X = [torch.empty(slabs.rows[g], D, dtype=torch.float64, device=slabs.t[g].device) for g in range(G)]
+    X = dev.CostSlabs(S, D, slabs.devices, slabs.row_bounds, pad_ld=False)
     f, g_pot = np.empty(S), np.empty(D)
     slabs.sync()
     iters, err = ctypes.c_int64(0), ctypes.c_double(0.0)
@@ -66,11 +70,14 @@ def _sinkhorn_slabs(a, b, slabs, reg, numItermax, stopThr, log):
                                        (ctypes.c_int64 * (G + 1))(*slabs.row_bounds), slabs.ld, S, D,
                                        a.ctypes.data, b.ctypes.data, float(reg), int(numItermax), float(stopThr), 10,
                                        f.ctypes.data, g_pot.ctypes.data,
-                                       (ctypes.c_void_p * G)(*[x.data_ptr() for x in X]),
+                                       (ctypes.c_void_p * G)(*[x.data_ptr() for x in X.t]),
                                        ctypes.byref(iters), ctypes.byref(err)), "sx_sinkhorn_ot_sharded_h")
-    plan = np.empty((S, D))
-    for g in range(G):
-        plan[slabs.row0[g]:slabs.row0[g] + slabs.rows[g]] = dev.to_host(X[g])
+    if as_slabs:
+        plan = X
+    else:
+        plan = np.empty((S, D))
+        for g in range(G):
+            plan[slabs.row0[g]:slabs.row0[g] + slabs.rows[g]] = dev.to_host(X.t[g])
     if log:
         return plan, {"niter": iters.value, "err": err.value, "f": f, "g": g_pot}
     return plan
