@@ -349,6 +349,28 @@ SX_API int    sx_price_dense_ot_fused_lb(const double *M, int64_t ld, const uint
                                          void *const *peer_bufs_dev, int rank, int G, int64_t *merged_out,
                                          int32_t *status_dev, void *ws, size_t ws_bytes, void *stream);
 
+/* ---- the big-M extension priced over the base slab (replaces, for the fused pass, the extended matrix the reference
+ * builds in extend_by_bigM, net_manager.py:381-400, and prices in check_optimality_condition, :474-497) ----
+ * sx_price_dense_ot_fused_bigm = sx_price_dense_ot_fused_lb over rows [row0, row0 + S_loc) of an S x D base matrix
+ * M, priced as that shard of the (S+1) x (D+1) extension: last column = bigM, last row = bigM, corner = `corner`.
+ * A small kernel first prices the shard's border arcs (i, D) and, when row0 + S_loc == S, the artificial row (S, j),
+ * j <= D, into the selection state the fused kernel then completes; the fused kernel reads the base slab as before
+ * (same bytes per arc, same lower-bound copy).  Arc ids are those of the extension, i (D + 1) + j, and count,
+ * minimum, NaN status and top-K are those of the physically extended matrix, bit for bit.
+ *   S: base rows.  y_src: the shard's S_loc source duals.  y_dst: D + 1 sink duals (the last = the artificial
+ *   sink's).  y_art: device pointer to u_S, the artificial source's dual (read only by the shard that ends at S;
+ *   may be NULL on the others).  bigM / corner: the border's costs.  Everything else as sx_price_dense_ot_fused_lb.
+ * Checks what sx_price_dense_ot_fused_lb checks, plus row0 + S_loc <= S and D + 1 < 2^31; on a bad argument
+ * nothing is launched.
+ */
+SX_API int    sx_price_dense_ot_fused_bigm(const double *M, int64_t ld, const uint32_t *lb, int64_t ld_lb, int64_t row0,
+                                           int64_t S_loc, int64_t S, int64_t D, const double *y_src,
+                                           const double *y_dst, const double *y_art, double bigM, double corner,
+                                           double tol, sx_fused_state *state, double *cand_rc, int64_t *cand_id,
+                                           int64_t cand_cap, int64_t K, int64_t *block, int64_t block_len,
+                                           void *const *peer_bufs_dev, int rank, int G, int64_t *merged_out,
+                                           int32_t *status_dev, void *ws, size_t ws_bytes, void *stream);
+
 /* ---- top-k most violating arcs (north_star extension; SURVEY.md section 8 row a9) -------
  * Among the candidates (rc, id) left by a pricing pass select the K smallest by (rc ascending,
  * id ascending).  sel / header are the pass's selection state and header (the candidate count
@@ -482,12 +504,21 @@ SX_API int    sx_sinkhorn_ot_sharded_h(int ndev, const int *devs, const double *
  *   fine: each worker copies its slice into pinned staging); returns count / min / top-K on the host and
  *   (status_h, may be NULL) the SX_STATUS_* bits that survived (SX_STATUS_NAN_RC).  Repeats the pass
  *   internally, with a larger candidate buffer, when the candidates overflowed it.
- * sx_ot_pricer_info: device / row range of shard g.  sx_ot_pricer_stats: passes, repeated passes, whether the
- *   fused kernel and the in-kernel merge are in use.
+ * sx_ot_pricer_info: device / row range of shard g (base rows for a bordered pricer).  sx_ot_pricer_stats:
+ *   passes, repeated passes, whether the fused kernel and the in-kernel merge are in use.
+ * sx_ot_pricer_create_bigm: the same pricer over the S x D base slabs of a problem extended by big-M (reference
+ *   net_manager.py:381-400: last column and last row = bigM, corner = `corner`), priced as the (S+1) x (D+1)
+ *   extension with sx_price_dense_ot_fused_bigm -- the extended matrix is never built.  sx_ot_pricer_price_h then
+ *   takes S + 1 source and D + 1 sink duals and returns arc ids of the extension.  Fused path only: even ld,
+ *   16-byte aligned slabs (SX_ERR_UNALIGNED otherwise) and K <= SX_TOPK_MAX_K (SX_ERR_TOO_LARGE), checked before
+ *   anything is allocated.
  */
 typedef struct sx_ot_pricer sx_ot_pricer;
 SX_API int    sx_ot_pricer_create(int ndev, const int *devs, const double *const *slabs, const int64_t *row_bounds,
                            int64_t ld, int64_t S, int64_t D, int64_t K, double tol, sx_ot_pricer **out);
+SX_API int    sx_ot_pricer_create_bigm(int ndev, const int *devs, const double *const *slabs,
+                                const int64_t *row_bounds, int64_t ld, int64_t S, int64_t D, double bigM,
+                                double corner, int64_t K, double tol, sx_ot_pricer **out);
 SX_API int    sx_ot_pricer_destroy(sx_ot_pricer *p);
 SX_API int    sx_ot_pricer_info(const sx_ot_pricer *p, int g, int *dev, int64_t *row0, int64_t *S_loc);
 SX_API int    sx_ot_pricer_price_h(sx_ot_pricer *p, const double *y_src_h, const double *y_dst_h,

@@ -86,7 +86,8 @@ __device__ __forceinline__ void stamp(FusedCtl *ctl, int i) {
 // 2 CTAs per SM hold at most 96 registers per thread: the 18 warps land 5 / 5 / 4 / 4 on the SM's four
 // sub-partitions, whose register files hold 16 384 registers each (112 per thread would pass a whole-SM count
 // but leave one CTA per SM).
-template <int ROWS, int STAGES, int LB_STAGES, int CWARPS, int MINB>
+// EXT_IDS: arc ids in the big-M extension's numbering (p.id_ld = D + 1; see price_tiles).
+template <int ROWS, int STAGES, int LB_STAGES, int CWARPS, int MINB, bool EXT_IDS>
 __global__ void __launch_bounds__((CWARPS + 1) * 32, MINB)
 price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_lb,
                    const DenseParams p0, const FusedParams f) {
@@ -129,8 +130,8 @@ price_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     // pass on this state was dense, where the re-reads would cost more than the fp64 walk (DESIGN.md 5).
     // n_violating_last is written after barrier 1 of a pass, so every CTA reads the same value here.
     const bool lb_walk = f.has_lb && ld_volatile_u64(&ctl->n_violating_last) <= f.lb_max_violating;
-    if (lb_walk) price_tiles<uint32_t, ROWS, LB_STAGES, CWARPS, false>(tmap_lb, p, smem_raw);
-    else         price_tiles<double, ROWS, STAGES, CWARPS, false>(tmap, p, smem_raw);
+    if (lb_walk) price_tiles<uint32_t, ROWS, LB_STAGES, CWARPS, false, EXT_IDS>(tmap_lb, p, smem_raw);
+    else         price_tiles<double, ROWS, STAGES, CWARPS, false, EXT_IDS>(tmap, p, smem_raw);
     if (blockIdx.x == 0 && tid == 0) ctl->walk = lb_walk ? 1u : 0u;
     stamp(ctl, 1);
 
@@ -220,6 +221,56 @@ __global__ void __launch_bounds__(256) fused_init_kernel(FusedState *st, unsigne
     if (blockIdx.x == 0 && threadIdx.x < sizeof(FusedCtl) / 4) reinterpret_cast<unsigned *>(&st->ctl)[threadIdx.x] = 0u;
 }
 
+// The border of the big-M extension (reference net_manager.py:390-393) of one row shard, priced into the selection
+// state the NEXT price_fused_kernel launch on this stream uses: arcs (i, D) at cost bigM for the shard's rows and,
+// on the shard that ends at S, the artificial row (S, j) at cost bigM and the corner (S, D) at cost `corner`.  The
+// fused kernel then prices the base slab with arc ids i (D + 1) + j (p.id_ld = D + 1), so count, minimum, NaN status
+// and candidates are those of the physically extended (S + 1) x (D + 1) matrix, without a copy of it.
+//
+// Why sel[ctl.pass & 1] is the right state, and clear: a fused pass reads `pass` at its start, prices into that
+// half, clears the OTHER half at its start and advances `pass` after barrier 1; sx_fused_state_init clears both
+// halves before the first pass.  So once the previous launch on the stream has finished, sel[pass & 1] is clear
+// and is the one the next fused launch prices into -- this kernel runs between the two.  It takes the violator
+// path of the walk (tile_epilogue / WarpTally / block_min_commit): exact count and minimum, NaN reduced costs raise
+// SX_STATUS_NAN_RC without being counted or selected, candidates are appended under the histogram bound.
+__global__ void __launch_bounds__(256) price_border_kernel(const DenseParams p0, FusedState *state,
+                                                          const double *y_art, long long S, double bigM,
+                                                          double corner) {
+    __shared__ long long scratch[256 / 32];
+    SelState *sel = &state->sel[ld_volatile_u64(&state->ctl.pass) & 1ull];
+    DenseParams p = p0;
+    p.sink.hdr = &sel->hdr;
+    p.sink.sel = sel;
+    const long long n_col = p.S_loc;                                     // (row0 + i, D), i < S_loc
+    const long long n = n_col + (p.row0 + p.S_loc == S ? p.D + 1 : 0);   // + (S, j), j <= D
+    const double v_art = __ldg(p.y_dst + p.D);
+    double tmin = INFINITY, lim = INFINITY;
+    WarpTally tally;
+    // the loop bound is uniform per block: every lane of a warp joins the votes of tile_epilogue
+    for (long long base = (long long)blockIdx.x * blockDim.x; base < n; base += (long long)gridDim.x * blockDim.x) {
+        const long long k = base + threadIdx.x;
+        double rc0[1] = {INFINITY}, rc1[1] = {INFINITY};
+        long long id = 0;
+        if (k < n_col) {
+            rc0[0] = bigM - (v_art - __ldg(p.y_src + k));
+            id = (p.row0 + k) * p.id_ld + p.D;
+        } else if (k < n) {
+            const long long j = k - n_col;
+            rc0[0] = (j < p.D ? bigM : corner) - (__ldg(p.y_dst + j) - __ldg(y_art));
+            id = S * p.id_ld + j;
+        }
+        tile_epilogue<1>(p, tally, tmin, lim, rc0, rc1, lt_or(rc0[0], lim, false), id, 0);
+    }
+    warp_flush(p.sink, tally);
+    block_min_commit(tmin, p.sink.hdr, scratch, 256 / 32, threadIdx.x >> 5, (unsigned long long)n);
+}
+
+struct BigMBorder {
+    long long     S;        // rows of the base matrix; the artificial row is S
+    const double *y_art;    // device: u_S
+    double        bigM, corner;
+};
+
 // the one pipeline shape the fused kernel is built for: 16 rows x 3 stages (fp64; 6 stages of the 4-byte copy: the
 // same 96 KB ring), 8 consumer warps, 2 CTAs per SM
 constexpr int kFRows = 16, kFStages = 3, kFLbStages = 6, kFWarps = 8, kFMinB = 2;
@@ -261,12 +312,16 @@ extern "C" int sx_price_dense_ot_fused(const double *M, int64_t ld, int64_t row0
                                       ws_bytes, stream);
 }
 
-extern "C" int sx_price_dense_ot_fused_lb(const double *M, int64_t ld, const uint32_t *lb, int64_t ld_lb, int64_t row0,
-                                          int64_t S_loc, int64_t D, const double *y_src, const double *y_dst,
-                                          double tol, sx_fused_state *state, double *cand_rc, int64_t *cand_id,
-                                          int64_t cand_cap, int64_t K, int64_t *block, int64_t block_len,
-                                          void *const *peer_bufs_dev, int rank, int G, int64_t *merged_out,
-                                          int32_t *status_dev, void *ws, size_t ws_bytes, void *stream) {
+namespace {
+
+// The fused pass over a base slab; with `bm` the border kernel first prices the big-M border into the same pass and
+// arc ids take the extended row stride D + 1.  Every argument is checked and both tensor maps are encoded before
+// the first launch, so a rejected call launches nothing.
+int fused_pass(const double *M, int64_t ld, const uint32_t *lb, int64_t ld_lb, int64_t row0, int64_t S_loc, int64_t D,
+               const double *y_src, const double *y_dst, double tol, sx_fused_state *state, double *cand_rc,
+               int64_t *cand_id, int64_t cand_cap, int64_t K, int64_t *block, int64_t block_len,
+               void *const *peer_bufs_dev, int rank, int G, int64_t *merged_out, int32_t *status_dev, void *ws,
+               size_t ws_bytes, void *stream, const BigMBorder *bm) {
     if (!M || !y_src || !y_dst || !state || !block || S_loc <= 0 || D <= 0 || ld < D || row0 < 0 || cand_cap < 0)
         return SX_ERR_INVALID;
     if (K < 1 || K > SX_TOPK_MAX_K || block_len < 2 * K + 6) return SX_ERR_INVALID;
@@ -282,7 +337,8 @@ extern "C" int sx_price_dense_ot_fused_lb(const double *M, int64_t ld, const uin
     cudaStream_t st = (cudaStream_t)stream;
 
     DenseParams p;
-    p.y_src = y_src; p.y_dst = y_dst; p.M = M; p.ld = ld; p.S_loc = S_loc; p.D = D; p.row0 = row0; p.thr = -tol;
+    p.y_src = y_src; p.y_dst = y_dst; p.M = M; p.ld = ld; p.S_loc = S_loc; p.D = D; p.row0 = row0;
+    p.id_ld = bm ? D + 1 : D; p.thr = -tol;
     p.sink.hdr = nullptr; p.sink.sel = nullptr;                   // set on the device from the pass parity
     p.sink.rc = cand_rc; p.sink.id = (int64_t *)cand_id; p.sink.cap = cand_cap;
     p.rc_out = nullptr; p.ld_out = 0; p.zero = 0; p.evict_first = 1; p.dyn_ctr = nullptr;
@@ -308,12 +364,14 @@ extern "C" int sx_price_dense_ot_fused_lb(const double *M, int64_t ld, const uin
     f.has_lb = lb ? 1 : 0;
     f.lb_max_violating = (unsigned long long)(lb_frac * (double)S_loc * (double)D);
 
-    auto kern = price_fused_kernel<kFRows, kFStages, kFLbStages, kFWarps, kFMinB>;
+    auto kern = bm ? price_fused_kernel<kFRows, kFStages, kFLbStages, kFWarps, kFMinB, true>
+                   : price_fused_kernel<kFRows, kFStages, kFLbStages, kFWarps, kFMinB, false>;
     constexpr size_t smem_f64 = tma_smem_bytes(kFRows, kFStages, kFWarps),
                      smem_lb = tma_smem_bytes(kFRows, kFLbStages, kFWarps, sizeof(uint32_t));
     constexpr size_t smem = smem_f64 > smem_lb ? smem_f64 : smem_lb;
     constexpr int threads = (kFWarps + 1) * 32;
-    static int occ_cached[64] = {0};
+    static int occ_cache[2][64] = {{0}};
+    int *occ_cached = occ_cache[bm ? 1 : 0];
     int dev = 0;
     SX_CUDA(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64) return SX_ERR_INVALID;
@@ -327,8 +385,42 @@ extern "C" int sx_price_dense_ot_fused_lb(const double *M, int64_t ld, const uin
     const long long total = p.n_row_tiles * p.n_col_blocks;
     long long grid = (long long)num_sms() * occ_cached[dev];
     if (grid > total) grid = total;
+    if (bm) {
+        const long long n = S_loc + (row0 + S_loc == bm->S ? D + 1 : 0);
+        long long bgrid = (n + 255) / 256;
+        if (bgrid > (long long)num_sms() * 4) bgrid = (long long)num_sms() * 4;
+        price_border_kernel<<<(unsigned)bgrid, 256, 0, st>>>(p, f.state, bm->y_art, bm->S, bm->bigM, bm->corner);
+        SX_LAUNCH_CHECK();
+    }
     void *args[] = {(void *)&map, (void *)&map_lb, (void *)&p, (void *)&f};
     // cooperative: the grid-wide barriers need every CTA resident (a plain launch measured the same speed)
     SX_CUDA(cudaLaunchCooperativeKernel((void *)kern, dim3((unsigned)grid), dim3(threads), args, smem, st));
     return SX_OK;
+}
+
+}  // namespace
+
+extern "C" int sx_price_dense_ot_fused_lb(const double *M, int64_t ld, const uint32_t *lb, int64_t ld_lb, int64_t row0,
+                                          int64_t S_loc, int64_t D, const double *y_src, const double *y_dst,
+                                          double tol, sx_fused_state *state, double *cand_rc, int64_t *cand_id,
+                                          int64_t cand_cap, int64_t K, int64_t *block, int64_t block_len,
+                                          void *const *peer_bufs_dev, int rank, int G, int64_t *merged_out,
+                                          int32_t *status_dev, void *ws, size_t ws_bytes, void *stream) {
+    return fused_pass(M, ld, lb, ld_lb, row0, S_loc, D, y_src, y_dst, tol, state, cand_rc, cand_id, cand_cap, K, block,
+                      block_len, peer_bufs_dev, rank, G, merged_out, status_dev, ws, ws_bytes, stream, nullptr);
+}
+
+extern "C" int sx_price_dense_ot_fused_bigm(const double *M, int64_t ld, const uint32_t *lb, int64_t ld_lb,
+                                            int64_t row0, int64_t S_loc, int64_t S, int64_t D, const double *y_src,
+                                            const double *y_dst, const double *y_art, double bigM, double corner,
+                                            double tol, sx_fused_state *state, double *cand_rc, int64_t *cand_id,
+                                            int64_t cand_cap, int64_t K, int64_t *block, int64_t block_len,
+                                            void *const *peer_bufs_dev, int rank, int G, int64_t *merged_out,
+                                            int32_t *status_dev, void *ws, size_t ws_bytes, void *stream) {
+    if (S_loc <= 0 || row0 < 0 || S < 1 || row0 + S_loc > S) return SX_ERR_INVALID;
+    if (row0 + S_loc == S && !y_art) return SX_ERR_INVALID;
+    if (D + 1 >= (1ll << 31)) return SX_ERR_TOO_LARGE;
+    const BigMBorder bm{S, y_art, bigM, corner};
+    return fused_pass(M, ld, lb, ld_lb, row0, S_loc, D, y_src, y_dst, tol, state, cand_rc, cand_id, cand_cap, K, block,
+                      block_len, peer_bufs_dev, rank, G, merged_out, status_dev, ws, ws_bytes, stream, &bm);
 }

@@ -110,7 +110,7 @@ price_dense_direct_kernel(const double *__restrict__ M, long long ld, const Dens
                 }
             }
         }
-        tile_epilogue<kDirectRows>(p, tally, tmin, lim, rc0, rc1, hit, (p.row0 + i0) * p.D + j0, p.D, kGap);
+        tile_epilogue<kDirectRows>(p, tally, tmin, lim, rc0, rc1, hit, (p.row0 + i0) * p.id_ld + j0, p.id_ld, kGap);
         rt += d_rt; cb += d_cb;
         if (cb >= p.n_col_blocks) { cb -= p.n_col_blocks; ++rt; }
     }
@@ -417,7 +417,8 @@ extern "C" int sx_price_dense_ot(const double *M, int64_t ld, int64_t row0, int6
     if (variant == 0 && (D >= (1ll << 31) || S_loc >= (1ll << 31))) variant = 1;
 
     DenseParams p;
-    p.y_src = y_src; p.y_dst = y_dst; p.M = M; p.ld = ld; p.S_loc = S_loc; p.D = D; p.row0 = row0; p.thr = -tol;
+    p.y_src = y_src; p.y_dst = y_dst; p.M = M; p.ld = ld; p.S_loc = S_loc; p.D = D; p.row0 = row0; p.id_ld = D;
+    p.thr = -tol;
     p.sink.hdr = header; p.sink.sel = (SelState *)sel; p.sink.rc = cand_rc; p.sink.id = (int64_t *)cand_id;
     p.sink.cap = cand_cap;
     p.rc_out = rc_out; p.ld_out = ld_out; p.zero = 0; p.evict_first = (uint32_t)g_tma_evict_first;

@@ -197,6 +197,7 @@ struct DenseParams {
     uint32_t      zero;    // 0, but only the host knows: see mbar_arrive_after
     uint32_t      evict_first;
     unsigned int *dyn_ctr; // tail stealing: device counter (0 at kernel start) or nullptr = static walk only
+    long long     id_ld;   // row stride of arc ids: D, or D + 1 when the slab is priced as part of a big-M extension
 };
 
 // Lazy epilogue of one warp's share of a tile: RPT rows x 2 columns per thread already in registers
@@ -248,7 +249,11 @@ __device__ __forceinline__ void tile_epilogue(const DenseParams &p, WarpTally &t
 //   operations as the fp64 walk, and unflagged ones enter the epilogue as +inf.  The running minimum is
 //   only ever updated from exact values, so count, minimum, NaN status and candidates are those of the
 //   fp64 walk, bit for bit.
-template <class T, int ROWS, int STAGES, int CWARPS, bool WRITE_RC>
+//
+// EXT_IDS: arc ids take the row stride p.id_ld (the big-M extension's D + 1) instead of p.D.  A compile-time choice:
+// a second loop-invariant stride live across the walk changes the register allocation (and the spills) of the
+// kernels that never need it, and every kernel built before the extension sets id_ld = D anyway.
+template <class T, int ROWS, int STAGES, int CWARPS, bool WRITE_RC, bool EXT_IDS = false>
 __device__ __forceinline__ void price_tiles(const CUtensorMap &tmap, const DenseParams &p, unsigned char *smem_raw) {
     static_assert(sizeof(T) == 8 || !WRITE_RC, "the lower-bound walk does not write reduced costs");
     static_assert(std::is_same<T, double>::value || std::is_same<T, uint32_t>::value, "fp64 M or its lower-bound words");
@@ -327,6 +332,7 @@ __device__ __forceinline__ void price_tiles(const CUtensorMap &tmap, const Dense
         WarpTally tally;
         // one tile: (rt, cb) in stage s of pipeline iteration it; `waited` = the stage's data is known to be there
         auto process = [&](long long rt, long long cb, int s, uint32_t it, bool waited) {
+            const long long id_ld = EXT_IDS ? p.id_ld : p.D;
             const long long j0 = cb * kBoxCols + 2 * c;
             const long long i0 = rt * ROWS + (long long)rg * RPT;
             const bool interior = (cb + 1) * kBoxCols <= p.D && (rt + 1) * ROWS <= p.S_loc;   // CTA-uniform
@@ -394,7 +400,7 @@ __device__ __forceinline__ void price_tiles(const CUtensorMap &tmap, const Dense
                     rc0[r] = f0 ? __ldg(row + (long long)r * p.ld) - w0 : INFINITY;
                     rc1[r] = f1 ? __ldg(row + (long long)r * p.ld + 1) - w1 : INFINITY;
                 }
-                tile_epilogue<RPT>(p, tally, tmin, lim, rc0, rc1, hit, (p.row0 + i0) * p.D + j0, p.D);
+                tile_epilogue<RPT>(p, tally, tmin, lim, rc0, rc1, hit, (p.row0 + i0) * id_ld + j0, id_ld);
                 return;
             }
             double rc0[RPT], rc1[RPT];
@@ -428,7 +434,7 @@ __device__ __forceinline__ void price_tiles(const CUtensorMap &tmap, const Dense
                     }
                 }
             }
-            tile_epilogue<RPT>(p, tally, tmin, lim, rc0, rc1, hit, (p.row0 + i0) * p.D + j0, p.D);
+            tile_epilogue<RPT>(p, tally, tmin, lim, rc0, rc1, hit, (p.row0 + i0) * id_ld + j0, id_ld);
         };
         uint32_t it = 0;
         for (long long k = 0; k < n_static; ++k, ++it) {

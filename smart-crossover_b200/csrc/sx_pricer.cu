@@ -13,6 +13,8 @@
 // The cost-matrix slabs are caller-owned device memory (the managers upload M once per problem).  On the fused
 // path the pricer builds one lower-bound copy per slab at create (sx_cost_lb_build: high words rounded toward
 // -inf, half the slab's bytes) and the fused pass streams it while few arcs violate.
+// A bordered pricer (sx_ot_pricer_create_bigm) holds the S x D base slabs and prices the (S+1) x (D+1) big-M
+// extension: each pass is sx_price_dense_ot_fused_bigm, the border kernel and the fused kernel over the base slab.
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -63,6 +65,8 @@ struct sx_ot_pricer {
     int64_t S = 0, D = 0, ld = 0, K = 0, Kp = 1, blk = 0, cap = 0;
     double tol = 0;
     bool fusable = false, merge_in_kernel = false, dead = false;
+    bool bigm = false;                                 // prices the big-M extension of the S x D base
+    double bigM = 0, corner = 0;
     std::vector<DevCtx *> ctx;
     // arguments of the pass in flight (read by the workers)
     const double *y_src_h = nullptr, *y_dst_h = nullptr;
@@ -89,21 +93,22 @@ int alloc_candidates(sx_ot_pricer *p, DevCtx *c, int64_t cap) {
 
 // One pass on one device; runs on that device's worker thread.
 int run_pass(sx_ot_pricer *p, DevCtx *c) {
-    const int64_t Kp = p->Kp, D = p->D;
-    // the duals this device needs: its own rows' source duals + every sink dual (pageable -> pinned)
-    // staged in chunks so that the DMA of one chunk overlaps the host copy of the next (the upload of the
-    // duals is most of what a pass costs beyond the kernel: 0.5-1 MB per GPU)
+    const int64_t Kp = p->Kp, D = p->D, Dy = p->bigm ? D + 1 : D;
+    // the duals this device needs: its own rows' source duals + every sink dual (+ u_S, the artificial source's, of
+    // a bordered pricer) (pageable -> pinned) staged in chunks so that the DMA of one chunk overlaps the host copy
+    // of the next (the upload of the duals is most of what a pass costs beyond the kernel: 0.5-1 MB per GPU)
     {
-        const size_t total = (size_t)(c->S_loc + D), chunk = 16384;          // 128 KB
+        const double *seg_from[3] = {p->y_src_h + c->row0, p->y_dst_h, p->y_src_h + p->S};
+        const size_t seg_end[3] = {(size_t)c->S_loc, (size_t)(c->S_loc + Dy), (size_t)(c->S_loc + Dy) + (p->bigm ? 1 : 0)};
+        const size_t total = seg_end[2], chunk = 16384;                      // 128 KB
         for (size_t off = 0; off < total; off += chunk) {
             const size_t len = total - off < chunk ? total - off : chunk;
-            for (size_t done = 0; done < len;) {                                // [off, off + len) spans the two host vectors
+            for (size_t done = 0; done < len;) {                                // [off, off + len) spans the host vectors
                 const size_t pos = off + done;
-                const bool in_src = pos < (size_t)c->S_loc;
-                const size_t left = in_src ? (size_t)c->S_loc - pos : total - pos;
+                const int s = pos < seg_end[0] ? 0 : pos < seg_end[1] ? 1 : 2;
+                const size_t left = seg_end[s] - pos;
                 const size_t n = left < len - done ? left : len - done;
-                const double *from = in_src ? p->y_src_h + c->row0 + pos : p->y_dst_h + (pos - (size_t)c->S_loc);
-                memcpy(c->h_y + pos, from, n * 8);
+                memcpy(c->h_y + pos, seg_from[s] + (pos - (s ? seg_end[s - 1] : 0)), n * 8);
                 done += n;
             }
             SX_CUDA(cudaMemcpyAsync(c->y_loc + off, c->h_y + off, len * 8, cudaMemcpyHostToDevice, c->st));
@@ -111,7 +116,14 @@ int run_pass(sx_ot_pricer *p, DevCtx *c) {
     }
     const int64_t cap = p->K > 0 ? p->cap : 0;
     int32_t *xstatus = reinterpret_cast<int32_t *>(c->merged + 2 * Kp + 5);
-    if (p->fusable) {
+    if (p->bigm) {
+        SXP(sx_price_dense_ot_fused_bigm(c->M, p->ld, c->lb, c->ld_lb, c->row0, c->S_loc, p->S, D, c->y_loc,
+                                         c->y_loc + c->S_loc, c->y_loc + c->S_loc + Dy, p->bigM, p->corner, p->tol,
+                                         (sx_fused_state *)c->fstate, c->cand_rc, c->cand_id, cap, Kp, c->block, p->blk,
+                                         p->G > 1 ? c->peer_bufs_dev : nullptr, c->g, p->G,
+                                         (p->G > 1 && p->merge_in_kernel) ? c->merged : nullptr, xstatus, c->topk_ws,
+                                         c->topk_ws_bytes, c->st));
+    } else if (p->fusable) {
         SXP(sx_price_dense_ot_fused_lb(c->M, p->ld, c->lb, c->ld_lb, c->row0, c->S_loc, D, c->y_loc,
                                        c->y_loc + c->S_loc, p->tol, (sx_fused_state *)c->fstate, c->cand_rc,
                                        c->cand_id, cap, Kp, c->block, p->blk, p->G > 1 ? c->peer_bufs_dev : nullptr,
@@ -234,9 +246,12 @@ extern "C" int sx_ot_pricer_destroy(sx_ot_pricer *p) {
 
 namespace {
 
-// want_lb: build the lower-bound copies (a pricer that prices once, sx_price_dense_ot_h, would only pay for them)
+struct Border { double bigM, corner; };
+
+// want_lb: build the lower-bound copies (a pricer that prices once, sx_price_dense_ot_h, would only pay for them).
+// bm: price the big-M extension of the S x D slabs (fused path only).
 int ot_pricer_create(int ndev, const int *devs, const double *const *slabs, const int64_t *row_bounds, int64_t ld,
-                     int64_t S, int64_t D, int64_t K, double tol, bool want_lb, sx_ot_pricer **out) {
+                     int64_t S, int64_t D, int64_t K, double tol, bool want_lb, const Border *bm, sx_ot_pricer **out) {
     if (!out) return SX_ERR_INVALID;
     *out = nullptr;
     if (ndev < 1 || ndev > 64 || !devs || !slabs || S < 1 || D < 1 || ld < D || K < 0) return SX_ERR_INVALID;
@@ -246,6 +261,12 @@ int ot_pricer_create(int ndev, const int *devs, const double *const *slabs, cons
         for (int g = 0; g < ndev; ++g) if (row_bounds[g + 1] <= row_bounds[g]) return SX_ERR_INVALID;
     }
     const int64_t Kp = K > 0 ? K : 1;
+    if (bm) {                                                 // the bordered form runs on the fused path only
+        for (int g = 0; g < ndev; ++g) if (!slabs[g]) return SX_ERR_INVALID;
+        if (Kp > SX_TOPK_MAX_K || D + 1 >= (1ll << 31)) return SX_ERR_TOO_LARGE;
+        if (ld % 2 != 0) return SX_ERR_UNALIGNED;
+        for (int g = 0; g < ndev; ++g) if (((uintptr_t)slabs[g] & 15) != 0) return SX_ERR_UNALIGNED;
+    }
     if (ndev > 1 && (K > SX_TOPK_MAX_K || (size_t)16 * ndev * Kp > 200 * 1024)) return SX_ERR_TOO_LARGE;
     int prev = 0;
     SX_CUDA(cudaGetDevice(&prev));
@@ -255,6 +276,9 @@ int ot_pricer_create(int ndev, const int *devs, const double *const *slabs, cons
     p->blk = 2 * Kp + 6;
     p->cap = K > 0 ? (64 * K > (1ll << 20) ? 64 * K : (1ll << 20)) : 0;
     p->fusable = (ld % 2 == 0) && Kp <= SX_TOPK_MAX_K;
+    p->bigm = bm != nullptr;
+    if (bm) { p->bigM = bm->bigM; p->corner = bm->corner; }
+    const int64_t n_y = D + (bm ? 2 : 0);                     // staged duals beyond the shard's sources
     p->merge_in_kernel = ndev > 1 && sx_fused_merge_fits(Kp, ndev);
     int rc = SX_OK;
     auto fail = [&](int code) { cudaSetDevice(prev); sx_ot_pricer_destroy(p); return code; };
@@ -276,7 +300,7 @@ int ot_pricer_create(int ndev, const int *devs, const double *const *slabs, cons
         }
 #define SXA(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) return fail(cuda_fail(_e)); } while (0)
         SXA(cudaStreamCreateWithFlags(&c->st, cudaStreamNonBlocking));
-        SXA(cudaMalloc(&c->y_loc, (size_t)(c->S_loc + D) * 8));
+        SXA(cudaMalloc(&c->y_loc, (size_t)(c->S_loc + n_y) * 8));
         SXA(cudaMalloc(&c->block, (size_t)p->blk * 8));
         SXA(cudaMalloc(&c->merged, (size_t)p->blk * 8));
         SXA(cudaMemsetAsync(c->block, 0, (size_t)p->blk * 8, c->st));
@@ -303,7 +327,7 @@ int ot_pricer_create(int ndev, const int *devs, const double *const *slabs, cons
             SXA(cudaMemsetAsync(c->ll_buf, 0, nb, c->st));
             SXA(cudaMalloc((void **)&c->peer_bufs_dev, sizeof(void *) * ndev));
         }
-        SXA(cudaHostAlloc((void **)&c->h_y, (size_t)(c->S_loc + D) * 8, cudaHostAllocDefault));
+        SXA(cudaHostAlloc((void **)&c->h_y, (size_t)(c->S_loc + n_y) * 8, cudaHostAllocDefault));
         SXA(cudaHostAlloc((void **)&c->h_out, (size_t)p->blk * 8, cudaHostAllocDefault));
         SXA(cudaStreamSynchronize(c->st));
     }
@@ -326,7 +350,14 @@ int ot_pricer_create(int ndev, const int *devs, const double *const *slabs, cons
 
 extern "C" int sx_ot_pricer_create(int ndev, const int *devs, const double *const *slabs, const int64_t *row_bounds,
                                    int64_t ld, int64_t S, int64_t D, int64_t K, double tol, sx_ot_pricer **out) {
-    return ot_pricer_create(ndev, devs, slabs, row_bounds, ld, S, D, K, tol, /*want_lb=*/true, out);
+    return ot_pricer_create(ndev, devs, slabs, row_bounds, ld, S, D, K, tol, /*want_lb=*/true, nullptr, out);
+}
+
+extern "C" int sx_ot_pricer_create_bigm(int ndev, const int *devs, const double *const *slabs,
+                                        const int64_t *row_bounds, int64_t ld, int64_t S, int64_t D, double bigM,
+                                        double corner, int64_t K, double tol, sx_ot_pricer **out) {
+    const Border bm{bigM, corner};
+    return ot_pricer_create(ndev, devs, slabs, row_bounds, ld, S, D, K, tol, /*want_lb=*/true, &bm, out);
 }
 
 extern "C" int sx_ot_pricer_info(const sx_ot_pricer *p, int g, int *dev, int64_t *row0, int64_t *S_loc) {
@@ -419,7 +450,7 @@ extern "C" int sx_price_dense_ot_h(const double *M_h, const double *M_dev, int64
     }
     sx_ot_pricer *p = nullptr;
     const double *slabs[1] = {M_dev};
-    int rc = ot_pricer_create(1, &dev, slabs, nullptr, ld, S, D, K, tol, /*want_lb=*/false, &p);
+    int rc = ot_pricer_create(1, &dev, slabs, nullptr, ld, S, D, K, tol, /*want_lb=*/false, nullptr, &p);
     if (rc == SX_OK) {
         rc = sx_ot_pricer_price_h(p, y_h, y_h + S, n_violating_h, min_rc_h, topk_rc_h, topk_id_h, topk_n_h, nullptr);
         sx_ot_pricer_destroy(p);

@@ -98,6 +98,8 @@ SIGNATURES = {
     "sx_cost_lb_build": (_int, [_p, _i64, _i64, _i64, _p, _i64, _p]),
     "sx_price_dense_ot_fused_lb": (_int, [_p, _i64, _p, _i64, _i64, _i64, _i64, _p, _p, _dbl, _p, _p, _p, _i64, _i64,
                                           _p, _i64, _p, _int, _int, _p, _p, _p, _sz, _p]),
+    "sx_price_dense_ot_fused_bigm": (_int, [_p, _i64, _p, _i64, _i64, _i64, _i64, _i64, _p, _p, _p, _dbl, _dbl, _dbl,
+                                            _p, _p, _p, _i64, _i64, _p, _i64, _p, _int, _int, _p, _p, _p, _sz, _p]),
     "sx_topk_workspace_bytes": (_sz, [_i64, _i64]),
     "sx_topk_select": (_int, [_p, _p, _i64, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
     "sx_topk_merge_workspace_bytes": (_sz, [_i64]),
@@ -114,6 +116,7 @@ SIGNATURES = {
                                         _p, _p, _p]),
     "sx_price_dense_ot_h": (_int, [_p, _p, _i64, _i64, _p, _dbl, _i64, _p, _p, _p, _p, _p]),
     "sx_ot_pricer_create": (_int, [_int, _p, _p, _p, _i64, _i64, _i64, _i64, _dbl, _p]),
+    "sx_ot_pricer_create_bigm": (_int, [_int, _p, _p, _p, _i64, _i64, _i64, _dbl, _dbl, _i64, _dbl, _p]),
     "sx_ot_pricer_destroy": (_int, [_p]),
     "sx_ot_pricer_info": (_int, [_p, _int, _p, _p, _p]),
     "sx_ot_pricer_price_h": (_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p]),

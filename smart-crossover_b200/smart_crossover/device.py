@@ -247,11 +247,22 @@ class Pricer:
         return M.data_ptr() % 16 == 0 and ld % 2 == 0
 
     def price_dense_fused(self, M, ld, row0, S_loc, D, y_src, y_dst, tol=TOL_RC, peer_bufs=None, rank=0, G=1,
-                          merged=None, xstatus=None, lb=None):
+                          merged=None, xstatus=None, lb=None, bigm=None):
         """begin + pricing + selection (+ push of the block to `peer_bufs`, + merge of the G blocks into
         `merged`) as one launch.  `lb`: the lower-bound copy of M (`cost_lb`); the pass may then stream it
-        instead of M, with the same results."""
-        if lb is not None:
+        instead of M, with the same results.  `bigm` = (S, y_art, bigM, corner): price the slab as rows
+        [row0, row0 + S_loc) of the (S+1) x (D+1) big-M extension of an S x D base (`sx_price_dense_ot_fused_bigm`):
+        y_dst then holds D + 1 sink duals, y_art (device, one element) is u_S, and ids are the extension's."""
+        if bigm is not None:
+            S, y_art, bigM, corner = bigm
+            check(lib.sx_price_dense_ot_fused_bigm(_ptr(M), ld, _ptr(lb), lb.stride(0) if lb is not None else 0, row0,
+                                                   S_loc, S, D, _ptr(y_src), _ptr(y_dst), _ptr(y_art), float(bigM),
+                                                   float(corner), float(tol), _ptr(self.fstate), _ptr(self.cand_rc),
+                                                   _ptr(self.cand_id), self.cap if self.K > 0 else 0, self.Kp,
+                                                   _ptr(self.block), self.block.numel(), peer_bufs, rank, G,
+                                                   _ptr(merged), _ptr(xstatus), _ptr(self.ws), self.ws.numel(),
+                                                   _stream()), "sx_price_dense_ot_fused_bigm")
+        elif lb is not None:
             check(lib.sx_price_dense_ot_fused_lb(_ptr(M), ld, _ptr(lb), lb.stride(0), row0, S_loc, D, _ptr(y_src),
                                                  _ptr(y_dst), float(tol), _ptr(self.fstate), _ptr(self.cand_rc),
                                                  _ptr(self.cand_id), self.cap if self.K > 0 else 0, self.Kp,
@@ -488,6 +499,11 @@ class CostSlabs:
         """(rows_g, D) view of shard g."""
         return self.t[g][:, :self.D]
 
+    def max(self) -> float:
+        """Largest entry of the S x D matrix over every shard (not the `ld` padding); NaN if any entry is NaN, as
+        `np.max` gives."""
+        return float(np.max([torch.amax(self.view(g)).item() for g in range(len(self.devices))]))
+
     def same_shards(self, other: "CostSlabs") -> bool:
         """Whether `other` has this matrix's shape, devices and row bounds."""
         return (self.S, self.D, self.devices, self.row_bounds) == (other.S, other.D, other.devices, other.row_bounds)
@@ -542,19 +558,29 @@ class CostSlabs:
 class OTPricer:
     """`sx_ot_pricer`: persistent pricer of one dense OT problem over the devices of its `CostSlabs`.
     `price(y_src, y_dst)` takes HOST vectors (the LP solver's duals) and returns a PriceResult; nothing is
-    allocated per pass.  One kernel per GPU and pass (price + select + NVLink push + merge)."""
+    allocated per pass.  One kernel per GPU and pass (price + select + NVLink push + merge).
 
-    def __init__(self, slabs: CostSlabs, K: int, tol: float = TOL_RC):
+    `bigm` = (bigM, corner): the slabs are the S x D base of a problem extended by big-M, and the pricer prices the
+    (S+1) x (D+1) extension (`sx_ot_pricer_create_bigm`; the extended matrix is never built): `price` takes S + 1
+    and D + 1 duals and returns arc ids of the extension."""
+
+    def __init__(self, slabs: CostSlabs, K: int, tol: float = TOL_RC, bigm=None):
         _require_cuda()
         self.slabs, self.K = slabs, int(K)
+        self.bigm = None if bigm is None else (float(bigm[0]), float(bigm[1]))
         G = len(slabs.devices)
         devs = (ctypes.c_int * G)(*slabs.devices)
         ptrs = (ctypes.c_void_p * G)(*[t.data_ptr() for t in slabs.t])
         self._h = ctypes.c_void_p()
         slabs.sync()
         bounds = (ctypes.c_int64 * (G + 1))(*slabs.row_bounds)
-        check(lib.sx_ot_pricer_create(G, devs, ptrs, bounds, slabs.ld, slabs.S, slabs.D, self.K, float(tol),
-                                      ctypes.byref(self._h)), "sx_ot_pricer_create")
+        if self.bigm is None:
+            check(lib.sx_ot_pricer_create(G, devs, ptrs, bounds, slabs.ld, slabs.S, slabs.D, self.K, float(tol),
+                                          ctypes.byref(self._h)), "sx_ot_pricer_create")
+        else:
+            check(lib.sx_ot_pricer_create_bigm(G, devs, ptrs, bounds, slabs.ld, slabs.S, slabs.D, self.bigm[0],
+                                               self.bigm[1], self.K, float(tol), ctypes.byref(self._h)),
+                  "sx_ot_pricer_create_bigm")
         Kp = max(self.K, 1)
         self._rc = np.empty(Kp, dtype=np.float64)
         self._id = np.empty(Kp, dtype=np.int64)
@@ -564,7 +590,8 @@ class OTPricer:
     def price(self, y_src: np.ndarray, y_dst: np.ndarray) -> PriceResult:
         y_src = np.ascontiguousarray(y_src, dtype=np.float64)
         y_dst = np.ascontiguousarray(y_dst, dtype=np.float64)
-        if y_src.size != self.slabs.S or y_dst.size != self.slabs.D:
+        ext = 1 if self.bigm is not None else 0
+        if y_src.size != self.slabs.S + ext or y_dst.size != self.slabs.D + ext:
             raise ValueError("dual vectors do not match the cost matrix")
         check(lib.sx_ot_pricer_price_h(self._h, y_src.ctypes.data, y_dst.ctypes.data, ctypes.byref(self._cnt),
                                        ctypes.byref(self._min), self._rc.ctypes.data, self._id.ctypes.data,

@@ -67,13 +67,16 @@ class BigMExtendedCost:
     """(S+1) x (D+1) cost matrix of the big-M extension (reference `net_manager.py:390-393`: last column and
     last row = bigM, corner = 0) as a VIEW of the original matrix: nothing is copied until somebody asks for
     the dense array (`np.asarray`), which the managers never do -- the sub-problem takes single entries
-    (`take_flat`) and the device builds its own extended copy (`CostSlabs.from_host(border=...)`)."""
+    (`take_flat`) and the device builds its own extended copy (`CostSlabs.from_host(border=...)`).
+
+    The base may be a `DeviceResidentCost`: `take_flat` then gathers inner entries from its slabs, the device
+    prices the extension over those slabs (`device.OTPricer(..., bigm=)`), and there is no dense array."""
 
     ndim = 2
     dtype = np.dtype(np.float64)
 
-    def __init__(self, base: np.ndarray, bigM: float) -> None:
-        self.base = np.asarray(base)
+    def __init__(self, base, bigM: float) -> None:
+        self.base = base if isinstance(base, DeviceResidentCost) else np.asarray(base)
         self.bigM = float(bigM)
         self.shape = (self.base.shape[0] + 1, self.base.shape[1] + 1)
         self.size = self.shape[0] * self.shape[1]
@@ -84,11 +87,16 @@ class BigMExtendedCost:
         i, j = np.divmod(np.asarray(ids, dtype=np.int64), D + 1)
         inner = (i < S) & (j < D)
         out = np.full(i.shape, self.bigM)
-        out[inner] = self.base[i[inner], j[inner]]
+        if isinstance(self.base, DeviceResidentCost):
+            out[inner] = self.base.take_flat(i[inner] * D + j[inner])
+        else:
+            out[inner] = self.base[i[inner], j[inner]]
         out[(i == S) & (j == D)] = 0.0
         return out
 
     def __array__(self, dtype=None, copy=None):
+        if isinstance(self.base, DeviceResidentCost):
+            return np.asarray(self.base)                # raises: a device-resident base has no host copy
         S, D = self.base.shape
         M = np.full(self.shape, self.bigM)
         M[:S, :D] = self.base
@@ -106,7 +114,9 @@ class BigMExtendedCost:
 
     flatten = ravel
 
-    def max(self):
+    def max(self, axis=None, out=None):
+        if axis is not None or out is not None:
+            raise ValueError("only the maximum over all entries is available")
         return max(float(self.base.max()), self.bigM, 0.0)
 
 
@@ -126,6 +136,12 @@ class DeviceResidentCost:
     def take_flat(self, ids: np.ndarray) -> np.ndarray:
         """Entries at row-major arc ids, gathered from the device shards (the restricted master's costs)."""
         return self.slabs.take_flat(ids)
+
+    def max(self, axis=None, out=None):
+        """Largest entry, taken on the shards' devices (what `np.max(cost)` calls); NaN if any entry is NaN."""
+        if axis is not None or out is not None:
+            raise ValueError("a device-resident cost matrix only gives its maximum over all entries")
+        return self.slabs.max()
 
     def __array__(self, dtype=None, copy=None):
         raise TypeError("this cost matrix is device resident; it has no host copy")
@@ -265,7 +281,8 @@ class OTManager:
     After `extend_by_bigM` the host-side `ot` is the (S+1) x (D+1) extended problem as in the reference,
     but its cost matrix is a view (`BigMExtendedCost`), not a copy; the device builds the extended matrix
     itself from the original block, so the S + D + 1 artificial arcs are priced by the same kernel as
-    everything else and arc ids come back in the extended numbering.
+    everything else and arc ids come back in the extended numbering.  A device-resident matrix keeps its slabs
+    and the pricer prices the border next to them (`device.OTPricer(..., bigm=)`), with the same ids and results.
     """
 
     def __init__(self, ot: OptTransport) -> None:
@@ -281,12 +298,16 @@ class OTManager:
         self._bigM = None
         if isinstance(ot.M, DeviceResidentCost):
             self._slabs = ot.M.slabs
+        elif isinstance(ot.M, BigMExtendedCost) and isinstance(ot.M.base, DeviceResidentCost):
+            self._slabs, self._bigM = ot.M.base.slabs, ot.M.bigM
 
     @classmethod
     def from_device_cost(cls, s: np.ndarray, d: np.ndarray, slabs) -> "OTManager":
         """Manager over a cost matrix that already sits on the device(s) as `device.CostSlabs` (generated or
         uploaded there by the caller).  Scoring, the tree build, pricing and the restricted master work as
-        usual; `to_MCF` / `get_mcf` / `extend_by_bigM` need the host matrix and are not available."""
+        usual.  `extend_by_bigM` keeps the slabs: the border of the extension is priced on the devices next to
+        them (`device.OTPricer(..., bigm=)`), so `cnet_ot` runs without a second, extended copy of the matrix.
+        `to_MCF` / `get_mcf` need the host matrix and are not available."""
         return cls(OptTransport(np.asarray(s, dtype=np.float64), np.asarray(d, dtype=np.float64),
                                 DeviceResidentCost(slabs)))
 
@@ -319,18 +340,29 @@ class OTManager:
                 self._slabs = dev.CostSlabs.from_host(self.ot.M, devices)
         return self._slabs
 
+    def _border(self):
+        """(bigM, corner) when the device slabs are the base of the big-M extension (a device-resident problem after
+        `extend_by_bigM`), else None."""
+        M = self.ot.M
+        if isinstance(M, BigMExtendedCost) and isinstance(M.base, DeviceResidentCost):
+            return M.bigM, 0.0
+        return None
+
     def _pricer(self, K: int):
         """One persistent pricer per top-K size (buffers, streams and worker threads live as long as the
         manager: a column-generation round allocates nothing)."""
         pr = self._pricers.get(K)
         if pr is None:
-            pr = self._pricers[K] = _dev().OTPricer(self._device_slabs(), K, tol=TOLERANCE_FOR_REDUCED_COSTS)
+            pr = self._pricers[K] = _dev().OTPricer(self._device_slabs(), K, tol=TOLERANCE_FOR_REDUCED_COSTS,
+                                                    bigm=self._border())
         return pr
 
-    def _drop_device_state(self):
+    def _drop_device_state(self, keep_slabs: bool = False):
         for pr in self._pricers.values():
             pr.close()
-        self._pricers, self._slabs = {}, None
+        self._pricers = {}
+        if not keep_slabs:
+            self._slabs = None
 
     def pricing_devices(self):
         """Devices the cost matrix is sharded over (diagnostics)."""
@@ -373,10 +405,12 @@ class OTManager:
         self.artificial_vars = np.concatenate([np.arange(S, dtype=np.int64) * (D + 1) + D,
                                                S * (D + 1) + np.arange(D + 1, dtype=np.int64)])
         self._bigM = float(bigM)
-        # `ot.M` becomes a view of the extended matrix: neither the host nor the PCIe link ever sees a copy
+        # `ot.M` becomes a view of the extended matrix: neither the host nor the PCIe link ever sees a copy.  A
+        # device-resident matrix keeps its slabs; the pricers built next price the border next to them.
+        device_resident = isinstance(self.ot.M, DeviceResidentCost)
         self.ot = OptTransport(np.append(self.ot.s, np.sum(self.ot.d)),
                                np.append(self.ot.d, np.sum(self.ot.s)), BigMExtendedCost(self.ot.M, bigM))
-        self._drop_device_state()
+        self._drop_device_state(keep_slabs=device_resident)
         self._mcf = None
         self._sorted = None
 
@@ -451,13 +485,22 @@ class OTManager:
             import torch
             dev = _dev()
             slabs = self._device_slabs()
+            Sb, Db = slabs.S, slabs.D                  # the slabs' own shape: (S - 1, D - 1) when they are the base
             rc = np.empty((S, D))
             for g, d in enumerate(slabs.devices):
                 with torch.cuda.device(d):
                     r0, rows = slabs.row0[g], slabs.rows[g]
-                    y_g = torch.from_numpy(np.concatenate([y[r0:r0 + rows], y[S:S + D]])).cuda()
+                    y_g = torch.from_numpy(np.concatenate([y[r0:r0 + rows], y[S:S + Db]])).cuda()
                     part = dev.price_dense_ot(slabs.view(g), y_g, K=0, tol=TOLERANCE_FOR_REDUCED_COSTS, want_rc=True)
-                    rc[r0:r0 + rows] = part.rc.cpu().numpy().reshape(rows, D)
+                    rc[r0:r0 + rows, :Db] = part.rc.cpu().numpy().reshape(rows, Db)
+            border = self._border()
+            if border is not None:
+                # the S + D + 1 border arcs, associated as the kernels do: c - (v_j - u_i)
+                bigM, corner = border
+                u, v = y[:S], y[S:S + D]
+                rc[:Sb, Db] = bigM - (v[Db] - u[:Sb])
+                rc[Sb, :Db] = bigM - (v[:Db] - u[Sb])
+                rc[Sb, Db] = corner - (v[Db] - u[Sb])
             res.rc = rc.ravel()
         return res
 
