@@ -207,6 +207,9 @@ SX_API int    sx_kruskal(const uint32_t *korder, int64_t n, const int32_t *tail,
  *   cost: indexed by arc id with leading dimension: cost[(k / D) * ld + k % D] when
  *   tail == NULL (dense OT cost matrix M), cost[k] otherwise.
  *   status_out (device int32): 0 or SX_ERR_NOT_SPANNING.
+ *   Accuracy: exact when every cost is a multiple of one 2^-e and max|y| < 2^52 * 2^-e; otherwise
+ *   |y - y_exact| <= 2 ceil(log2 H) * eps * max|y_exact| (H = 2 (N - 1)), normwise: the error of a node
+ *   follows its tour position, not its root path, so relative to a small |y| it can be large.
  */
 SX_API size_t sx_tree_potentials_workspace_bytes(int64_t N);
 SX_API int    sx_tree_potentials(const int64_t *tree, int64_t n_tree, const int32_t *tail,
@@ -218,7 +221,10 @@ SX_API int    sx_tree_potentials(const int64_t *tree, int64_t n_tree, const int3
 /* sx_tree_flows: primal flows of the tree basis, the solution of B x = b[:-1] with B = A[:-1, tree]
  * that the reference gets from SuperLU (tree_BI.py:74-76; the dropped row is the root's).  The flow
  * on tree arc t is +/- the sum of b over the subtree below it, taken as a difference of tour-order
- * prefix sums carried in double-double (each flow is accurate to an ulp of the exact subtree sum).
+ * prefix sums carried in double-double.  With s the exact subtree sum and sum|b| taken over the non-root
+ * nodes: |flow - s| <= ulp(s) / 2 + 2^-103 H sum|b| (H = 2 (N - 1)), hence within 1 ulp of s whenever
+ * sum|b| <= 2^50 |s| / H.  A subtree whose supplies cancel exactly gets +-0.0 when the tour's prefix
+ * sums are exact in double-double (supplies on one grid 2^-e spanning fewer than ~100 bits).
  *   b: N supplies (A x = b); flow_out[t] belongs to tree[t]; same workspace size and status as
  *   sx_tree_potentials.
  */

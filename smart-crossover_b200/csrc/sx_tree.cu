@@ -17,8 +17,17 @@
 // The same tour gives the tree's primal flows (sx_tree_flows; reference tree_BI.py:74-76 solves
 // B x = b[:-1] with SuperLU): the flow on a tree arc is +/- the sum of the supplies b over the
 // subtree hanging below it, i.e. a difference of two prefix sums of b taken in tour order.  The
-// prefix sums are carried in double-double (error-free TwoSum), so each flow is the correctly
-// rounded-to-1-ulp subtree sum no matter how large the running total is.
+// prefix sums are carried in double-double (error-free TwoSum): each prefix is off by at most about
+// 2^-105 H sum|b| (sum over the non-root nodes), so a flow is within 1/2 ulp + 2^-103 H sum|b| of the
+// exact subtree sum s, which is within 1 ulp of s whenever sum|b| <= 2^50 |s| / H.  It is not 1 ulp
+// regardless of the running total: a subtree sum 1e20 times smaller than sum|b| loses digits.
+//
+// Accuracy of the potentials (plain fp64 sums): every partial sum of the pointer jumping is the sum of
+// a contiguous stretch of the tour, i.e. a difference of two potentials.  So the potentials are exact
+// when all costs are multiples of one 2^-e and max|y| < 2^52 * 2^-e (integer costs, for one), and in
+// general the error is normwise, under one eps * max|y| per round: tested at <= 2 ceil(log2 H) eps max|y|.
+// Relative to a node's own |y| it can be far larger: with 1% of the costs 1e6 times the rest, tens of
+// thousands of nodes of a 1e5-node tree miss 1e-9 * |y| (DESIGN.md, tree kernels against exact references).
 #include "sx_common.cuh"
 #include "sx_gridbar.cuh"
 
@@ -106,6 +115,11 @@ tree_tour_kernel(long long H, long long N, long long root, int rounds, TreeArray
         a.node[0][succ].pred = (int)h;
         a.node[0][h].rank = 1;
     }
+    // A node without a half-edge is not spanned.  This check is needed as well as the one on unreached
+    // half-edges in the read-out: N - 1 arcs with a cycle can still form ONE tour through every half-edge
+    // (three parallel arcs between two nodes do), and then only the isolated nodes give them away.
+    for (long long v = gtid; v < N; v += gsz)
+        if (__ldcg(a.first + v) < 0) *status = SX_ERR_NOT_SPANNING;
     sync_all();
     if (gtid == 0) {
         const int f = __ldcg(a.first + root);
@@ -217,13 +231,17 @@ __global__ void __launch_bounds__(1024) flow_scan_kernel(long long H, const doub
 }
 
 // flow(t) = +/- (P[rank(up) - 1] - P[rank(down) - 2]): supplies of the subtree below arc t.
+// Arcs the tour never reached (not spanning; flow_scatter_kernel has set the status) are skipped: their
+// ranks run up to 2^rounds, past the H prefix sums.
 __global__ void flow_finalize_kernel(long long T, const TourNode *__restrict__ node,
                                      const double *__restrict__ phi, const double *__restrict__ plo,
                                      double *__restrict__ flow) {
     for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < T;
          t += (long long)gridDim.x * blockDim.x) {
         const long long ha = 2 * t, hb = 2 * t + 1;            // ha: minus -> plus, hb: plus -> minus
-        const int ra = node[ha].rank, rb = node[hb].rank;
+        const TourNode na = node[ha], nb = node[hb];
+        if (na.pred != -1 || nb.pred != -1) continue;
+        const int ra = na.rank, rb = nb.rank;
         const bool a_down = ra < rb;
         const long long r1 = (a_down ? ra : rb) - 1, r2 = (a_down ? rb : ra) - 1;  // tour positions (down, up), r1 < r2
         dd top{phi[r2], plo[r2]};
