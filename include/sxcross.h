@@ -100,6 +100,9 @@ SX_API double      sx_key_to_f64(long long key);        /* decode sx_price_heade
  *   out/in sums in ascending arc id (SciPy csr_matvec order), f_inv = 1/max(f1,f2),
  *   indicator = max over the two end nodes of |f_inv * x_hat|.  node_ptr (N+1) /
  *   node_arc / node_sign are the CSR arrays of the incidence matrix A (formats.py:118).
+ *   An entry with node_sign 0 (a stored zero of A) is no incidence: it enters neither sum, so a
+ *   NaN or infinite x_hat cannot reach that node through it.  u = inf gives x_hat = x + inf * 0 =
+ *   NaN, as in the reference; f = inf gives f_inv = 0, a subnormal f gives f_inv = inf.
  */
 SX_API int    sx_score_ot(const double *x, const double *s, const double *d, int64_t S, int64_t D,
                    double *score_out, uint32_t *hist12_out, void *stream);
@@ -258,7 +261,13 @@ SX_API int    sx_push_tree_h(const int64_t *tree_h, const double *flow_h, int64_
  *   SX_ERR_UNALIGNED otherwise), 1 = vectorised direct loads, 2 = scalar loads (any
  *   alignment), -1 = choose automatically.
  * sx_price_arcs replaces net_manager.py:293-319 for an arc list:
- *   rc_k = c_k - (y[tail_k] - y[head_k]), negated where vbasis_k == -2.
+ *   rc_k = c_k - (y[tail_k] - y[head_k]), negated where vbasis_k == -2 (+0.0 becomes -0.0).
+ *   Arc ids reported are id0 + k.  16-byte aligned c / tail / head / rc_out and a 4-byte aligned
+ *   vbasis take a vectorised kernel for the first E & ~3 arcs; anything else goes through the
+ *   scalar one, with the same results.
+ *   Its header->min_rc_key is the minimum over the reduced costs that are not NaN (+inf if all of
+ *   them are, as for an empty list); a zero minimum reads +0.0, since the key does not keep the
+ *   sign of zero.
  * Candidates: violators that can still be among the K most violating arcs are appended to
  *   cand_rc / cand_id (capacity cand_cap, unordered).  "Can still be" is decided from a running
  *   histogram of the appended reduced costs in `sel`, so the list stays O(K log(n / K)) long
