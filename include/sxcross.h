@@ -106,7 +106,9 @@ SX_API double      sx_key_to_f64(long long key);        /* decode sx_price_heade
  */
 SX_API int    sx_score_ot(const double *x, const double *s, const double *d, int64_t S, int64_t D,
                    double *score_out, uint32_t *hist12_out, void *stream);
-SX_API int    sx_score_set_tuning(int min_ctas_per_sm);   /* 4 (default, 64 registers) or 3 (78 registers) resident CTAs per SM */
+SX_API int    sx_score_set_tuning(int min_ctas_per_sm);   /* 4 (default, 64 registers) or 3 (78 registers) resident CTAs per SM,
+                                                             anything else SX_ERR_INVALID.  Both return the same scores and
+                                                             histogram bits; process-wide, for bench sweeps */
 SX_API size_t sx_score_mcf_workspace_bytes(int64_t N, int64_t E);
 SX_API int    sx_score_mcf(const double *x, const double *u, const int32_t *tail, const int32_t *head,
                     const int64_t *node_ptr, const int32_t *node_arc, const int8_t *node_sign,
@@ -292,11 +294,15 @@ SX_API int    sx_price_arcs(const double *c, const int32_t *tail, const int32_t 
                      int64_t *cand_id, int64_t cand_cap, double *rc_out, void *stream);
 
 /* Tuning knobs of sx_price_dense_ot (bench sweeps): index into the table of TMA pipeline shapes
- * {rows per box, stages, consumer warps, CTAs per SM} of variant 0 (see sx_price.cu), and the
- * CTAs per SM of the direct-load variants.  Negative / zero values leave a knob unchanged. */
+ * {rows per box, stages, consumer warps, CTAs per SM} of variant 0 (see sx_price.cu; 0..13, default 6),
+ * and the CTAs per SM of the direct-load variants (default 16).  Negative / zero values leave a knob
+ * unchanged; a shape past the table is SX_ERR_INVALID.  Every accepted shape, every CTA count and every
+ * option below returns the same bits: the same reduced costs, count, minimum, status and top-K
+ * after selection.  They change speed only. */
 SX_API int    sx_price_set_tuning(int tma_shape, int direct_ctas_per_sm);
 /* TMA descriptor / cache options of variant 0: l2_promotion 0..3 = none, 64 B, 128 B, 256 B (default);
- * evict_first 1 (default) / 0 = L2 evict-first or normal policy on the loads.  Negative = unchanged. */
+ * evict_first 1 (default) / 0 = L2 evict-first or normal policy on the loads.  Negative = unchanged,
+ * l2_promotion > 3 is SX_ERR_INVALID.  Cache hints only: the results do not change. */
 SX_API int    sx_price_set_tma_options(int l2_promotion, int evict_first);
 
 /* ---- K4 fused: one launch per pricing pass -------------------------------------------------
