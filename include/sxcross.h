@@ -121,6 +121,10 @@ SX_API int    sx_score_mcf(const double *x, const double *u, const int32_t *tail
  *   order_asc_out[p] = arc id of the p-th smallest key; ties by ascending arc id;
  *   -0.0 == +0.0; NaN sorts last (NumPy order).  sorted_key_out (optional, may be NULL)
  *   receives the keys in sorted order.
+ * sx_argsort_u64: the same order for uint64 keys, by their low 8 * max(2, ceil(key_bits / 8)) bits
+ *   (1 <= key_bits <= 64): whole bytes, at least two, so key_bits <= 16 sorts 16 bits and 17 sorts 24.
+ *   Bits above that range do not enter the order (keys equal below it are ties, by ascending id) and the
+ *   keys need not be below 2^key_bits; sorted_key_out carries each key whole, those bits included.
  * sx_queue_from_order:   queue = order_asc[::-1] widened to int64 (net_manager.py:184,379).
  * sx_kruskal_order:      descending key, ties by ASCENDING id = stable argsort of -key, the
  *   order SciPy's Kruskal visits arcs in (tree_BI.py:47,53; SURVEY.md H1).
